@@ -6,6 +6,7 @@
     python bench.py --impl reference [--config C] ...                # CPU arm: the oracle port on all host cores (+ the
                                                                      #   Python reference per core when baseline/_ref is staged)
     torchrun --nproc-per-node N ... bench.py --gpus N ...            # N > 1: one rank per GPU, NCCL
+    python bench.py ... --dump-outputs DIR                           # + what the last timed step computed, DIR/<name>.npy
 
 --config 3 (default; BASELINE.json configs[2], SURVEY.md §8d): gym-PBN/Bittner-100 steady-state-distribution estimate —
 2^20 chains per GPU, each step advances every chain by 9600 SSD iterations (histogram the 7 target genes, flip each gene
@@ -44,6 +45,8 @@ SEED = 0
 METRIC = "bittner100_env_steps_per_s"
 UNIT = "env-steps/s"
 SURVEY_INSTR_PER_UPDATE = 150.0  # SURVEY.md §8d: algorithmic thread-instructions per asynchronous micro-step
+DUMP_SAMPLE = 8192  # chains / envs whose state --dump-outputs writes (a fixed seeded sample: config 5 alone has 2^28 state bits)
+DUMP_LIMIT = 64 << 20
 
 
 def workload_config(n_gpus):
@@ -84,6 +87,28 @@ class ClockSampler:
         reasons = sorted({names[k] for r in self.rows if len(r) >= 7 for k in range(4) if r[3 + k].lower().startswith("active")})
         return {"sm_mhz": float(np.median(sm)) if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "reasons": reasons, "samples": len(sm)}
+
+
+def dump_outputs(out_dir, sim, planes, arrays):
+    """--dump-outputs: writes out_dir/<name>.npy for every device tensor in `arrays` (whole) and, for every packed state in
+    `planes`, the 0/1 node values of the same DUMP_SAMPLE chains (seeded, sorted ids) as float32 [sample][n].  Integer
+    results are stored as float64, which holds every count the workloads reach exactly."""
+    import torch
+
+    pick = np.sort(np.random.default_rng(0).choice(sim.B, min(sim.B, DUMP_SAMPLE), replace=False))
+    idx = torch.from_numpy(pick).to(sim.device)
+    arrays = dict(arrays, **{name: sim.unpack(p).index_select(0, idx) for name, p in planes.items()})
+    host = {}
+    for name, t in arrays.items():
+        a = t.cpu().numpy()
+        host[name] = a.astype(np.float32 if a.dtype.itemsize < 4 or a.dtype == np.float32 else np.float64)
+    total = sum(a.nbytes for a in host.values())
+    if total > DUMP_LIMIT:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT}-byte limit")
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    for name, a in host.items():
+        np.save(out / f"{name}.npy", a)
 
 
 # ------------------------------------------------------------------------------------------------ env.step workloads
@@ -295,7 +320,7 @@ def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    steps = max(1, args.steps)
+    steps = args.steps
     per_step = max(2.0, min(12.0, 60.0 / (steps + args.warmup)))
     wl = EnvWorkload(args.config) if args.config != 3 else None
     sample = (lambda s: wl.cpu_sample(s)) if wl else cpu_sample
@@ -416,7 +441,7 @@ def timed_ssd(D, net, chains_local, env0, steps, tgt, flush, warm=0):
     t_steps = sum(e[0].elapsed_time(e[2]) for e in ev) * 1e-3
     t_kernel = sum(e[0].elapsed_time(e[1]) for e in ev) * 1e-3 / steps
     tail_us = sum(e[1].elapsed_time(e[2]) for e in ev) * 1e3 / steps
-    return D.max_seconds(t_steps), t_kernel, tail_us, rows, sim.launches - launches0
+    return D.max_seconds(t_steps), t_kernel, tail_us, rows, sim.launches - launches0, sim
 
 
 def cross_n_check(D, net, tgt):
@@ -468,16 +493,20 @@ def run_gpu_ssd(args):
     # warm-up happens inside timed_ssd before its timed region; stdout is restored after the first collective has run
     sampler.start()
     time.sleep(0.2)
-    t_w, t_kernel, tail_w, rows, launches = timed_ssd(D, net, CHAINS_PER_GPU, rank * CHAINS_PER_GPU, args.steps, tgt, flush, warm)
+    t_w, t_kernel, tail_w, rows, launches, sim = timed_ssd(D, net, CHAINS_PER_GPU, rank * CHAINS_PER_GPU, args.steps, tgt, flush,
+                                                           warm)
     clocks = sampler.stop()
     D.restore_stdout()
     units = float(CHAINS_PER_GPU) * ITERS_PER_STEP * args.steps * world
     value = units / t_w
     assert int(rows.sum().item()) == (warm + args.steps) * CHAINS_PER_GPU * ITERS_PER_STEP * world  # every iteration was histogrammed
+    if args.dump_outputs and rank == 0:  # the all-reduced histogram of the last step and the chains' states after it
+        dump_outputs(args.dump_outputs, sim, {"state": sim.state}, {"hist": rows[-1]})
+    del sim
 
     # ---- strong scaling: the ONE 1.0e10-iteration estimate (2^20 chains in all) sharded over the ranks by global chain id
     s0, s1 = pdist.shard_range(CHAINS_PER_GPU, rank, world, align=32)
-    t_s, t_kernel_s, tail_s, rows_s, _ = timed_ssd(D, net, s1 - s0, s0, args.steps, tgt, flush, 1)
+    t_s, t_kernel_s, tail_s, rows_s, _, _ = timed_ssd(D, net, s1 - s0, s0, args.steps, tgt, flush, 1)
     assert int(rows_s.sum().item()) == (1 + args.steps) * CHAINS_PER_GPU * ITERS_PER_STEP
     strong = {"value": float(CHAINS_PER_GPU) * ITERS_PER_STEP * args.steps / t_s, "unit": UNIT, "scaling": "strong",
               "chains_total": CHAINS_PER_GPU, "ms_per_step": t_s * 1e3 / args.steps, "kernel_ms": t_kernel_s * 1e3,
@@ -582,6 +611,14 @@ def run_gpu_env(args):
     D.barrier()
     launches = wl.sim.launches - launches0
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:  # what the last step handed back, before the end-to-end loop steps the envs again
+        sim = wl.sim
+        arrays = {"reward": sim.reward, "terminated": sim.terminated, "truncated": sim.truncated, "inner": sim.inner}
+        planes = {"obs": sim.obs_state}
+        if args.config != 5:  # vec_step: episode bookkeeping and the observation each finished episode ended in
+            arrays.update(ep_return=wl.ep_return, ep_len=wl.ep_len, stats=wl.stats)
+            planes["final_obs"] = wl.final_obs
+        dump_outputs(args.dump_outputs, sim, planes, arrays)
     t = D.max_seconds(sum(a.elapsed_time(b) for a, b in ev) * 1e-3)
     units = float(wl.B) * args.steps * world
     value = units / t
@@ -631,7 +668,14 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", type=int, default=3, choices=[2, 3, 4, 5],
                     help="BASELINE.json configuration, 1-based as SURVEY.md §8d numbers them (3 = the headline SSD workload)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float32/float64; state "
+                         f"arrays for a fixed seeded sample of {DUMP_SAMPLE} chains or envs); same arguments, same inputs")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's outputs; the reference arm times samples and keeps none")
     if args.impl == "reference":
         run_reference(args)
     elif args.config == 3:
