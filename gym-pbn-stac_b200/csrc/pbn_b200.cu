@@ -873,6 +873,26 @@ __device__ __forceinline__ void tt_micro_step_words_sa(const TtView &tv, u32 wa,
     sts_u32(wd, v ? (old | m) : (old & ~m));
 }
 
+// control="write" (the PBCN envs of sampled_data.py and self_triggering.py): the control vector goes into nodes 0..M-1 before
+// every update.  For M <= 32 that is one masked store into the first state word, of bits gathered once per env.step, instead
+// of M single-bit writes fed by M global loads per update.  `ctl` = the env.step's actions from index 1 on (pbcn: the env
+// has a control vector there).
+struct CtlWrite {
+    const int *ctl;
+    u32 bits, mask;
+    __device__ __forceinline__ CtlWrite(const EnvView &ev, const int *c, bool pbcn)
+        : ctl(c), bits(0u), mask(ev.n_control >= 32 ? 0xFFFFFFFFu : ((1u << ev.n_control) - 1u)) {
+        if (pbcn && ev.control_write && ev.n_control <= 32)
+            for (int k = 0; k < ev.n_control; k++) bits |= (ctl[k] != 0 ? 1u : 0u) << k;
+    }
+    __device__ __forceinline__ void apply(const EnvView &ev, const Col &st) const {
+        if (!ev.control_write) return;
+        if (ev.n_control <= 32) st.set_word(0, (st.word(0) & ~mask) | bits);
+        else
+            for (int k = 0; k < ev.n_control; k++) st.put(k, ctl[k] != 0);
+    }
+};
+
 template <int NET, int MODE>
 __global__ void __launch_bounds__(PBN_BLOCK, 4) k_env_step(NetView nv, EnvView ev, DrawView dv, u32 *state, int *n_steps,
                                                         const int *target_att, const int *actions, int K, u32 *obs_state,
@@ -932,18 +952,9 @@ __global__ void __launch_bounds__(PBN_BLOCK, 4) k_env_step(NetView nv, EnvView e
     } break;
     case PBN_ENV_PBCN_SD: {  // sampled_data.py:139-189
         int interval = act[0], tstep = -1;
-        // control="write": the control vector goes into nodes 0..M-1 before every update; for M <= 32 that is one masked
-        // store into the first state word instead of M single-bit writes fed by M global loads per update
-        u32 cbits = 0;
-        const u32 cmask = ev.n_control >= 32 ? 0xFFFFFFFFu : ((1u << ev.n_control) - 1u);
-        if (ev.control_write && ev.n_control <= 32)
-            for (int c = 0; c < ev.n_control; c++) cbits |= (act[1 + c] != 0 ? 1u : 0u) << c;
+        const CtlWrite cw(ev, act + 1, true);
         auto one = [&](int i, auto &&step) {
-            if (ev.control_write) {
-                if (ev.n_control <= 32) st.set_word(0, (st.word(0) & ~cmask) | cbits);
-                else
-                    for (int c = 0; c < ev.n_control; c++) st.put(c, act[1 + c] != 0);
-            }
+            cw.apply(ev, st);
             step(); in++;
             int r = pbcn_reward_sa(ev, cv, tm) - 1;  // time_step_cost = 1
             if (tstep >= 0) r -= ev.successful_reward;                // overshoot penalty
@@ -975,10 +986,7 @@ __global__ void __launch_bounds__(PBN_BLOCK, 4) k_env_step(NetView nv, EnvView e
         if (pv < 1 || pv > 10) { bad++; pv = pv < 1 ? 1 : 10; }  // a stop probability of 0 would never end the macro step
         const double prob = (double)pv / 10.0;                 // convert value in [1,10] to [0.1 .. 1]
         const u32 stop_thr = (u32)ceil(prob * 2147483648.0);   // Philox: stop iff r31 < ceil(prob * 2^31)
-        u32 cbits = 0;
-        const u32 cmask = ev.n_control >= 32 ? 0xFFFFFFFFu : ((1u << ev.n_control) - 1u);
-        if (pbcn && ev.control_write && ev.n_control <= 32)
-            for (int c = 0; c < ev.n_control; c++) cbits |= (act[1 + c] != 0 ? 1u : 0u) << c;
+        const CtlWrite cw(ev, act + 1, pbcn);
         double total = 0.0;
         int i = 0;
         bool end = false;
@@ -990,11 +998,7 @@ __global__ void __launch_bounds__(PBN_BLOCK, 4) k_env_step(NetView nv, EnvView e
                 if (match_range_sa(cv, ev.tgt_first, ev.tgt_first + ev.n_tgt)) { r = 20; tm = 1; }
                 else { r = -4 - (a != 0); tm = 0; }
             } else {
-                if (ev.control_write) {
-                    if (ev.n_control <= 32) st.set_word(0, (st.word(0) & ~cmask) | cbits);
-                    else
-                        for (int c = 0; c < ev.n_control; c++) st.put(c, act[1 + c] != 0);
-                }
+                cw.apply(ev, st);
                 update();
                 r = pbcn_reward_sa(ev, cv, tm) - 1;  // time step cost
             }
@@ -1069,28 +1073,29 @@ __device__ __forceinline__ bool is_attracting_flat(const EnvView &ev, const int 
 
 // ---- pieces of one env.step of the step-until-attractor envs, shared by the kernels below
 // the intervention: pbn_target.py:261-269 (one node) / pbn_target_multi.py:120-134 (a set of nodes, the observation captured
-// BEFORE the first update).  Returns the pending action cost (MULTI: -len(actions)).
-__device__ __forceinline__ int att_begin(const NetView &nv, const EnvView &ev, const Col &st, const Col &ob, const int *act, int K,
-                                         int &bad) {
-    const int w32 = nv.w32;
+// BEFORE the first update).  An env.step with an out-of-range node is counted here, once, whichever pass finishes it.
+// Returns the pending action cost (MULTI: -len(actions)).
+__device__ __forceinline__ int att_begin(const NetView &nv, const EnvView &ev, const VecView &vx, unsigned long long *s_stats,
+                                         const Col &st, const Col &ob, const int *act, int K) {
+    int bad = 0, cnt = 0;
     if (ev.kind != PBN_ENV_MULTI) {
         const int a = act[0];
         if (a != 0) flip_node(st, a - 1, nv.n, bad);
-        return 0;
-    }
-    int cnt = 0;
-    for (int k = 0; k < K; k++) {
-        const int a = act[k];
-        if (a < 0) continue;
-        if (ev.dedup) {
-            bool dup = false;
-            for (int j = 0; j < k; j++) dup |= (act[j] == a);
-            if (dup) continue;
+    } else {
+        for (int k = 0; k < K; k++) {
+            const int a = act[k];
+            if (a < 0) continue;
+            if (ev.dedup) {
+                bool dup = false;
+                for (int j = 0; j < k; j++) dup |= (act[j] == a);
+                if (dup) continue;
+            }
+            cnt++;
+            if (a != 0) flip_node(st, a - 1, nv.n, bad);
         }
-        cnt++;
-        if (a != 0) flip_node(st, a - 1, nv.n, bad);
+        for (int w = 0; w < nv.w32; w++) ob.set_word(w, st.word(w));  // observation captured BEFORE the update (:133)
     }
-    for (int w = 0; w < w32; w++) ob.set_word(w, st.word(w));  // observation captured BEFORE the update (:133)
+    if (bad && vx.enabled) atomicAdd(&s_stats[6], 1ULL);  // env.steps whose intervention was out of range (ignored)
     return -cnt;  // reward -= len(actions)
 }
 // reward and flags of a finished env.step; `ob` = the observation the loop ended on (MULTI), st = the state
@@ -1107,10 +1112,42 @@ __device__ __forceinline__ void att_result(const EnvView &ev, const int *att_off
 
 // Budgeted / resumable execution (include/pbn_b200.h: PbnStepPlan).  Lists are {count, queue head, -, -, env ids...}.
 struct PlanView {
-    int budget, resume, dbg_a;
+    int budget, resume;
     unsigned char *running;
     int *list_in, *list_out;
 };
+
+// out of budget: park the env for a resume pass, which goes on from its state, update count and pending cost
+__device__ __forceinline__ void att_park(const PlanView &pl, const Col &st, u32 *state, int *inner_steps, int *reward, long long B,
+                                         long long e, int w32, int in, int pend) {
+    store_state(st, state, B, e, w32);
+    inner_steps[e] = in;
+    reward[e] = pend;
+    pl.running[e] = 1;
+    pl.list_out[4 + atomicAdd(&pl.list_out[0], 1)] = (int)e;
+}
+// a finished env.step: results, flags and the vector-env epilogue.  `fo` = the column the observation is (MULTI: the state
+// observed last), used_a / used_b = the draws record (Draw::tell); pl.running is null without a plan.
+template <int MODE>
+__device__ __forceinline__ void att_finish(const NetView &nv, const EnvView &ev, const DrawView &dv, const PlanView &pl, const VecView &vx,
+                                           unsigned long long *s_stats, const int *att_off, const u32 *cubes, const Col &st,
+                                           const Col &fo, u32 *state, int *n_steps, int *target_att, u32 *obs_state, int *reward,
+                                           unsigned char *terminated, unsigned char *truncated, int *inner_steps, long long B,
+                                           long long e, long long env0, int in, int pend, u32 used_a, u32 used_b) {
+    const int w32 = nv.w32;
+    int rew, tm;
+    att_result(ev, att_off, cubes, st, fo, w32, target_att[e], pend, rew, tm);
+    store_state(st, state, B, e, w32);
+    if (obs_state) store_state(fo, obs_state, B, e, w32);
+    reward[e] = rew;
+    terminated[e] = (unsigned char)tm;
+    const int tr = (n_steps[e] == ev.horizon);
+    truncated[e] = (unsigned char)tr;
+    if (inner_steps) inner_steps[e] = in;
+    if (pl.running) pl.running[e] = 0;
+    if (dv.used) { dv.used[2 * e] = used_a; dv.used[2 * e + 1] = used_b; }
+    if (vx.enabled) vec_finish<MODE>(nv, ev, vx, s_stats, state, n_steps, target_att, obs_state, B, e, env0, rew, tm, tr, in);
+}
 
 // W1: one-word networks (N <= 32) — the group runner keeps the state in a register; a separate instantiation, because both
 // runners inlined in one kernel made it 120 KB of SASS and instruction fetch its top stall (ncu: no_inst 21 %)
@@ -1170,8 +1207,7 @@ __global__ void __launch_bounds__(PBN_BLOCK, 2) k_env_step_att(NetView nv, EnvVi
     int osh = 2;
     if (resume) {
         const long long nb = gridDim.x;
-        int A = hi <= nb * 4 * 8 ? 4 : 8;
-        if (pl.dbg_a > 0) A = pl.dbg_a;
+        const int A = hi <= nb * 4 * 8 ? 4 : 8;
         if (grp && A == 8 && hi > nb * 8 * 8 * PBN_COOP_WIDE_FACTOR && ev.n_att > 0 && att_off[ev.n_att] <= 4) osh = 1;
         const int qmax = 32 >> osh;
         const long long q = (hi + nb * A - 1) / (nb * A);
@@ -1206,29 +1242,8 @@ __global__ void __launch_bounds__(PBN_BLOCK, 2) k_env_step_att(NetView nv, EnvVi
             e = nxt;
             load_state(st, state, B, e, w32);
             d.init(dv, e, env0 + e);
-            const int *act = actions + e * K;
             n_steps[e] += 1;
-            int bad = 0;
-            if (!multi) {  // pbn_target.py:261-269
-                const int a = act[0];
-                if (a != 0) flip_node(st, a - 1, nv.n, bad);
-            } else {  // pbn_target_multi.py:120-134
-                int cnt = 0;
-                for (int k = 0; k < K; k++) {
-                    const int a = act[k];
-                    if (a < 0) continue;
-                    if (ev.dedup) {
-                        bool dup = false;
-                        for (int j = 0; j < k; j++) dup |= (act[j] == a);
-                        if (dup) continue;
-                    }
-                    cnt++;
-                    if (a != 0) flip_node(st, a - 1, nv.n, bad);
-                }
-                pend = -cnt;  // reward -= len(actions)
-                for (int w = 0; w < w32; w++) ob.set_word(w, st.word(w));  // observation captured BEFORE the update (:133)
-            }
-            if (bad && vx.enabled) atomicAdd(&s_stats[6], 1ULL);
+            pend = att_begin(nv, ev, vx, s_stats, st, ob, actions + e * K, K);
             micro_step<NET, MODE, TQ>(nv, blob, st, d);
             in = 1;
             used = 1;
@@ -1242,12 +1257,8 @@ __global__ void __launch_bounds__(PBN_BLOCK, 2) k_env_step_att(NetView nv, EnvVi
             // while not force and not is_attracting_state(state): graph.step()                  (pbn_target.py:270-271)
             // while not is_attracting_state(observation): observation = graph.step()            (pbn_target_multi.py:135-146)
             const bool done = (!multi && ev.force) || in >= ev.max_inner || is_attracting(ev, att_off, cubes, multi ? ob : st, w32);
-            if (!done && pl.budget > 0 && used >= pl.budget) {  // out of budget: park the env for a resume pass
-                store_state(st, state, B, e, w32);
-                inner_steps[e] = in;
-                reward[e] = pend;
-                pl.running[e] = 1;
-                pl.list_out[4 + atomicAdd(&pl.list_out[0], 1)] = (int)e;
+            if (!done && pl.budget > 0 && used >= pl.budget) {
+                att_park(pl, st, state, inner_steps, reward, B, e, w32, in, pend);
                 have = false;
                 nxt = resume ? static_n + (long long)atomicAdd(&pl.list_in[1], 1) : lo + atomicAdd(&s_next, 1);
             } else if (!done) {
@@ -1257,24 +1268,11 @@ __global__ void __launch_bounds__(PBN_BLOCK, 2) k_env_step_att(NetView nv, EnvVi
                 in++;
                 used++;
             } else {
-                int rew, tm = 0;
-                const int ta = target_att[e];
-                if (!multi) {  // PBNTargetEnv._get_reward, pbn_target.py:303-326: any cube of the target attractor
-                    if (match_range(cubes, att_off[ta], att_off[ta + 1], st, w32)) { rew = 20; tm = 1; } else rew = -5;
-                } else {  // in_target returns at the first mismatch of the FIRST cube (Q12), pbn_target_multi.py:190-225
-                    rew = pend;
-                    if (att_off[ta] < att_off[ta + 1] && cube_match(cubes, att_off[ta], ob, w32)) { rew += 1000; tm = 1; }
-                }
-                store_state(st, state, B, e, w32);
-                if (obs_state) store_state(multi ? ob : st, obs_state, B, e, w32);
-                reward[e] = rew;
-                terminated[e] = (unsigned char)tm;
-                const int tr = (n_steps[e] == ev.horizon);
-                truncated[e] = (unsigned char)tr;
-                if (inner_steps) inner_steps[e] = in;
-                if (pl.running) pl.running[e] = 0;
-                d.done(dv, e);
-                if (vx.enabled) vec_finish<MODE>(nv, ev, vx, s_stats, state, n_steps, const_cast<int *>(target_att), obs_state, B, e, env0, rew, tm, tr, in);
+                u32 ua, ub;
+                d.tell(ua, ub);
+                att_finish<MODE>(nv, ev, dv, pl, vx, s_stats, att_off, cubes, st, multi ? ob : st, state, n_steps,
+                                 const_cast<int *>(target_att), obs_state, reward, terminated, truncated, inner_steps, B, e, env0,
+                                 in, pend, ua, ub);
                 have = false;
                 nxt = resume ? static_n + (long long)atomicAdd(&pl.list_in[1], 1) : lo + atomicAdd(&s_next, 1);
             }
@@ -1290,38 +1288,21 @@ __global__ void __launch_bounds__(PBN_BLOCK, 2) k_env_step_att(NetView nv, EnvVi
             qn = __shfl_sync(0xFFFFFFFFu, qn, 0);
             const bool drained = (resume ? static_n : lo) + qn >= hi;
             if (coop_on && hv != 0u && (grp || (__popc(live) <= PBN_COOP_MAX && drained))) {
-                const int nl = __popc(hv);
-                int k = 1;
-                while (k < nl) k <<= 1;                 // groups: 1, 2, 4, 8 (or 16 in a wide resume pass)
-                const int g = 32 / k;                   // lanes per group
-                const int grp = (int)lane / g;
-                const bool active = grp < nl;
-                const int owner = active ? (int)__fns(hv, 0u, grp + 1) : 0;  // the grp-th live lane
-                const long long eL = __shfl_sync(0xFFFFFFFFu, e, owner);
-                const int inL = __shfl_sync(0xFFFFFFFFu, in, owner);
                 // the group stops at the cap or when the launch's budget for the env is used up, whichever comes first
                 int stop_in = ev.max_inner;
                 if (pl.budget > 0 && in - used + pl.budget < stop_in) stop_in = in - used + pl.budget;
-                stop_in = __shfl_sync(0xFFFFFFFFu, stop_in, owner);
-                u32 *colL = sst + (threadIdx.x & ~31u) + (u32)owner;
-                unsigned char *wb = coop_buf + (threadIdx.x >> 5) * coop_warp_bytes(w32);
                 // the call returns when `exit_at` groups have stopped: their owners finalize on the next trip (and, while the
                 // block's queue lasts, start the next env), the other envs come back here — in wider groups once the queue
                 // is empty, which is why the first stop ends the call then
-                const int exit_at = drained ? 1 : (k > 8 ? 2 * PBN_COOP_EXIT_AT : PBN_COOP_EXIT_AT);
-                const int fin = coop_steps<TQ, W1>(nv, ev, dv, blob, att_off, cubes, colL, env0 + eL, inL, stop_in, active, g, 0u, wb, exit_at);
-                __syncwarp();
-                for (int r = 0; r < nl; r++) {          // hand each group's count back to the lane that owns the env
-                    const int v = __shfl_sync(0xFFFFFFFFu, fin, r * g);
-                    if ((int)lane == (int)__fns(hv, 0u, r + 1) && v != in) {
-                        used += v - in;
-                        in = v;
-                        d.seek(dv, e, env0 + e, 2u * (u32)v, 0u);
-                        if (multi)
-                            for (int w = 0; w < w32; w++) ob.set_word(w, st.word(w));
-                    }
+                const int exit_at = drained ? 1 : (__popc(hv) > 8 ? 2 * PBN_COOP_EXIT_AT : PBN_COOP_EXIT_AT);
+                const int v = coop_take_over<TQ, W1>(hv, nv, ev, dv, blob, att_off, cubes, sst, coop_buf, env0 + e, in, 0u, stop_in, exit_at);
+                if (v != in) {
+                    used += v - in;
+                    in = v;
+                    d.seek(dv, e, env0 + e, 2u * (u32)v, 0u);
+                    if (multi)
+                        for (int w = 0; w < w32; w++) ob.set_word(w, st.word(w));
                 }
-                __syncwarp();
             }
         }
     }
@@ -1364,13 +1345,13 @@ __global__ void __launch_bounds__(PBN_BLOCK, PBN_FIRST_MIN_BLOCKS) k_env_step_fi
     const bool valid = e < B;
     const bool multi = ev.kind == PBN_ENV_MULTI;
     Col st{sst + threadIdx.x}, ob{sst + w32 * PBN_BLOCK + threadIdx.x};
-    int pend = 0, bad = 0;
+    int pend = 0;
     if (valid) {
         load_state(st, state, B, e, w32);
         n_steps[e] += 1;
-        pend = att_begin(nv, ev, st, ob, actions + e * K, K, bad);
     }
-    __syncthreads();
+    __syncthreads();  // the images are staged and s_stats is zeroed before att_begin counts into it
+    if (valid) pend = att_begin(nv, ev, vx, s_stats, st, ob, actions + e * K, K);
     Draw<PBN_DRAW_PHILOX> dummy;
     const u32 c2 = (u32)(env0 + e), c3 = (u32)((u64)(env0 + e) >> 32);
     u32 x0 = 0, x1 = 0, x2 = 0, x3 = 0;
@@ -1447,27 +1428,12 @@ __global__ void __launch_bounds__(PBN_BLOCK, PBN_FIRST_MIN_BLOCKS) k_env_step_fi
         if (test(t + 1)) break;
         round(x2, x3, db);
     }
-    if (valid && run) {  // out of budget: park the env for a resume pass
-        store_state(st, state, B, e, w32);
-        inner_steps[e] = in;
-        reward[e] = pend;
-        pl.running[e] = 1;
-        pl.list_out[4 + atomicAdd(&pl.list_out[0], 1)] = (int)e;
-    } else if (valid) {
-        const Col &fo = (multi && in == 1) ? ob : st;  // MULTI: the observation is the state from the second update on
-        int rew, tm;
-        att_result(ev, att_off, cubes, st, fo, w32, target_att[e], pend, rew, tm);
-        store_state(st, state, B, e, w32);
-        if (obs_state) store_state(fo, obs_state, B, e, w32);
-        reward[e] = rew;
-        terminated[e] = (unsigned char)tm;
-        const int tr = (n_steps[e] == ev.horizon);
-        truncated[e] = (unsigned char)tr;
-        inner_steps[e] = in;
-        pl.running[e] = 0;
-        if (dv.used) { dv.used[2 * e] = 2 * in; dv.used[2 * e + 1] = 0; }
-        if (bad && vx.enabled) atomicAdd(&s_stats[6], 1ULL);
-        if (vx.enabled) vec_finish<PBN_DRAW_PHILOX>(nv, ev, vx, s_stats, state, n_steps, target_att, obs_state, B, e, env0, rew, tm, tr, in);
+    if (valid && run) {
+        att_park(pl, st, state, inner_steps, reward, B, e, w32, in, pend);
+    } else if (valid) {  // MULTI: the observation is the state from the second update on; an update takes two stream words
+        att_finish<PBN_DRAW_PHILOX>(nv, ev, dv, pl, vx, s_stats, att_off, cubes, st, (multi && in == 1) ? ob : st, state, n_steps,
+                                    target_att, obs_state, reward, terminated, truncated, inner_steps, B, e, env0, in, pend,
+                                    2u * (u32)in, 0u);
     }
     vec_flush_stats(vx, s_stats);
 }
@@ -1828,33 +1794,20 @@ __device__ __forceinline__ void ssd_loop(const SsdLoopArgs &a, const Col &st, Dr
                         }
                     }
                     if constexpr (NET == PBN_NET_PRED) {
-                        // straggler mode (see coop_run): the last chains of the warp inside their attractor loops are finished
-                        // by groups of lanes, all groups at once
+                        // straggler mode (as in k_env_step_att): the last chains of the warp inside their attractor loops are
+                        // finished by groups of lanes, all groups at once
                         const unsigned hv = __ballot_sync(0xFFFFFFFFu, live && !start && k < kk);
                         if (hv != 0u && __popc(__ballot_sync(0xFFFFFFFFu, active && k < kk)) <= PBN_COOP_MAX) {
-                            const int nl = __popc(hv);
-                            int kg = 1;
-                            while (kg < nl) kg <<= 1;
-                            const int g = 32 / kg, grp = (int)lane / g;
-                            const bool on = grp < nl;
-                            const int owner = on ? (int)__fns(hv, 0u, grp + 1) : 0;
-                            const long long idL = __shfl_sync(0xFFFFFFFFu, a.chain_id, owner);
-                            const int inL = __shfl_sync(0xFFFFFFFFu, in, owner);
-                            const u32 baseL = __shfl_sync(0xFFFFFFFFu, pos - (u32)in, owner);
-                            u32 *colL = a.sst + (threadIdx.x & ~31u) + (u32)owner;
-                            unsigned char *wb = a.coop_buf + (threadIdx.x >> 5) * coop_warp_bytes(w32);
-                            const int fin = w32 == 1 ? coop_steps<TQ, true>(nv, a.ev, a.dv, a.blob, a.att_off, a.cubes, colL, idL, inL, a.ev.max_inner, on, g, baseL, wb, 32)
-                                                     : coop_steps<TQ, false>(nv, a.ev, a.dv, a.blob, a.att_off, a.cubes, colL, idL, inL, a.ev.max_inner, on, g, baseL, wb, 32);
-                            __syncwarp();
-                            for (int r = 0; r < nl; r++) {
-                                const int v = __shfl_sync(0xFFFFFFFFu, fin, r * g);
-                                if ((int)lane == (int)__fns(hv, 0u, r + 1) && v != in) {
-                                    pos += (u32)(v - in);
-                                    in = v;
-                                    d.seek(a.dv, 0, a.chain_id, 2u * pos, 0u);  // later iterations go on drawing from this stream
-                                }
+                            const u32 base = pos - (u32)in;
+                            const int v = w32 == 1 ? coop_take_over<TQ, true>(hv, nv, a.ev, a.dv, a.blob, a.att_off, a.cubes, a.sst, a.coop_buf,
+                                                                              a.chain_id, in, base, a.ev.max_inner, 32)
+                                                   : coop_take_over<TQ, false>(hv, nv, a.ev, a.dv, a.blob, a.att_off, a.cubes, a.sst, a.coop_buf,
+                                                                               a.chain_id, in, base, a.ev.max_inner, 32);
+                            if (v != in) {
+                                pos += (u32)(v - in);
+                                in = v;
+                                d.seek(a.dv, 0, a.chain_id, 2u * pos, 0u);  // later iterations go on drawing from this stream
                             }
-                            __syncwarp();
                         }
                     }
                 }
@@ -2109,41 +2062,50 @@ extern "C" int pbn_rollout(const PbnNet *net, uint32_t *state, int64_t B, int64_
     return PBN_OK;
 }
 
+// Persistent grid of k_env_step_att: as many blocks as stay resident, each owning a contiguous range of envs (group mode: one
+// env per four lanes).  A resume pass learns its env count on the device; B only bounds it.
+static int att_grid(const void *kernel, size_t smem, long long B, bool grp_mode, long long &grid, long long &per_block) {
+    int dev = 0, sms = 0, bps = 0;
+    CK(cudaGetDevice(&dev));
+    CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, kernel, PBN_BLOCK, smem));
+    const int envs_per_block = grp_mode ? PBN_BLOCK / 4 : PBN_BLOCK;
+    grid = (long long)sms * (bps > 0 ? bps : 1);
+    if (grid > (B + envs_per_block - 1) / envs_per_block) grid = (B + envs_per_block - 1) / envs_per_block;
+    per_block = (B + grid - 1) / grid;
+    grid = (B + per_block - 1) / per_block;
+    return PBN_OK;
+}
+
 static int env_step_impl(const PbnEnv *env, uint32_t *state, int32_t *n_steps, const int32_t *target_att,
                          const int32_t *actions, int32_t K, uint32_t *obs_state, int32_t *reward, uint8_t *terminated,
                          uint8_t *truncated, int32_t *inner_steps, int64_t B, int64_t env0, const PbnDraws *draws,
                          const PbnVecState *vec, void *stream, double *reward_f64 = nullptr, const PbnStepPlan *plan = nullptr) {
     if (!env || !state || !actions || !reward || !terminated || !truncated || B < 0 || K < 1) return fail(PBN_ERR_ARG, "bad argument");
     if (!reward_f64 && vec && vec->reward_f64) reward_f64 = vec->reward_f64;
-    {
-        const int kd = env->v.kind;
-        if ((kd == PBN_ENV_PBN_ST || kd == PBN_ENV_PBCN_ST) && !reward_f64)
-            return fail(PBN_ERR_ARG, "self-triggering envs return a float64 reward: call pbn_env_step_f64");
-        if ((kd == PBN_ENV_PBN_ST && K != 2) || (kd == PBN_ENV_PBCN_ST && K != 1 + env->v.n_control))
-            return fail(PBN_ERR_ARG, "wrong action width for this env kind");
-    }
-    if ((env->v.kind == PBN_ENV_TARGET || env->v.kind == PBN_ENV_MULTI) && (!n_steps || !target_att))
-        return fail(PBN_ERR_ARG, "target envs need n_steps and target_att");
-    if ((env->v.kind == PBN_ENV_PBN_SD && K != 2) || (env->v.kind == PBN_ENV_PBCN_SD && K != 1 + env->v.n_control))
+    const EnvView &ev = env->v;
+    const bool att = ev.kind == PBN_ENV_TARGET || ev.kind == PBN_ENV_MULTI;
+    const bool st_kind = ev.kind == PBN_ENV_PBN_ST || ev.kind == PBN_ENV_PBCN_ST;
+    if (st_kind && !reward_f64) return fail(PBN_ERR_ARG, "self-triggering envs return a float64 reward: call pbn_env_step_f64");
+    if (((ev.kind == PBN_ENV_PBN_ST || ev.kind == PBN_ENV_PBN_SD) && K != 2) ||
+        ((ev.kind == PBN_ENV_PBCN_ST || ev.kind == PBN_ENV_PBCN_SD) && K != 1 + ev.n_control))
         return fail(PBN_ERR_ARG, "wrong action width for this env kind");
+    if (att && (!n_steps || !target_att)) return fail(PBN_ERR_ARG, "target envs need n_steps and target_att");
     if (int rc = check_draws(draws)) return rc;
     if (B == 0) return PBN_OK;
     const NetView &nv = env->net->v;
-    const EnvView &ev = env->v;
     const DrawView dv = make_draws(draws);
     VecView vx;
     memset(&vx, 0, sizeof vx);
     if (vec) {
-        const bool st_kind = ev.kind == PBN_ENV_PBN_ST || ev.kind == PBN_ENV_PBCN_ST;
         if (st_kind && (!vec->ep_return_f64 || !vec->return_sum_f64))
             return fail(PBN_ERR_ARG, "the vector step of a self-triggering env needs ep_return_f64 and return_sum_f64");
         if ((!st_kind && !vec->ep_return) || !vec->ep_len || !vec->stats || !obs_state) return fail(PBN_ERR_ARG, "vector step needs ep_return, ep_len, stats and obs_state");
         if (vec->autoreset) {
             if (int rc = check_draws(&vec->reset_draws)) return rc;
-            const bool tgt = ev.kind == PBN_ENV_TARGET || ev.kind == PBN_ENV_MULTI;
             if (ev.n_att < (ev.kind == PBN_ENV_TARGET ? 2 : 1)) return fail(PBN_ERR_ARG, "autoreset needs attractors");
-            if (!tgt && !env->has_small_att) return fail(PBN_ERR_ARG, "autoreset needs an attractor with at most 10 states (pbn_env.py:196-199)");
-            if (tgt && !vec->target_state) return fail(PBN_ERR_ARG, "autoreset of target envs needs target_state");
+            if (!att && !env->has_small_att) return fail(PBN_ERR_ARG, "autoreset needs an attractor with at most 10 states (pbn_env.py:196-199)");
+            if (att && !vec->target_state) return fail(PBN_ERR_ARG, "autoreset of target envs needs target_state");
             vx.rdv = make_draws(&vec->reset_draws);
         }
         vx.enabled = 1; vx.autoreset = vec->autoreset;
@@ -2159,7 +2121,6 @@ static int env_step_impl(const PbnEnv *env, uint32_t *state, int32_t *n_steps, c
     }
     const int block = block_for(B);
     const unsigned grid = (unsigned)((B + block - 1) / block);
-    const bool att = ev.kind == PBN_ENV_TARGET || ev.kind == PBN_ENV_MULTI;
     cudaStream_t s = (cudaStream_t)stream;
     PlanView pl;
     memset(&pl, 0, sizeof pl);
@@ -2170,7 +2131,6 @@ static int env_step_impl(const PbnEnv *env, uint32_t *state, int32_t *n_steps, c
         if (plan->budget < 0 || (plan->phase != 0 && plan->phase != 1)) return fail(PBN_ERR_ARG, "bad step plan");
         if (ev.kind == PBN_ENV_MULTI && plan->budget == 1) return fail(PBN_ERR_ARG, "MULTI envs need a budget of at least 2 updates");
         pl.budget = plan->budget; pl.resume = plan->resume != 0;
-        if (const char *dbg = getenv("PBN_PLAN_A")) pl.dbg_a = atoi(dbg);  // experiments: active warps per block of a resume pass
         pl.running = plan->running;
         pl.list_out = plan->work + (size_t)plan->phase * (size_t)(B + 4);
         pl.list_in = plan->work + (size_t)(plan->phase ^ 1) * (size_t)(B + 4);
@@ -2181,57 +2141,53 @@ static int env_step_impl(const PbnEnv *env, uint32_t *state, int32_t *n_steps, c
     const size_t coop_bytes = (size_t)(block / 32) * coop_warp_bytes(nv.w32);
     // a budgeted first pass has no tail to cut (every lane owns an env, nobody runs past the budget); images that leave no
     // room run without the group machinery as well
-    const int coop_on = att && smem + coop_bytes <= 200 * 1024 && !(plan && !pl.resume && pl.budget > 0);
+    const bool first_pass = plan && !pl.resume && pl.budget > 0;
+    const int coop_on = att && smem + coop_bytes <= 200 * 1024 && !first_pass;
     if (coop_on) smem += coop_bytes;
-    if (plan && !pl.resume && pl.budget > 0 && nv.kind == PBN_NET_PRED) {  // lockstep first pass (Philox: checked above)
+    // group mode pays when env.steps can be long; under a small cap a lane per env (4x the envs in flight) is faster
+    const int grp_mode = coop_on && nv.kind == PBN_NET_PRED && dv.mode == PBN_DRAW_PHILOX && ev.n_att > 0 && !ev.force &&
+                         (ev.max_inner > 64 || pl.resume);
+
+    // one launch function per kernel; the instantiation is picked below
+    auto launch_first = [&](auto kernel, size_t sm) -> int {
+        if (int rc = set_smem(kernel, sm)) return rc;
+        kernel<<<grid, block, sm, s>>>(nv, ev, dv, state, n_steps, const_cast<int32_t *>(target_att), actions, K, obs_state, reward,
+                                       terminated, truncated, inner_steps, B, env0, pl, vx);
+        return PBN_OK;
+    };
+    auto launch_att = [&](auto kernel) -> int {
+        if (int rc = set_smem(kernel, smem)) return rc;
+        long long pgrid = 0, per_block = 0;
+        if (int rc = att_grid((const void *)kernel, smem, B, grp_mode, pgrid, per_block)) return rc;
+        kernel<<<(unsigned)pgrid, block, smem, s>>>(nv, ev, dv, state, n_steps, target_att, actions, K, obs_state, reward,
+                                                   terminated, truncated, inner_steps, B, env0, per_block, coop_on, grp_mode, pl, vx);
+        return PBN_OK;
+    };
+    auto launch_step = [&](auto kernel) -> int {
+        const size_t smem1 = (size_t)nv.blob_bytes + ev.img_bytes + (size_t)nv.w32 * block * 4;  // one column per env
+        if (int rc = set_smem(kernel, smem1)) return rc;
+        kernel<<<grid, block, smem1, s>>>(nv, ev, dv, state, n_steps, target_att, actions, K, obs_state, reward, terminated,
+                                          truncated, inner_steps, B, env0, vx, reward_f64);
+        return PBN_OK;
+    };
+    int rc = PBN_OK;
+    if (first_pass && nv.kind == PBN_NET_PRED) {  // lockstep first pass (Philox: checked above)
         const bool fast = nv.off_rec16 != 0 && nv.w32 <= 8 && (nv.ts == 4 || nv.ts == 16);
         const size_t smem_f = (size_t)nv.blob_fast_bytes + ev.img_bytes + col_align_bytes(nv.w32) + (size_t)2 * nv.w32 * block * 4;
-#define FIRST(TQ, FAST, SM)                                                                                       \
-        if (int rc = set_smem(k_env_step_first<TQ, FAST>, SM)) return rc;                                         \
-        k_env_step_first<TQ, FAST><<<grid, block, SM, s>>>(nv, ev, dv, state, n_steps, const_cast<int32_t *>(target_att), actions, K, \
-                                                      obs_state, reward, terminated, truncated, inner_steps, B, env0, pl, vx)
-        if (fast && nv.ts == 4) { FIRST(1, true, smem_f); }
-        else if (fast) { FIRST(4, true, smem_f); }
-        else if (nv.ts == 4) { FIRST(1, false, smem); }
-        else if (nv.ts == 16) { FIRST(4, false, smem); }
-        else { FIRST(0, false, smem); }
-#undef FIRST
-        CK(cudaGetLastError());
-        return PBN_OK;
-    }
-#define ATT_LAUNCH(NK, MD, TQ, W1)                                                                                \
-        if (int rc = set_smem(k_env_step_att<NK, MD, TQ, W1>, smem)) return rc;                                   \
-        CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_env_step_att<NK, MD, TQ, W1>, block, smem));     \
-        att_grid();                                                                                               \
-        k_env_step_att<NK, MD, TQ, W1><<<(unsigned)pgrid, block, smem, s>>>(nv, ev, dv, state, n_steps, target_att, actions, K, obs_state, \
-                                                         reward, terminated, truncated, inner_steps, B, env0, per_block, coop_on, grp_mode, pl, vx)
-#define CALL(NK, MD, TQ)                                                                                          \
-    if (att) {                                                                                                    \
-        /* persistent grid: as many blocks as stay resident, each owning a contiguous range of envs */            \
-        int dev = 0, sms = 0, bps = 0;                                                                            \
-        CK(cudaGetDevice(&dev));                                                                                  \
-        CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));                                    \
-        long long pgrid = 0, per_block = 0;                                                                       \
-        /* group mode pays when env.steps can be long; under a small cap a lane per env (4x the envs in flight) is faster */ \
-        const int grp_mode = coop_on && NK == PBN_NET_PRED && MD == PBN_DRAW_PHILOX && ev.n_att > 0 && !ev.force && \
-                             (ev.max_inner > 64 || pl.resume);                                                    \
-        auto att_grid = [&]() {                                                                                   \
-            pgrid = (long long)sms * (bps > 0 ? bps : 1);                                                         \
-            const long long cap_grid = grp_mode ? (B + PBN_BLOCK / 4 - 1) / (PBN_BLOCK / 4) : (long long)grid;    \
-            if (pgrid > cap_grid) pgrid = cap_grid;  /* (a resume pass learns its env count on the device) */     \
-            per_block = (B + pgrid - 1) / pgrid;                                                                  \
-            pgrid = (B + per_block - 1) / per_block;                                                              \
-        };                                                                                                        \
-        if (NK == PBN_NET_PRED && MD == PBN_DRAW_PHILOX && nv.w32 == 1) { ATT_LAUNCH(NK, MD, TQ, true); }         \
-        else { ATT_LAUNCH(NK, MD, TQ, false); }                                                                   \
-    } else {                                                                                                      \
-        const size_t smem1 = (size_t)nv.blob_bytes + ev.img_bytes + (size_t)nv.w32 * block * 4; /* one column per env */ \
-        if (int rc = set_smem(k_env_step<NK, MD>, smem1)) return rc;                                              \
-        k_env_step<NK, MD><<<grid, block, smem1, s>>>(nv, ev, dv, state, n_steps, target_att, actions, K, obs_state, \
-                                                     reward, terminated, truncated, inner_steps, B, env0, vx, reward_f64); \
-    }
-    DISPATCH(nv.kind, dv.mode, att ? nv.ts : 0, CALL);
+        if (fast && nv.ts == 4) rc = launch_first(k_env_step_first<1, true>, smem_f);
+        else if (fast) rc = launch_first(k_env_step_first<4, true>, smem_f);
+        else if (nv.ts == 4) rc = launch_first(k_env_step_first<1, false>, smem);
+        else if (nv.ts == 16) rc = launch_first(k_env_step_first<4, false>, smem);
+        else rc = launch_first(k_env_step_first<0, false>, smem);
+    } else {
+#define CALL(NK, MD, TQ)                                                                                                   \
+        if (!att) rc = launch_step(k_env_step<NK, MD>);                                                                    \
+        else if (NK == PBN_NET_PRED && MD == PBN_DRAW_PHILOX && nv.w32 == 1) rc = launch_att(k_env_step_att<NK, MD, TQ, true>); \
+        else rc = launch_att(k_env_step_att<NK, MD, TQ, false>)
+        DISPATCH(nv.kind, dv.mode, att ? nv.ts : 0, CALL);
 #undef CALL
+    }
+    if (rc) return rc;
     CK(cudaGetLastError());
     return PBN_OK;
 }

@@ -214,9 +214,6 @@ __device__ __forceinline__ int coop_steps(const NetView &nv, const EnvView &ev, 
     unsigned live = __ballot_sync(0xFFFFFFFFu, running);
     for (;;) {
         // ---- phase A: 4g updates' worth of the stream, from the even update at or before position p
-#ifdef PBN_COOP_PROF
-        const long long t0 = clock64();
-#endif
         const u32 p = pos_base + (u32)in, u0 = p & 1u;
         {
             u32 x[PBN_COOP_NB][4];
@@ -245,17 +242,11 @@ __device__ __forceinline__ int coop_steps(const NetView &nv, const EnvView &ev, 
         if constexpr (!W1)
             for (int w = (int)sub; w < w32; w += g) sts_u32(ckp + 4u * w, lds_u32(col + 1024u * w));
         __syncwarp();
-#ifdef PBN_COOP_PROF
-        const long long t1 = clock64();
-#endif
         // ---- phase B
         int first;
         if (n_cubes <= g) first = coop_phase_b<W1, false, false>(ebuf, E, st, col, care0, val0, care1, val1, cc, cubes, n_cubes, w32, g, sub);
         else if (n_cubes <= 2 * g) first = coop_phase_b<W1, true, false>(ebuf, E, st, col, care0, val0, care1, val1, cc, cubes, n_cubes, w32, g, sub);
         else first = coop_phase_b<W1, true, true>(ebuf, E, st, col, care0, val0, care1, val1, cc, cubes, n_cubes, w32, g, sub);
-#ifdef PBN_COOP_PROF
-        const long long t2 = clock64();
-#endif
         // ---- stop entry: first match of any lane's cubes, or the entry at which the cap is reached
         int cap = stop_in - in;
         cap = (cap < 0 ? 0 : cap) + (int)u0;
@@ -296,11 +287,43 @@ __device__ __forceinline__ int coop_steps(const NetView &nv, const EnvView &ev, 
         n_stopped += __popc(live & ~now) >> (__ffs(g) - 1);  // whole groups leave together
         live = now;
         __syncwarp();  // every read of the batch's entries precedes the next batch's writes
-#ifdef PBN_COOP_PROF
-        if (blockIdx.x == 0 && threadIdx.x == 0 && in < 1200) printf("coop g=%d in=%d A=%lld B=%lld tail=%lld\n", g, in, t1 - t0, t2 - t1, clock64() - t2);
-#endif
         if (live == 0u || n_stopped >= exit_at) break;
     }
     if (W1 && active) *col_ptr = st;  // every lane of the group holds the same word
     return in;
+}
+
+// Hands the envs of the lanes in `hv` (a ballot of the warp) to lane groups, all at once: k groups of 32/k lanes, k the least
+// power of two >= the number of envs, group r on the env of the r-th lane of hv.  Every lane passes its own env's id, update count `in`, stream base
+// (coop_steps: pos_base) and stop_in; the owners' values are used.  sst: the block's state columns (lane l's at sst + l within
+// its warp), coop_buf: the block's staging, coop_warp_bytes(w32) per warp.  Returns the owner's new update count, and `in`
+// to every other lane.
+template <int TQ, bool W1>
+__device__ __forceinline__ int coop_take_over(unsigned hv, const NetView &nv, const EnvView &ev, const DrawView &dv,
+                                              const unsigned char *blob, const int *att_off, const u32 *cubes, u32 *sst,
+                                              unsigned char *coop_buf, long long id, int in, u32 base, int stop_in, int exit_at) {
+    const u32 lane = threadIdx.x & 31u;
+    const int nl = __popc(hv);
+    int k = 1;
+    while (k < nl) k <<= 1;
+    const int g = 32 / k;  // lanes per group
+    const int grp = (int)lane / g;
+    const bool on = grp < nl;
+    const int owner = on ? (int)__fns(hv, 0u, grp + 1) : 0;  // the grp-th lane of hv
+    const long long idL = __shfl_sync(0xFFFFFFFFu, id, owner);
+    const int inL = __shfl_sync(0xFFFFFFFFu, in, owner);
+    const u32 baseL = __shfl_sync(0xFFFFFFFFu, base, owner);
+    const int stopL = __shfl_sync(0xFFFFFFFFu, stop_in, owner);
+    u32 *colL = sst + (threadIdx.x & ~31u) + (u32)owner;
+    unsigned char *wb = coop_buf + (threadIdx.x >> 5) * coop_warp_bytes(nv.w32);
+    const int fin = coop_steps<TQ, W1>(nv, ev, dv, blob, att_off, cubes, colL, idL, inL, stopL, on, g, baseL, wb, exit_at);
+    __syncwarp();
+    int out = in;
+#pragma unroll 1  // (unrolled, its __fns calls add ~4 % to the kernel's code)
+    for (int r = 0; r < nl; r++) {  // each group's count back to the lane that owns the env
+        const int v = __shfl_sync(0xFFFFFFFFu, fin, r * g);
+        if ((int)lane == (int)__fns(hv, 0u, r + 1)) out = v;
+    }
+    __syncwarp();
+    return out;
 }

@@ -799,9 +799,11 @@ def test_vector_env_self_triggering_matches_oracle(tag):
     assert abs(float(vec.return_sum_f64) - ret_sum) < 1e-9 * max(1.0, abs(ret_sum))
 
 
-def test_vector_env_out_of_range_actions_are_ignored_and_counted():
+@pytest.mark.parametrize("plan", [None, (4, 16)])
+def test_vector_env_out_of_range_actions_are_ignored_and_counted(plan):
     """A policy network can emit anything: an action outside [0, N] must not touch another env's state column or the staged
-    network image; the intervention is dropped (the step equals action 0) and counted in the statistics."""
+    network image; the intervention is dropped (the step equals action 0) and counted in the statistics.  The planned step
+    counts it too for the envs its first pass parks (their intervention is not applied again when they resume)."""
     import gym_PBN
     from gym_PBN.b200.vector_env import PBNVectorEnv
 
@@ -810,6 +812,8 @@ def test_vector_env_out_of_range_actions_are_ignored_and_counted():
     env = gym_PBN.make("gym-PBN/Bittner-28-v0", all_attractors=atts, max_inner_steps=32)
     B, seed = 2048, 23
     vec_bad, vec_ok = PBNVectorEnv(env, B, seed=seed), PBNVectorEnv(env, B, seed=seed)
+    if plan is not None:
+        vec_bad.sim.plan_budgets = vec_ok.sim.plan_budgets = plan
     vec_bad.reset(), vec_ok.reset()
     rng = np.random.default_rng(3)
     n_bad = 0
