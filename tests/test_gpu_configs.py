@@ -6,7 +6,7 @@ torch = pytest.importorskip("torch")
 pytestmark = pytest.mark.gpu
 
 import oracle as orc  # noqa: E402
-from golden_util import cubes_to_attractors, load, synthetic_pbcn  # noqa: E402
+from golden_util import cubes_to_attractors, hittable_cubes, load, synthetic_pbcn  # noqa: E402
 
 
 @pytest.fixture(scope="module")
@@ -176,8 +176,14 @@ def test_step_plan_split_invariance(eng, name, kind, n_act, care, budgets):
             assert parked[0] > 0 and inner.max() > budgets[0]  # the split actually happened
 
 
-@pytest.mark.parametrize("name,kind,n_act", [("200_5_kmeans", "multi", 3), ("28_15_median", "target", 1)])
-def test_step_plan_two_lane_groups(eng, name, kind, n_act):
+@pytest.mark.parametrize("name,kind,n_act,n_cubes", [
+    pytest.param("200_5_kmeans", "multi", 3, 2, id="200_5_kmeans-multi-3"),
+    pytest.param("28_15_median", "target", 1, 2, id="28_15_median-target-1"),
+    # three and four cubes: the lanes of a two-lane group test cube sub + 2 as well (the TWO branch at g = 2)
+    pytest.param("28_15_median", "target", 1, 3, id="28_15_median-target-1-3cubes"),
+    pytest.param("200_5_kmeans", "multi", 3, 4, id="200_5_kmeans-multi-3-4cubes"),
+])
+def test_step_plan_two_lane_groups(eng, name, kind, n_act, n_cubes):
     """A resume pass whose list exceeds 8 envs per warp over the whole grid runs 16 envs per warp in groups of TWO lanes (envs
     with at most four cubes): same words, same result as the oracle's unsplit step."""
     net = eng.engine.Network(eng.compiler.load_bittner(name))
@@ -191,6 +197,8 @@ def test_step_plan_two_lane_groups(eng, name, kind, n_act):
         for i in rng.choice(n, size=n // 2 if n < 64 else 40, replace=False):
             c[i] = int(rng.integers(0, 2))
         atts.append([tuple(c)])
+    if n_cubes > 2:  # cubes 2 (and 3) are reachable ones (golden_util.hittable_cubes), in the second attractor
+        atts[1] += hittable_cubes(onet, n_cubes - 2, seed, care=5)
     multi = kind == "multi"
     env = eng.engine.EnvImage(net, eng.abi.ENV_MULTI if multi else eng.abi.ENV_TARGET, attractors=atts, horizon=100, max_inner=400, dedup=True)
     oenv = orc.Env(orc.ENV_MULTI if multi else orc.ENV_TARGET, n, attractors=atts, horizon=100, max_inner=400, dedup=1)
@@ -198,6 +206,7 @@ def test_step_plan_two_lane_groups(eng, name, kind, n_act):
     ost, ons, ota = np.zeros((B, n), np.uint8), np.zeros(B, np.int32), np.zeros(B, np.int32)
     sim.env_reset(env)
     orc.env_reset(onet, oenv, ost, ons, ota, orc.Draws(seed=seed, epoch=0))
+    cubes = np.array([[2 if v == "*" else v for v in c] for a in atts for c in a], np.int8)
     for t in range(2):
         act = rng.integers(0, n + 1, size=(B, n_act)).astype(np.int32)
         sim.env_step(env, torch.from_numpy(act), budget=2)
@@ -210,6 +219,10 @@ def test_step_plan_two_lane_groups(eng, name, kind, n_act):
         assert np.array_equal(sim.reward.cpu().numpy(), rew) and np.array_equal(sim.inner.cpu().numpy(), inner)
         assert np.array_equal(sim.terminated.cpu().numpy(), term) and np.array_equal(sim.truncated.cpu().numpy(), trunc)
         assert inner.max() == 400  # cap hits included
+        if n_cubes > 2:  # envs stopped by the loop on cube 2 or 3 alone: only the lanes' second cubes test those
+            stopped = (inner > 2) & (inner < 400)
+            match = [((obs[stopped] == c) | (c == 2)).all(1) for c in cubes]
+            assert (~match[0] & ~match[1] & (match[2] | match[-1])).sum() > 100
 
 
 def test_step_plan_matches_single_launch(eng):

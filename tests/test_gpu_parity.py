@@ -7,7 +7,7 @@ torch = pytest.importorskip("torch")
 pytestmark = pytest.mark.gpu
 
 import oracle as orc  # noqa: E402
-from golden_util import Traj, cubes_to_attractors, load, pbn_data_from  # noqa: E402
+from golden_util import Traj, cubes_to_attractors, load, pbn_data_from, random_predictor_net, random_tt_data  # noqa: E402
 
 
 @pytest.fixture(scope="module")
@@ -179,42 +179,17 @@ def test_golden_ssd_replay(eng):
 # ------------------------------------------------------------------------------------------------ Philox mode vs oracle
 def _nets(eng, which):
     if which == "tt":
-        rng = np.random.default_rng(5)
-        n = 70
-        pbn_data = []
-        for i in range(n):
-            k = int(rng.integers(0, 6))
-            mask = np.zeros(n, bool)
-            mask[rng.choice(n, size=k, replace=False)] = True
-            f1, f2 = rng.integers(0, 2, 2**k), rng.integers(0, 2, 2**k)
-            c = float(rng.uniform(0.05, 0.95))
-            pbn_data.append((mask, (c * f1 + (1 - c) * f2).reshape([2] * k), f"n{i}", k == 0))
+        pbn_data = random_tt_data(70, seed=5)
         return eng.engine.Network(eng.compiler.compile_pbn_data(pbn_data)), orc.net_from_pbn_data(pbn_data)
     sets, ids = orc.load_bittner(which)
     return eng.engine.Network(eng.compiler.load_bittner(which)), orc.net_from_predictor_sets(sets, ids)
-
-
-def _random_predictor_net(eng, n, fmax, seed):
-    """Synthetic predictor sets with 1..fmax predictors per node (the last column of some nodes empty, as add_to_buff leaves it)."""
-    rng = np.random.default_rng(seed)
-    ids = [1000 + 3 * i for i in range(n)]
-    sets = []
-    for i in range(n):
-        f = fmax if i == 0 else int(rng.integers(1, fmax + 1))
-        buf = np.empty((3, fmax), dtype=object)
-        others = [x for x in range(n) if x != i]
-        for k in range(f):
-            trio = rng.choice(others, 3, replace=False)
-            buf[0, k], buf[1, k], buf[2, k] = float(rng.uniform(0.05, 1.0)), rng.normal(size=(4, 1)), np.array([ids[t] for t in trio])
-        sets.append(buf)
-    return eng.engine.Network(eng.compiler.compile_predictor_sets(sets, ids)), orc.net_from_predictor_sets(sets, ids)
 
 
 @pytest.mark.parametrize("fmax", [1, 2, 5, 6, 9, 13, 17, 18, 23])
 def test_threshold_row_layouts(eng, fmax):
     """Predictor selection for every threshold-row layout: one quad (<= 5 predictors), leading quad + 2..4 quads (6..17),
     flat rows (more): rollout (async, sync) and SSD against the oracle."""
-    net, onet = _random_predictor_net(eng, 40, fmax, seed=fmax)
+    net, onet = random_predictor_net(eng, 40, fmax, seed=fmax)
     B, seed = 512, 77
     sim = eng.engine.Simulator(net, B, seed=seed, env0=64)
     sim.rand_state()
@@ -235,7 +210,7 @@ def test_threshold_row_layouts(eng, fmax):
 def test_fast_record_paths(eng, n, fmax):
     """The fast asynchronous paths read 16-byte predictor records from aligned state columns (1..8 words per column);
     networks whose records exceed 32 KB (200 nodes x 12 predictors) take the generic path.  Both against the oracle."""
-    net, onet = _random_predictor_net(eng, n, fmax, seed=n + fmax)
+    net, onet = random_predictor_net(eng, n, fmax, seed=n + fmax)
     B, seed = 300, 5
     sim = eng.engine.Simulator(net, B, seed=seed, env0=64)
     sim.rand_state()
