@@ -1452,6 +1452,26 @@ __global__ void __launch_bounds__(PBN_BLOCK) k_rand_state(NetView nv, DrawView d
     d.done(dv, e);
 }
 
+// Index of the first attractor with a cube containing each env's state, -1 if none: is_attracting_state (pbn_target.py:562-574)
+// as an index.  The cube image is staged into shared memory when it is small (staged = 1), else read from global memory.
+__global__ void __launch_bounds__(PBN_BLOCK) k_attractor_index(EnvView ev, int w32, const u32 *state, long long B, int *att_out,
+                                                               int staged) {
+    const unsigned char *img = staged ? smem_raw : ev.img;
+    u32 *sst = reinterpret_cast<u32 *>(smem_raw + (staged ? ev.img_bytes : 0));
+    if (staged) stage(smem_raw, ev.img, ev.img_bytes);
+    const int *att_off = reinterpret_cast<const int *>(img);
+    const u32 *cubes = reinterpret_cast<const u32 *>(img + ev.off_cubes);
+    const long long e = (long long)blockIdx.x * PBN_BLOCK + threadIdx.x;
+    Col st{sst + threadIdx.x};
+    if (e < B) load_state(st, state, B, e, w32);
+    __syncthreads();
+    if (e >= B) return;
+    int idx = -1;
+    for (int a = 0; a < ev.n_att && idx < 0; a++)
+        if (match_range(cubes, att_off[a], att_off[a + 1], st, w32)) idx = a;
+    att_out[e] = idx;
+}
+
 // ----------------------------------------------------------------------------------------------- K3 SSD
 struct SsdParams {
     int g;
@@ -2280,6 +2300,25 @@ extern "C" int pbn_rand_state(const PbnNet *net, uint32_t *state, int64_t B, int
     cudaStream_t s = (cudaStream_t)stream;
     if (dv.mode == PBN_DRAW_PHILOX) k_rand_state<PBN_DRAW_PHILOX><<<grid, block, 0, s>>>(net->v, dv, state, B, env0);
     else k_rand_state<PBN_DRAW_REPLAY><<<grid, block, 0, s>>>(net->v, dv, state, B, env0);
+    CK(cudaGetLastError());
+    return PBN_OK;
+}
+
+extern "C" int pbn_env_attractor_index(const PbnEnv *env, const uint32_t *state, int64_t B, int32_t *att_out, void *stream) {
+    if (!env || !state || !att_out || B < 0) return fail(PBN_ERR_ARG, "bad argument");
+    const EnvView &ev = env->v;
+    if (ev.n_att < 1) return fail(PBN_ERR_ARG, "the env has no attractor list");
+    if (B == 0) return PBN_OK;
+    const int w32 = env->net->v.w32;
+    const int block = block_for(B);
+    const unsigned grid = (unsigned)((B + block - 1) / block);
+    const size_t cols = (size_t)w32 * block * 4;
+    // staged only while three blocks stay resident per SM: the kernel is one pass over the states, and a large cube list
+    // read by every thread of a block is served from L1 as well
+    const int staged = (size_t)ev.img_bytes + cols <= 64 * 1024;
+    const size_t smem = cols + (staged ? (size_t)ev.img_bytes : 0);
+    if (int rc = set_smem(k_attractor_index, smem)) return rc;
+    k_attractor_index<<<grid, block, smem, (cudaStream_t)stream>>>(ev, w32, state, B, att_out, staged);
     CK(cudaGetLastError());
     return PBN_OK;
 }

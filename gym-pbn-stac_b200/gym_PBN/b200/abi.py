@@ -78,6 +78,7 @@ EXPORTS = {
                                 C.c_int64, C.POINTER(PbnDraws), C.c_void_p]),
     "pbn_env_reset_cur": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                     C.c_int32, C.c_int64, C.c_int64, C.POINTER(PbnDraws), C.c_void_p]),
+    "pbn_env_attractor_index": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]),
     "pbn_rand_state": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.POINTER(PbnDraws), C.c_void_p]),
     "pbn_ssd": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_double,
                           C.c_void_p, C.c_int32, C.c_void_p, C.POINTER(PbnDraws), C.c_void_p]),

@@ -455,6 +455,26 @@ def bucket_hist(sim: "Simulator", tgt_nodes, hist):
     return hist
 
 
+def attractor_index(sim_or_state, env_image: EnvImage, out=None):
+    """int32 [B] device tensor: index of the first attractor of `env_image` with a cube containing each env's state, -1 if
+    none.  sim_or_state: a Simulator (its live state) or packed state planes int32 [W32][B] on the image's device."""
+    state = sim_or_state.state if isinstance(sim_or_state, Simulator) else sim_or_state
+    net = env_image.net
+    if state.dim() != 2 or state.shape[0] != net.w32 or state.dtype != torch.int32 or state.device != net.device:
+        raise ValueError(f"state must be int32 planes [{net.w32}][B] on {net.device}")
+    state = state.contiguous()
+    B = state.shape[1]
+    if out is None:
+        out = torch.empty(B, dtype=torch.int32, device=net.device)
+    elif out.shape != (B,) or out.dtype != torch.int32 or out.device != net.device or not out.is_contiguous():
+        raise ValueError(f"out must be a contiguous int32 tensor [{B}] on {net.device}")
+    with on_device(net.device):
+        abi.check(abi.lib().pbn_env_attractor_index(env_image.handle, _ptr(state), B, _ptr(out), _stream()))
+    if isinstance(sim_or_state, Simulator):
+        sim_or_state.launches += 1
+    return out
+
+
 def issue_peak(kind, iters=2000):
     """(ops/s) of the instruction-issue microbenchmarks: kind 0 = INT ALU ops, kind 1 = Philox4x32-10 blocks."""
     ms, ops = C.c_float(), C.c_double()

@@ -211,6 +211,10 @@ int pbn_env_reset_cur(const PbnEnv *env, uint32_t *state, int32_t *n_steps, int3
                       const uint8_t *mask, double *probabilities, int32_t *pair_ids, int32_t sample_pair, int64_t B,
                       int64_t env0, const PbnDraws *draws, void *stream);
 
+/* att_out[e] = index of the first attractor that has a cube containing state e, -1 if none (pbn_target.py:562-574,
+   is_attracting_state, as an index).  state: planes [W32][B].  PBN_ERR_ARG when the env has no attractor list. */
+int pbn_env_attractor_index(const PbnEnv *env, const uint32_t *state, int64_t B, int32_t *att_out, void *stream);
+
 /* Graph.genRandState base.py:368-370 */
 int pbn_rand_state(const PbnNet *net, uint32_t *state, int64_t B, int64_t env0, const PbnDraws *draws, void *stream);
 
