@@ -8,7 +8,7 @@ from pathlib import Path
 HERE = Path(__file__).resolve().parent
 ROOT = HERE.parent
 SRC = [HERE / "csrc" / "pbn_b200.cu", HERE / "csrc" / "pbn_fit.cu"]
-DEPS = SRC + [HERE / "csrc" / "pbn_device.cuh", HERE / "csrc" / "pbn_fit.cuh", HERE / "csrc" / "pbn_coop.cuh", ROOT / "include" / "pbn_b200.h"]
+DEPS = SRC + [HERE / "csrc" / "pbn_device.cuh", HERE / "csrc" / "pbn_fit.cuh", HERE / "csrc" / "pbn_coop.cuh", HERE / "csrc" / "pbn_smem.cuh", ROOT / "include" / "pbn_b200.h"]
 LIB = HERE / "lib" / "libpbn_b200.so"
 
 NVCC_FLAGS = [

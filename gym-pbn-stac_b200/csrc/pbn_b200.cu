@@ -10,6 +10,7 @@
 #include <map>
 #include <mutex>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "pbn_device.cuh"
@@ -20,11 +21,15 @@ static int fail(int code, const std::string &msg) {
     g_err = msg;
     return code;
 }
+// A failed runtime call also stays the thread's last error; it is consumed here, so that it cannot surface as the failure of a
+// later call's cudaGetLastError().
 #define CK(call)                                                                                     \
     do {                                                                                             \
         cudaError_t e_ = (call);                                                                     \
-        if (e_ != cudaSuccess)                                                                       \
+        if (e_ != cudaSuccess) {                                                                     \
+            cudaGetLastError();                                                                      \
             return fail(PBN_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(e_));           \
+        }                                                                                            \
     } while (0)
 
 int pbn_fail_(int code, const std::string &msg) { return fail(code, msg); }  // for the other translation units
@@ -387,6 +392,7 @@ __device__ __forceinline__ void ssd_fast_update(const SsdFast &f, u32 wa, u32 wb
 }
 
 #include "pbn_coop.cuh"
+#include "pbn_smem.cuh"
 
 // the state half of an update, predicated (`on`) and reporting the old and the new word — for callers that track the state
 // incrementally (the lockstep first pass of the step-until-attractor envs keeps per-cube mismatch counts)
@@ -427,9 +433,9 @@ template <int NET, int MODE, int TQ>
 __global__ void __launch_bounds__(PBN_BLOCK) k_rollout(NetView nv, DrawView dv, u32 *state, long long B, long long env0,
                                                        long long steps, int sync) {
     unsigned char *blob = smem_raw;
-    const int bb = sync ? nv.blob_bytes : nv.blob_fast_bytes;  // asynchronous rollouts also stage the 16-byte records
-    u32 *sst = align_cols(reinterpret_cast<u32 *>(smem_raw + bb), nv.w32);
-    stage(blob, nv.blob, bb);
+    const RolloutSmem L = rollout_smem(nv, sync);
+    u32 *sst = align_cols(reinterpret_cast<u32 *>(smem_raw + L.cols), nv.w32);
+    stage(blob, nv.blob, L.image);
     const long long e = (long long)blockIdx.x * PBN_BLOCK + threadIdx.x;
     Col st{sst + threadIdx.x};
     Col tmp{sst + nv.w32 * PBN_BLOCK + threadIdx.x};
@@ -706,10 +712,11 @@ __global__ void __launch_bounds__(PBN_BLOCK) k_sync_sliced(NetView nv, DrawView 
     const int n = nv.n, fmax = nv.fmax, w32 = nv.w32;
     const int npad = w32 * 32;
     unsigned char *blob = smem_raw;
-    u32 *lm = reinterpret_cast<u32 *>(smem_raw + nv.blob_bytes);
+    const SlicedSmem L = sliced_smem(nv);
+    u32 *lm = reinterpret_cast<u32 *>(smem_raw + L.lm);
     const int lrow = fmax * 16 + 4;
-    u32 *words = lm + (size_t)n * lrow;  // [8 warps][2][npad]
-    stage(blob, nv.blob, nv.blob_bytes);
+    u32 *words = reinterpret_cast<u32 *>(smem_raw + L.words);  // [8 warps][2][npad]
+    stage(blob, nv.blob, L.image);
     {
         const uint4 *src = reinterpret_cast<const uint4 *>(nv.lutmask);
         uint4 *dst = reinterpret_cast<uint4 *>(lm);
@@ -901,10 +908,11 @@ __global__ void __launch_bounds__(PBN_BLOCK, 4) k_env_step(NetView nv, EnvView e
     resolve_epoch(dv);
     resolve_epoch(vx.rdv);
     unsigned char *blob = smem_raw;
-    unsigned char *img = smem_raw + nv.blob_bytes;
-    u32 *sst = reinterpret_cast<u32 *>(img + ev.img_bytes);
+    const EnvSmem L = env_smem(nv, ev, 1, false, false);
+    unsigned char *img = smem_raw + L.img;
+    u32 *sst = reinterpret_cast<u32 *>(smem_raw + L.cols);
     __shared__ unsigned long long s_stats[8];
-    stage(blob, nv.blob, nv.blob_bytes);
+    stage(blob, nv.blob, L.image);
     stage(img, ev.img, ev.img_bytes);
     if (threadIdx.x < 8) s_stats[threadIdx.x] = 0;
     const int *att_off = reinterpret_cast<const int *>(img);
@@ -1160,13 +1168,14 @@ __global__ void __launch_bounds__(PBN_BLOCK, 2) k_env_step_att(NetView nv, EnvVi
     resolve_epoch(dv);
     resolve_epoch(vx.rdv);
     unsigned char *blob = smem_raw;
-    unsigned char *img = smem_raw + nv.blob_bytes;
-    u32 *sst = reinterpret_cast<u32 *>(img + ev.img_bytes);
+    const EnvSmem L = env_smem(nv, ev, 2, false, coop_on);
+    unsigned char *img = smem_raw + L.img;
+    u32 *sst = reinterpret_cast<u32 *>(smem_raw + L.cols);
     const int w32 = nv.w32;
-    unsigned char *coop_buf = reinterpret_cast<unsigned char *>(sst + 2 * w32 * PBN_BLOCK);  // straggler-mode staging, per warp
+    unsigned char *coop_buf = reinterpret_cast<unsigned char *>(sst + L.coop);  // straggler-mode staging, per warp
     __shared__ int s_next;
     __shared__ unsigned long long s_stats[8];
-    stage(blob, nv.blob, nv.blob_bytes);
+    stage(blob, nv.blob, L.image);
     stage(img, ev.img, ev.img_bytes);
     if (threadIdx.x < 8) s_stats[threadIdx.x] = 0;
     const int *att_off = reinterpret_cast<const int *>(img);
@@ -1330,13 +1339,13 @@ __global__ void __launch_bounds__(PBN_BLOCK, PBN_FIRST_MIN_BLOCKS) k_env_step_fi
     resolve_epoch(dv);
     resolve_epoch(vx.rdv);
     unsigned char *blob = smem_raw;
-    const int bb = FAST ? nv.blob_fast_bytes : nv.blob_bytes;
-    unsigned char *img = smem_raw + bb;
+    const EnvSmem L = env_smem(nv, ev, 2, FAST, false);
+    unsigned char *img = smem_raw + L.img;
     const int w32 = nv.w32;
-    u32 *sst = reinterpret_cast<u32 *>(img + ev.img_bytes);
+    u32 *sst = reinterpret_cast<u32 *>(smem_raw + L.cols);
     if (FAST) sst = align_cols(sst, w32);
     __shared__ unsigned long long s_stats[8];
-    stage(blob, nv.blob, bb);
+    stage(blob, nv.blob, L.image);
     stage(img, ev.img, ev.img_bytes);
     if (threadIdx.x < 8) s_stats[threadIdx.x] = 0;
     const int *att_off = reinterpret_cast<const int *>(img);
@@ -1457,7 +1466,7 @@ __global__ void __launch_bounds__(PBN_BLOCK) k_rand_state(NetView nv, DrawView d
 __global__ void __launch_bounds__(PBN_BLOCK) k_attractor_index(EnvView ev, int w32, const u32 *state, long long B, int *att_out,
                                                                int staged) {
     const unsigned char *img = staged ? smem_raw : ev.img;
-    u32 *sst = reinterpret_cast<u32 *>(smem_raw + (staged ? ev.img_bytes : 0));
+    u32 *sst = reinterpret_cast<u32 *>(smem_raw + index_smem(ev, w32, staged).cols);
     if (staged) stage(smem_raw, ev.img, ev.img_bytes);
     const int *att_off = reinterpret_cast<const int *>(img);
     const u32 *cubes = reinterpret_cast<const u32 *>(img + ev.off_cubes);
@@ -1473,17 +1482,6 @@ __global__ void __launch_bounds__(PBN_BLOCK) k_attractor_index(EnvView ev, int w
 }
 
 // ----------------------------------------------------------------------------------------------- K3 SSD
-struct SsdParams {
-    int g;
-    int smem_hist;  // 1: per-block shared histogram (g <= 12), 0: global atomics
-    int fast_t0;    // >= 0: the targets are nodes t0, t0+1, .. t0+g-1 inside one state word (bucket = bit-reversed field)
-    int win;        // iterations per window of the step-until-attractor path (0 = iteration by iteration)
-    float inv;      // 1/log2(1-p) <= 0; a value > 0 means flips disabled (p == 0)
-    float gdelta;   // margin of the lg2.approx shortcut of the gap draw (geom_gap_approx); >= 0.5: shortcut off
-    double p;
-    short tgt[24];
-};
-
 // bucket = target-node bits, first target = most significant (pbn_target.py:383-391)
 __device__ __forceinline__ int ssd_bucket(const SsdParams &sp, const u32 *s_tgt, const Col &st) {
     if (sp.fast_t0 >= 0) {
@@ -1873,14 +1871,15 @@ __global__ void __launch_bounds__(PBN_BLOCK, HAS_ENV ? 3 : PBN_SSD_MIN_BLOCKS) k
                                                    long long chains, long long env0, int iters,
                                                    unsigned long long *hist) {
     unsigned char *blob = smem_raw;
-    const int bb = HAS_ENV ? nv.blob_bytes : nv.blob_fast_bytes;  // the all-attracting paths also stage the 16-byte records
-    unsigned char *img = smem_raw + bb;
-    const int img_bytes = HAS_ENV ? ev.img_bytes : 0;
-    u32 *s_tgt = reinterpret_cast<u32 *>(img + img_bytes);
-    u32 *shist = s_tgt + 32;
+    const SsdSmem L = ssd_smem(nv, ev, sp, HAS_ENV);
+    unsigned char *img = smem_raw + L.img;
+    u32 *s_tgt = reinterpret_cast<u32 *>(smem_raw + L.tgt);
+    u32 *shist = reinterpret_cast<u32 *>(smem_raw + L.hist);
     const int nb = 1 << sp.g;
+    // the columns (L.cols) addressed from the histogram: from smem_raw + L.cols, ptxas allocates the SSD loops' registers
+    // differently (other register counts and spill sizes in several instantiations)
     u32 *sst = align_cols(shist + (sp.smem_hist ? nb : 0), nv.w32);
-    stage(blob, nv.blob, bb);
+    stage(blob, nv.blob, L.image);
     if (HAS_ENV) stage(img, ev.img, ev.img_bytes);
     if (threadIdx.x == 0) {
 #pragma unroll
@@ -1894,8 +1893,8 @@ __global__ void __launch_bounds__(PBN_BLOCK, HAS_ENV ? 3 : PBN_SSD_MIN_BLOCKS) k
     const int w32 = nv.w32;
     Col st{sst + threadIdx.x};
     const int win = sp.win;
-    u32 *flipbuf = (HAS_ENV && win > 0) ? sst + w32 * PBN_BLOCK : nullptr;
-    unsigned char *coop_buf = flipbuf ? reinterpret_cast<unsigned char *>(flipbuf + (PBN_BLOCK / 32) * win * w32 * 32) : nullptr;
+    u32 *flipbuf = (HAS_ENV && win > 0) ? sst + L.flip : nullptr;
+    unsigned char *coop_buf = flipbuf ? reinterpret_cast<unsigned char *>(flipbuf + L.coop) : nullptr;
     const bool active = e < chains;
     if (active) load_state(st, state, chains, e, w32);
     __syncthreads();
@@ -2020,25 +2019,40 @@ extern "C" int pbn_issue_peak(int32_t kind, int64_t iters, float *ms_out, double
 }
 
 // ----------------------------------------------------------------------------------------------- launch glue
+// A launch's dynamic shared memory (its layout's bytes) against what a block of `kernel` may have: the device's opt-in maximum
+// less the kernel's static shared memory.  A layout that does not fit is refused and nothing is launched.
 template <class K>
-static int set_smem(K kernel, size_t bytes) {
-    // static + dynamic shared memory above 48 KB needs the opt-in; kernels carry up to 2 KB of static shared memory
-    if (bytes > 46 * 1024) CK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
+static int fit_smem(K kernel, const char *name, size_t bytes) {
+    int dev = 0, optin = 0;
+    cudaFuncAttributes fa;
+    CK(cudaGetDevice(&dev));
+    CK(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+    CK(cudaFuncGetAttributes(&fa, kernel));
+    const size_t avail = (size_t)optin - fa.sharedSizeBytes;
+    if (bytes > avail)
+        return fail(PBN_ERR_UNSUPPORTED, std::string(name) + " needs " + std::to_string(bytes) +
+                                             " bytes of shared memory per block; the device allows " + std::to_string(avail));
+    // static + dynamic shared memory above 48 KB needs the opt-in
+    if (fa.sharedSizeBytes + bytes > 48 * 1024) CK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
     return PBN_OK;
 }
-static inline int block_for(long long) { return PBN_BLOCK; }  // columns use a compile-time word stride of PBN_BLOCK
 
-// kernels are instantiated per (network kind, draw source, threshold quads TQ); TQ = 1 covers predictor sets with
-// up to 5 predictors per node (every shipped *_5_* set), TQ = 4 up to 17 (the 28_15 set), TQ = 0 reads the count at run time
-#define DISPATCH(NETKIND, MODE, TS, CALL)                                                        \
-    do {                                                                                         \
-        if ((NETKIND) == PBN_NET_PRED && (MODE) == PBN_DRAW_PHILOX && (TS) == 4) { CALL(PBN_NET_PRED, PBN_DRAW_PHILOX, 1); } \
-        else if ((NETKIND) == PBN_NET_PRED && (MODE) == PBN_DRAW_PHILOX && (TS) == 16) { CALL(PBN_NET_PRED, PBN_DRAW_PHILOX, 4); } \
-        else if ((NETKIND) == PBN_NET_PRED && (MODE) == PBN_DRAW_PHILOX) { CALL(PBN_NET_PRED, PBN_DRAW_PHILOX, 0); }         \
-        else if ((NETKIND) == PBN_NET_PRED) { CALL(PBN_NET_PRED, PBN_DRAW_REPLAY, 0); }          \
-        else if ((MODE) == PBN_DRAW_PHILOX) { CALL(PBN_NET_TT, PBN_DRAW_PHILOX, 0); }            \
-        else { CALL(PBN_NET_TT, PBN_DRAW_REPLAY, 0); }                                           \
-    } while (0)
+// Kernels are instantiated per (network kind, draw source, threshold quads TQ); TQ = 1 covers predictor sets with up to 5
+// predictors per node (every shipped *_5_* set), TQ = 4 up to 17 (the 28_15 set), TQ = 0 reads the count at run time.
+// f(NK, MD, TQ) gets the three as std::integral_constant, usable as template arguments.
+template <int V>
+using Ic = std::integral_constant<int, V>;
+template <class F>
+static int dispatch(int kind, int mode, int ts, F &&f) {
+    if (kind == PBN_NET_PRED && mode == PBN_DRAW_PHILOX) {
+        if (ts == 4) return f(Ic<PBN_NET_PRED>(), Ic<PBN_DRAW_PHILOX>(), Ic<1>());
+        if (ts == 16) return f(Ic<PBN_NET_PRED>(), Ic<PBN_DRAW_PHILOX>(), Ic<4>());
+        return f(Ic<PBN_NET_PRED>(), Ic<PBN_DRAW_PHILOX>(), Ic<0>());
+    }
+    if (kind == PBN_NET_PRED) return f(Ic<PBN_NET_PRED>(), Ic<PBN_DRAW_REPLAY>(), Ic<0>());
+    if (mode == PBN_DRAW_PHILOX) return f(Ic<PBN_NET_TT>(), Ic<PBN_DRAW_PHILOX>(), Ic<0>());
+    return f(Ic<PBN_NET_TT>(), Ic<PBN_DRAW_REPLAY>(), Ic<0>());
+}
 
 static int check_draws(const PbnDraws *d) {
     if (!d) return fail(PBN_ERR_ARG, "draws is null");
@@ -2054,7 +2068,6 @@ extern "C" int pbn_rollout(const PbnNet *net, uint32_t *state, int64_t B, int64_
     if (B == 0 || steps == 0) return PBN_OK;
     const NetView &nv = net->v;
     const DrawView dv = make_draws(draws);
-    const int block = block_for(B);
     cudaStream_t s = (cudaStream_t)stream;
     if (sync == 2) {  // bit-sliced synchronous mode
         if (nv.kind != PBN_NET_PRED || !nv.lutmask || nv.ts != 4)
@@ -2062,24 +2075,23 @@ extern "C" int pbn_rollout(const PbnNet *net, uint32_t *state, int64_t B, int64_
         if (dv.mode != PBN_DRAW_PHILOX) return fail(PBN_ERR_UNSUPPORTED, "bit-sliced synchronous mode has no replay source (use sync=1)");
         if (env0 & 31) return fail(PBN_ERR_ARG, "env0 must be a multiple of 32: a group of 32 consecutive env ids shares the random words");
         if (steps >= (1 << 20)) return fail(PBN_ERR_ARG, "at most 2^20 steps per launch");
-        const size_t sm = (size_t)nv.blob_bytes + (size_t)nv.n * (nv.fmax * 16 + 4) * 4 + (size_t)(PBN_BLOCK / 32) * 2 * nv.w32 * 32 * 4;
+        const size_t sm = sliced_smem(nv).bytes;
         if (sm > 200 * 1024) return fail(PBN_ERR_UNSUPPORTED, "network too large for the bit-sliced tables");
-        if (int rc = set_smem(k_sync_sliced, sm)) return rc;
+        if (int rc = fit_smem(k_sync_sliced, "k_sync_sliced", sm)) return rc;
         const long long groups = (B + 31) / 32;
         const unsigned g2 = (unsigned)((groups + PBN_BLOCK / 32 - 1) / (PBN_BLOCK / 32));
         k_sync_sliced<<<g2, PBN_BLOCK, sm, s>>>(nv, dv, state, B, env0, (int)steps);
         CK(cudaGetLastError());
         return PBN_OK;
     }
-    const unsigned grid = (unsigned)((B + block - 1) / block);
-    const size_t smem = (size_t)(sync ? nv.blob_bytes : nv.blob_fast_bytes) + col_align_bytes(nv.w32) + (size_t)2 * nv.w32 * PBN_BLOCK * 4;
-#define CALL(NK, MD, TQ)                                                           \
-    if (int rc = set_smem(k_rollout<NK, MD, TQ>, smem)) return rc;                 \
-    k_rollout<NK, MD, TQ><<<grid, block, smem, s>>>(nv, dv, state, B, env0, steps, sync)
-    DISPATCH(nv.kind, dv.mode, nv.ts, CALL);
-#undef CALL
-    CK(cudaGetLastError());
-    return PBN_OK;
+    const unsigned grid = (unsigned)((B + PBN_BLOCK - 1) / PBN_BLOCK);
+    const size_t smem = rollout_smem(nv, sync).bytes;
+    return dispatch(nv.kind, dv.mode, nv.ts, [&](auto NK, auto MD, auto TQ) {
+        if (int rc = fit_smem(k_rollout<NK, MD, TQ>, "k_rollout", smem)) return rc;
+        k_rollout<NK, MD, TQ><<<grid, PBN_BLOCK, smem, s>>>(nv, dv, state, B, env0, steps, sync);
+        CK(cudaGetLastError());
+        return PBN_OK;
+    });
 }
 
 // Persistent grid of k_env_step_att: as many blocks as stay resident, each owning a contiguous range of envs (group mode: one
@@ -2139,8 +2151,7 @@ static int env_step_impl(const PbnEnv *env, uint32_t *state, int32_t *n_steps, c
             vx.cur.prob = vec->probabilities; vx.cur.pair = vec->pair_ids; vx.cur.sample_pair = vec->sample_pair != 0;
         }
     }
-    const int block = block_for(B);
-    const unsigned grid = (unsigned)((B + block - 1) / block);
+    const unsigned grid = (unsigned)((B + PBN_BLOCK - 1) / PBN_BLOCK);
     cudaStream_t s = (cudaStream_t)stream;
     PlanView pl;
     memset(&pl, 0, sizeof pl);
@@ -2156,57 +2167,53 @@ static int env_step_impl(const PbnEnv *env, uint32_t *state, int32_t *n_steps, c
         pl.list_in = plan->work + (size_t)(plan->phase ^ 1) * (size_t)(B + 4);
         CK(cudaMemsetAsync(pl.list_out, 0, 16, s));
     }
-    // two columns per env + (step-until-attractor kernel) the per-warp staging of its straggler mode
-    size_t smem = (size_t)nv.blob_bytes + ev.img_bytes + (size_t)2 * nv.w32 * block * 4;
-    const size_t coop_bytes = (size_t)(block / 32) * coop_warp_bytes(nv.w32);
     // a budgeted first pass has no tail to cut (every lane owns an env, nobody runs past the budget); images that leave no
-    // room run without the group machinery as well
+    // room run without the group machinery (the per-warp staging of the straggler mode) as well
     const bool first_pass = plan && !pl.resume && pl.budget > 0;
-    const int coop_on = att && smem + coop_bytes <= 200 * 1024 && !first_pass;
-    if (coop_on) smem += coop_bytes;
+    const int coop_on = att && env_smem(nv, ev, 2, false, true).bytes <= 200 * 1024 && !first_pass;
     // group mode pays when env.steps can be long; under a small cap a lane per env (4x the envs in flight) is faster
     const int grp_mode = coop_on && nv.kind == PBN_NET_PRED && dv.mode == PBN_DRAW_PHILOX && ev.n_att > 0 && !ev.force &&
                          (ev.max_inner > 64 || pl.resume);
+    // the lockstep first pass of predictor networks takes the fast-path update where the records and the state width allow it
+    const bool fast = nv.off_rec16 != 0 && nv.w32 <= 8 && (nv.ts == 4 || nv.ts == 16);
 
     // one launch function per kernel; the instantiation is picked below
-    auto launch_first = [&](auto kernel, size_t sm) -> int {
-        if (int rc = set_smem(kernel, sm)) return rc;
-        kernel<<<grid, block, sm, s>>>(nv, ev, dv, state, n_steps, const_cast<int32_t *>(target_att), actions, K, obs_state, reward,
-                                       terminated, truncated, inner_steps, B, env0, pl, vx);
+    auto launch_first = [&](auto kernel, bool fst) -> int {
+        const size_t sm = env_smem(nv, ev, 2, fst, false).bytes;
+        if (int rc = fit_smem(kernel, "k_env_step_first", sm)) return rc;
+        kernel<<<grid, PBN_BLOCK, sm, s>>>(nv, ev, dv, state, n_steps, const_cast<int32_t *>(target_att), actions, K, obs_state,
+                                           reward, terminated, truncated, inner_steps, B, env0, pl, vx);
         return PBN_OK;
     };
     auto launch_att = [&](auto kernel) -> int {
-        if (int rc = set_smem(kernel, smem)) return rc;
+        const size_t sm = env_smem(nv, ev, 2, false, coop_on).bytes;
+        if (int rc = fit_smem(kernel, "k_env_step_att", sm)) return rc;
         long long pgrid = 0, per_block = 0;
-        if (int rc = att_grid((const void *)kernel, smem, B, grp_mode, pgrid, per_block)) return rc;
-        kernel<<<(unsigned)pgrid, block, smem, s>>>(nv, ev, dv, state, n_steps, target_att, actions, K, obs_state, reward,
-                                                   terminated, truncated, inner_steps, B, env0, per_block, coop_on, grp_mode, pl, vx);
+        if (int rc = att_grid((const void *)kernel, sm, B, grp_mode, pgrid, per_block)) return rc;
+        kernel<<<(unsigned)pgrid, PBN_BLOCK, sm, s>>>(nv, ev, dv, state, n_steps, target_att, actions, K, obs_state, reward,
+                                                     terminated, truncated, inner_steps, B, env0, per_block, coop_on, grp_mode, pl, vx);
         return PBN_OK;
     };
     auto launch_step = [&](auto kernel) -> int {
-        const size_t smem1 = (size_t)nv.blob_bytes + ev.img_bytes + (size_t)nv.w32 * block * 4;  // one column per env
-        if (int rc = set_smem(kernel, smem1)) return rc;
-        kernel<<<grid, block, smem1, s>>>(nv, ev, dv, state, n_steps, target_att, actions, K, obs_state, reward, terminated,
-                                          truncated, inner_steps, B, env0, vx, reward_f64);
+        const size_t sm = env_smem(nv, ev, 1, false, false).bytes;
+        if (int rc = fit_smem(kernel, "k_env_step", sm)) return rc;
+        kernel<<<grid, PBN_BLOCK, sm, s>>>(nv, ev, dv, state, n_steps, target_att, actions, K, obs_state, reward, terminated,
+                                           truncated, inner_steps, B, env0, vx, reward_f64);
         return PBN_OK;
     };
-    int rc = PBN_OK;
-    if (first_pass && nv.kind == PBN_NET_PRED) {  // lockstep first pass (Philox: checked above)
-        const bool fast = nv.off_rec16 != 0 && nv.w32 <= 8 && (nv.ts == 4 || nv.ts == 16);
-        const size_t smem_f = (size_t)nv.blob_fast_bytes + ev.img_bytes + col_align_bytes(nv.w32) + (size_t)2 * nv.w32 * block * 4;
-        if (fast && nv.ts == 4) rc = launch_first(k_env_step_first<1, true>, smem_f);
-        else if (fast) rc = launch_first(k_env_step_first<4, true>, smem_f);
-        else if (nv.ts == 4) rc = launch_first(k_env_step_first<1, false>, smem);
-        else if (nv.ts == 16) rc = launch_first(k_env_step_first<4, false>, smem);
-        else rc = launch_first(k_env_step_first<0, false>, smem);
-    } else {
-#define CALL(NK, MD, TQ)                                                                                                   \
-        if (!att) rc = launch_step(k_env_step<NK, MD>);                                                                    \
-        else if (NK == PBN_NET_PRED && MD == PBN_DRAW_PHILOX && nv.w32 == 1) rc = launch_att(k_env_step_att<NK, MD, TQ, true>); \
-        else rc = launch_att(k_env_step_att<NK, MD, TQ, false>)
-        DISPATCH(nv.kind, dv.mode, att ? nv.ts : 0, CALL);
-#undef CALL
-    }
+    const int rc = dispatch(nv.kind, dv.mode, att ? nv.ts : 0, [&](auto NK, auto MD, auto TQ) -> int {
+        if (!att) return launch_step(k_env_step<NK, MD>);
+        if constexpr (NK == PBN_NET_PRED && MD == PBN_DRAW_PHILOX) {
+            if (first_pass) {  // lockstep first pass (Philox: checked above)
+                if constexpr (TQ > 0) {
+                    if (fast) return launch_first(k_env_step_first<TQ, true>, true);
+                }
+                return launch_first(k_env_step_first<TQ, false>, false);
+            }
+        }
+        if (NK == PBN_NET_PRED && MD == PBN_DRAW_PHILOX && nv.w32 == 1) return launch_att(k_env_step_att<NK, MD, TQ, true>);
+        return launch_att(k_env_step_att<NK, MD, TQ, false>);
+    });
     if (rc) return rc;
     CK(cudaGetLastError());
     return PBN_OK;
@@ -2279,13 +2286,12 @@ static int env_reset_impl(const PbnEnv *env, uint32_t *state, int32_t *n_steps, 
     if (int rc = check_draws(draws)) return rc;
     if (B == 0) return PBN_OK;
     const DrawView dv = make_draws(draws);
-    const int block = block_for(B);
-    const unsigned grid = (unsigned)((B + block - 1) / block);
+    const unsigned grid = (unsigned)((B + PBN_BLOCK - 1) / PBN_BLOCK);
     cudaStream_t s = (cudaStream_t)stream;
     if (dv.mode == PBN_DRAW_PHILOX)
-        k_env_reset<PBN_DRAW_PHILOX><<<grid, block, 0, s>>>(env->net->v, ev, dv, state, n_steps, target_att, target_state, mask, B, env0, cv);
+        k_env_reset<PBN_DRAW_PHILOX><<<grid, PBN_BLOCK, 0, s>>>(env->net->v, ev, dv, state, n_steps, target_att, target_state, mask, B, env0, cv);
     else
-        k_env_reset<PBN_DRAW_REPLAY><<<grid, block, 0, s>>>(env->net->v, ev, dv, state, n_steps, target_att, target_state, mask, B, env0, cv);
+        k_env_reset<PBN_DRAW_REPLAY><<<grid, PBN_BLOCK, 0, s>>>(env->net->v, ev, dv, state, n_steps, target_att, target_state, mask, B, env0, cv);
     CK(cudaGetLastError());
     return PBN_OK;
 }
@@ -2295,11 +2301,10 @@ extern "C" int pbn_rand_state(const PbnNet *net, uint32_t *state, int64_t B, int
     if (int rc = check_draws(draws)) return rc;
     if (B == 0) return PBN_OK;
     const DrawView dv = make_draws(draws);
-    const int block = block_for(B);
-    const unsigned grid = (unsigned)((B + block - 1) / block);
+    const unsigned grid = (unsigned)((B + PBN_BLOCK - 1) / PBN_BLOCK);
     cudaStream_t s = (cudaStream_t)stream;
-    if (dv.mode == PBN_DRAW_PHILOX) k_rand_state<PBN_DRAW_PHILOX><<<grid, block, 0, s>>>(net->v, dv, state, B, env0);
-    else k_rand_state<PBN_DRAW_REPLAY><<<grid, block, 0, s>>>(net->v, dv, state, B, env0);
+    if (dv.mode == PBN_DRAW_PHILOX) k_rand_state<PBN_DRAW_PHILOX><<<grid, PBN_BLOCK, 0, s>>>(net->v, dv, state, B, env0);
+    else k_rand_state<PBN_DRAW_REPLAY><<<grid, PBN_BLOCK, 0, s>>>(net->v, dv, state, B, env0);
     CK(cudaGetLastError());
     return PBN_OK;
 }
@@ -2310,15 +2315,13 @@ extern "C" int pbn_env_attractor_index(const PbnEnv *env, const uint32_t *state,
     if (ev.n_att < 1) return fail(PBN_ERR_ARG, "the env has no attractor list");
     if (B == 0) return PBN_OK;
     const int w32 = env->net->v.w32;
-    const int block = block_for(B);
-    const unsigned grid = (unsigned)((B + block - 1) / block);
-    const size_t cols = (size_t)w32 * block * 4;
+    const unsigned grid = (unsigned)((B + PBN_BLOCK - 1) / PBN_BLOCK);
     // staged only while three blocks stay resident per SM: the kernel is one pass over the states, and a large cube list
     // read by every thread of a block is served from L1 as well
-    const int staged = (size_t)ev.img_bytes + cols <= 64 * 1024;
-    const size_t smem = cols + (staged ? (size_t)ev.img_bytes : 0);
-    if (int rc = set_smem(k_attractor_index, smem)) return rc;
-    k_attractor_index<<<grid, block, smem, (cudaStream_t)stream>>>(ev, w32, state, B, att_out, staged);
+    const int staged = index_smem(ev, w32, true).bytes <= 64 * 1024;
+    const size_t smem = index_smem(ev, w32, staged).bytes;
+    if (int rc = fit_smem(k_attractor_index, "k_attractor_index", smem)) return rc;
+    k_attractor_index<<<grid, PBN_BLOCK, smem, (cudaStream_t)stream>>>(ev, w32, state, B, att_out, staged);
     CK(cudaGetLastError());
     return PBN_OK;
 }
@@ -2413,31 +2416,26 @@ extern "C" int pbn_ssd(const PbnNet *net, const PbnEnv *env, uint32_t *state, in
     for (int k = 1; k < g; k++)
         if (tgt[k] != tgt[0] + k) sp.fast_t0 = -1;
     if (sp.fast_t0 >= 0 && (tgt[0] >> 5) != ((tgt[0] + g - 1) >> 5)) sp.fast_t0 = -1;
-    const int block = block_for(chains);
-    if (iters >= (1LL << 31) || (sp.smem_hist && (double)iters * block >= 4294967296.0))
+    if (iters >= (1LL << 31) || (sp.smem_hist && (double)iters * PBN_BLOCK >= 4294967296.0))
         return fail(PBN_ERR_ARG, "iters too large for one launch; split the estimate");
-    const unsigned grid = (unsigned)((chains + block - 1) / block);
+    const unsigned grid = (unsigned)((chains + PBN_BLOCK - 1) / PBN_BLOCK);
     EnvView ev;
     memset(&ev, 0, sizeof ev);
     if (env) ev = env->v;
     // windowed step-until-attractor path: flip masks of `win` iterations per warp, 2 KB per warp (networks up to 256 nodes)
     sp.win = (env && draws->mode == PBN_DRAW_PHILOX && !ev.force && nv.w32 <= 8) ? (16 / nv.w32 > 2 ? 16 / nv.w32 : 2) : 0;
-    const size_t smem = (size_t)(env ? nv.blob_bytes : nv.blob_fast_bytes) + (env ? ev.img_bytes : 0) + 128 + (sp.smem_hist ? ((size_t)4 << g) : 0) + col_align_bytes(nv.w32) + (size_t)nv.w32 * PBN_BLOCK * 4 +
-                        (size_t)(block / 32) * sp.win * nv.w32 * 32 * 4 + (sp.win ? (size_t)(block / 32) * coop_warp_bytes(nv.w32) : 0);
+    const size_t smem = ssd_smem(nv, ev, sp, env != nullptr).bytes;
     cudaStream_t s = (cudaStream_t)stream;
     if (draws->mode == PBN_DRAW_PHILOX) sp.gdelta = geom_shortcut_delta(sp.inv, s);  // gaps are drawn with the verified shortcut
-#define CALL(NK, MD, TQ)                                                                                  \
-    if (env) {                                                                                            \
-        if (int rc = set_smem(k_ssd<NK, MD, TQ, true>, smem)) return rc;                                  \
-        k_ssd<NK, MD, TQ, true><<<grid, block, smem, s>>>(nv, ev, dv, sp, state, chains, env0, (int)iters, (unsigned long long *)hist);  \
-    } else {                                                                                              \
-        if (int rc = set_smem(k_ssd<NK, MD, TQ, false>, smem)) return rc;                                 \
-        k_ssd<NK, MD, TQ, false><<<grid, block, smem, s>>>(nv, ev, dv, sp, state, chains, env0, (int)iters, (unsigned long long *)hist); \
-    }
-    DISPATCH(nv.kind, dv.mode, nv.ts, CALL);
-#undef CALL
-    CK(cudaGetLastError());
-    return PBN_OK;
+    auto launch = [&](auto kernel) -> int {
+        if (int rc = fit_smem(kernel, "k_ssd", smem)) return rc;
+        kernel<<<grid, PBN_BLOCK, smem, s>>>(nv, ev, dv, sp, state, chains, env0, (int)iters, (unsigned long long *)hist);
+        CK(cudaGetLastError());
+        return PBN_OK;
+    };
+    return dispatch(nv.kind, dv.mode, nv.ts, [&](auto NK, auto MD, auto TQ) {
+        return env ? launch(k_ssd<NK, MD, TQ, true>) : launch(k_ssd<NK, MD, TQ, false>);
+    });
 }
 
 struct HistParams { int g; short tgt[24]; };
