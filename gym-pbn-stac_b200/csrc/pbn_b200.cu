@@ -1617,58 +1617,77 @@ __device__ __forceinline__ void ssd_count(SsdCount &c, const SsdLoopArgs &a, con
     c.run++;
 }
 
-// Perturbation state of the static loop: the lane's two event slots, and its perturbation stream held as "next block index +
-// the unused half of the last block" (a round takes two words, so every second round computes a block).
-// "No pending event" is any value >= W here: an applied event is only ever lowered by W per iteration (it wraps to a value
-// above 2^32 - 2^31) until the next round overwrites it, and a round comes at the latest after 64 gaps of at most 2^25.
+// Perturbation state of the static loop.  Each event is resolved once, when its round is drawn: the iteration it is due in,
+// the shared address of the word it flips and the bit.  Checking a slot in an iteration is then a compare, a select and one
+// shared-memory XOR.  An applied event stays in its slot until the next round overwrites it: its iteration has passed, and
+// the iteration counter never meets it again.  The lane's perturbation stream is held as "next block index + the unused
+// half of the last block" (a round takes two words, so every second round computes a block).
 struct SsdFastPerturb {
-    u32 e0, e1, last_p1;
+    u32 t0, t1;   // iteration each slot's event is due in
+    u32 a0, a1;   // shared address of the word it flips
+    u32 m0, m1;   // the bit it flips
+    u32 next;     // iteration of the last generated event: the next round is drawn in it
+    u32 last_p1;  // (position of the last generated event) + 1, relative to the window of iteration `next`
     u32 blk, half, sx, sy;
 };
 
-// flip the bit of an event that lies inside the window: word (node>>5) of column (e&31), byte offset = (e&31)*4 + (node>>5)*1024,
-// node = e>>5; predicated, no branch in the source (ptxas may still branch around the atomic)
-__device__ __forceinline__ void ssd_fast_apply(const SsdFast &f, u32 e) {
-    asm volatile("{ .reg .pred p; setp.lt.u32 p, %0, %1; @p red.shared.xor.b32 [%2], %3; }"
-                 :: "r"(e), "r"(f.W), "r"((f.warp_cols | ((e << 2) & 0x7Cu)) | (e & 0xFFFFFC00u)),
-                    "r"(1u << ((e >> 5) & 31u)) : "memory");
+// XOR the slot's bit in if its event is due in iteration `it`, else XOR 0: every lane issues the atomic (a predicated
+// atomic becomes a branch with reconvergence code)
+__device__ __forceinline__ void ssd_fast_apply(u32 t_due, u32 a, u32 m, u32 it) { red_xor_u32(a, t_due == it ? m : 0u); }
+
+// the slot of an event at position e relative to the window of iteration `it`: window e / W (ssd_window_div), and in it
+// bit (c>>5) of chain (c&31), i.e. word (c>>10) of column (c&31) at byte offset (c&31)*4 + (c>>10)*1024
+__device__ __forceinline__ void ssd_fast_slot(const SsdFast &f, const SsdParams &sp, u32 e, u32 it, u32 &t_due, u32 &a, u32 &m) {
+    const u32 q = __umulhi(e >> 4, sp.wq_mul) >> sp.wq_sh;
+    const u32 c = e - q * f.W;
+    t_due = it + q;
+    a = f.warp_cols | ((c << 2) & 0x7Cu) | (c & 0xFFFFFC00u);
+    m = 1u << ((c >> 5) & 31u);
 }
 
 __device__ __forceinline__ u32 ssd_fast_gap(const SsdFast &f, u32 word, bool &ok) { return geom_gap_approx(word, f.inv, f.gdelta, &ok); }
 
-__device__ __forceinline__ void ssd_fast_perturb(const SsdFast &f, SsdFastPerturb &ps, const Draw<PBN_DRAW_PHILOX> &dp, const DrawView &dv) {
-    ssd_fast_apply(f, ps.e0);
-    ssd_fast_apply(f, ps.e1);
-    // last_p1 comes out of a warp reduction: the compiler knows it is the same in every lane and branches on it without
-    // reconvergence code
-    while (ps.last_p1 <= f.W) {  // every pending event lay inside this window and has just been applied: the next round
-        u32 wa, wb;
-        if (ps.half == 0u) {  // a round takes two words: every second one computes a block
-            u32 x2, x3;
-            philox4x32_10_rk(ps.blk, dp.c1, dp.c2, dp.c3, dv, wa, wb, x2, x3);
-            ps.blk++;
-            ps.sx = x2; ps.sy = x3;
-            ps.half = 1u;
-        } else {
-            wa = ps.sx; wb = ps.sy;
-            ps.half = 0u;
-        }
-        bool ok0, ok1;
-        u32 g0 = ssd_fast_gap(f, wa, ok0), g1 = ssd_fast_gap(f, wb, ok1);
-        if (!(ok0 && ok1)) {  // within the margin of an integer (or shortcut off): the defining polynomial
-            if (!ok0) g0 = geom_gap(wa, f.inv);
-            if (!ok1) g1 = geom_gap(wb, f.inv);
-        }
-        const u32 incl = warp_scan_add(g0 + g1 + 2u);
-        ps.e1 = ps.last_p1 - 1u + incl;
-        ps.e0 = ps.e1 - 1u - g1;
-        ps.last_p1 = __reduce_max_sync(0xFFFFFFFFu, ps.e1) + 1u;  // lane 31's: positions ascend with the lane
-        ssd_fast_apply(f, ps.e0);
-        ssd_fast_apply(f, ps.e1);
+// iteration `it` of the perturbation process: apply the events due in it, and draw rounds while the last generated event
+// lies inside its window (a round is drawn only when every pending event is due in this iteration, so two slots suffice)
+__device__ __forceinline__ void ssd_fast_perturb(const SsdFast &f, const SsdParams &sp, SsdFastPerturb &ps, const Draw<PBN_DRAW_PHILOX> &dp,
+                                                 const DrawView &dv, u32 it) {
+    ssd_fast_apply(ps.t0, ps.a0, ps.m0, it);
+    ssd_fast_apply(ps.t1, ps.a1, ps.m1, it);
+    if (ps.next == it) {
+        // last_p1 comes out of a warp reduction: the compiler knows it is the same in every lane and branches on it without
+        // reconvergence code
+        u32 last_p1 = ps.last_p1;
+        do {
+            u32 wa, wb;
+            if (ps.half == 0u) {  // a round takes two words: every second one computes a block
+                u32 x2, x3;
+                philox4x32_10_rk(ps.blk, dp.c1, dp.c2, dp.c3, dv, wa, wb, x2, x3);
+                ps.blk++;
+                ps.sx = x2; ps.sy = x3;
+                ps.half = 1u;
+            } else {
+                wa = ps.sx; wb = ps.sy;
+                ps.half = 0u;
+            }
+            bool ok0, ok1;
+            u32 g0 = ssd_fast_gap(f, wa, ok0), g1 = ssd_fast_gap(f, wb, ok1);
+            if (!(ok0 && ok1)) {  // within the margin of an integer (or shortcut off): the defining polynomial
+                if (!ok0) g0 = geom_gap(wa, f.inv);
+                if (!ok1) g1 = geom_gap(wb, f.inv);
+            }
+            const u32 incl = warp_scan_add(g0 + g1 + 2u);
+            const u32 e1 = last_p1 - 1u + incl;
+            const u32 e0 = e1 - 1u - g1;
+            last_p1 = __reduce_max_sync(0xFFFFFFFFu, e1) + 1u;  // lane 31's: positions ascend with the lane
+            ssd_fast_slot(f, sp, e0, it, ps.t0, ps.a0, ps.m0);
+            ssd_fast_slot(f, sp, e1, it, ps.t1, ps.a1, ps.m1);
+            ssd_fast_apply(ps.t0, ps.a0, ps.m0, it);
+            ssd_fast_apply(ps.t1, ps.a1, ps.m1, it);
+        } while (last_p1 <= f.W);
+        const u32 q = __umulhi((last_p1 - 1u) >> 4, sp.wq_mul) >> sp.wq_sh;  // >= 1: the window of the last event
+        ps.next = it + q;
+        ps.last_p1 = last_p1 - q * f.W;
     }
-    ps.e0 -= f.W;
-    ps.e1 -= f.W;
-    ps.last_p1 -= f.W;
     __syncwarp();
 }
 
@@ -1677,6 +1696,7 @@ __device__ __forceinline__ void ssd_fast_perturb(const SsdFast &f, SsdFastPertur
 template <int TQ>
 __device__ __forceinline__ int ssd_loop_pred_static(const SsdLoopArgs &a, const Col &st, Draw<PBN_DRAW_PHILOX> &d,
                                                     Draw<PBN_DRAW_PHILOX> &dp, SsdPerturb &ps0, SsdCount &cnt) {
+    if (a.iters < 2) return 0;
     const NetView &nv = a.nv;
     SsdFast f;
     f.col = keep(smem_addr(st.s));
@@ -1693,7 +1713,9 @@ __device__ __forceinline__ int ssd_loop_pred_static(const SsdLoopArgs &a, const 
     f.b_up = keep(32u - (u32)a.sp.g);
     f.inv = a.sp.inv;
     f.gdelta = 0.5f - a.sp.gdelta;  // the shortcut compares against 0.5 - margin (negative: never taken)
-    SsdFastPerturb ps{ps0.e0, ps0.e1, ps0.last_p1, dp.blk, 0u, 0u, 0u};  // (entered at the start of the loop: dp has no buffered words)
+    // entered at the start of the loop: no pending events, the first round due in iteration 0, no buffered words in dp
+    // (the empty slots still hold a valid address: every lane XORs through both slots in every iteration)
+    SsdFastPerturb ps{~0u, ~0u, f.warp_cols, f.warp_cols, 0u, 0u, 0u, ps0.last_p1, dp.blk, 0u, 0u, 0u};
     u32 ublk = 0;
     int t = 0;
     u32 cur = (u32)cnt.cur, run = cnt.run;
@@ -1713,24 +1735,31 @@ __device__ __forceinline__ int ssd_loop_pred_static(const SsdLoopArgs &a, const 
         // shared-memory loads are over when the state half needs them
         const FastDraw da = ssd_fast_draw<TQ>(f, x0, x1);
         count();
-        ssd_fast_perturb(f, ps, dp, a.dv);
+        ssd_fast_perturb(f, a.sp, ps, dp, a.dv, (u32)t);
         ssd_fast_apply_update(f, da);
         __syncwarp();
         const FastDraw db = ssd_fast_draw<TQ>(f, x2, x3);
         count();
-        ssd_fast_perturb(f, ps, dp, a.dv);
+        ssd_fast_perturb(f, a.sp, ps, dp, a.dv, (u32)t + 1u);
         ssd_fast_apply_update(f, db);
         __syncwarp();
     }
     d.blk = ublk;
     d.have = 0;
-    // hand the perturbation stream and the pending events back to the generic loop (an odd last iteration)
+    // hand the perturbation stream and the pending events back to the generic loop (an odd last iteration), as positions
+    // relative to the window of iteration t; the loop drew a round in iteration 0, so both slots hold events
     dp.blk = ps.blk;
     dp.have = ps.half ? 2 : 0;
     dp.b0 = ps.sx; dp.b1 = ps.sy;
-    ps0.e0 = ps.e0 >= 0x80000000u ? 0xFFFFFFFFu : ps.e0;
-    ps0.e1 = ps.e1 >= 0x80000000u ? 0xFFFFFFFFu : ps.e1;
-    ps0.last_p1 = ps.last_p1;
+    const u32 tu = (u32)t;
+    auto position = [&](u32 t_due, u32 addr, u32 m) {
+        if (t_due < tu) return 0xFFFFFFFFu;  // applied
+        const u32 x = addr ^ f.warp_cols;   // (word << 10) | (chain << 2)
+        return (t_due - tu) * f.W + ((x & 0xFFFFFC00u) | ((31u - __clz(m)) << 5) | ((x >> 2) & 31u));
+    };
+    ps0.e0 = position(ps.t0, ps.a0, ps.m0);
+    ps0.e1 = position(ps.t1, ps.a1, ps.m1);
+    ps0.last_p1 = (ps.next - tu) * f.W + ps.last_p1;
     cnt.cur = (int)cur; cnt.run = run;
     return t;
 }
@@ -2388,6 +2417,18 @@ extern "C" int pbn_geom_shortcut_check(double p, float *delta, uint32_t *disagre
     return PBN_OK;
 }
 
+// The static SSD loop finds the window (iteration) of a perturbation position e without a divide: e / W, W = 32 n, is
+// umulhi(e >> 4, wq_mul) >> wq_sh.  Exact for every position the loop forms: those are below 2^31 + 2^14 (a round starts
+// at most W <= 8192 into its window and spans 64 gaps of at most 2^25 + 1), so y = e >> 4 < 2^28 and e / W = y / d with
+// d = 2n >= 2.  With sh = ceil(log2 d) - 1 and mul = ceil(2^(32+sh) / d) = (2^(32+sh) + r) / d, 0 <= r < d <= 2^(sh+1):
+// y mul / 2^(32+sh) = y / d + y r / (d 2^(32+sh)) and y r < 2^28 2^(sh+1) < 2^(32+sh), so the excess is below 1/d and
+// cannot reach the next integer.  mul < 2^32 because d > 2^sh.
+static void ssd_window_div(int n, SsdParams &sp) {
+    const unsigned long long d = 2ull * (unsigned)n;
+    sp.wq_sh = 63 - __builtin_clzll(d - 1);
+    sp.wq_mul = (unsigned)(((1ull << (32 + sp.wq_sh)) + d - 1) / d);
+}
+
 extern "C" int pbn_ssd(const PbnNet *net, const PbnEnv *env, uint32_t *state, int64_t chains, int64_t env0, int64_t iters,
                        double p, const int32_t *tgt, int32_t g, uint64_t *hist, const PbnDraws *draws, void *stream) {
     if (!net || !state || !tgt || !hist || chains < 0 || iters < 0) return fail(PBN_ERR_ARG, "bad argument");
@@ -2405,6 +2446,7 @@ extern "C" int pbn_ssd(const PbnNet *net, const PbnEnv *env, uint32_t *state, in
     sp.g = g; sp.p = p; sp.smem_hist = g <= 12;
     sp.inv = p <= 0 ? 1.0f : (p >= 1 ? 0.0f : (float)(1.0 / std::log2(1.0 - p)));
     sp.gdelta = 1.0f;
+    ssd_window_div(nv.n, sp);
     memset(sp.tgt, 0, sizeof sp.tgt);
     for (int k = 0; k < g; k++) {
         if (tgt[k] < 0 || tgt[k] >= nv.n) return fail(PBN_ERR_ARG, "target node out of range");

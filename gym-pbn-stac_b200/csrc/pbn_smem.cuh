@@ -9,6 +9,8 @@ struct SsdParams {
     int win;        // iterations per window of the step-until-attractor path (0 = iteration by iteration)
     float inv;      // 1/log2(1-p) <= 0; a value > 0 means flips disabled (p == 0)
     float gdelta;   // margin of the lg2.approx shortcut of the gap draw (geom_gap_approx); >= 0.5: shortcut off
+    unsigned wq_mul;  // window of a perturbation position e: e / (32 n) = umulhi(e >> 4, wq_mul) >> wq_sh (ssd_window_div)
+    int wq_sh;
     double p;
     short tgt[24];
 };
