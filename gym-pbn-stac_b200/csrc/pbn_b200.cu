@@ -47,6 +47,7 @@ extern "C" const char *pbn_version(void) { return "pbn_b200 0.1 (sm_100a)"; }
 struct PbnNet {
     NetView v;
     std::vector<void *> owned;
+    u32 tt_const;  // TT: index (in the threshold table) of two constant entries, 0 (never 1) and 2^31 (always 1)
 };
 struct PbnEnv {
     EnvView v;
@@ -193,6 +194,13 @@ extern "C" int pbn_net_create(const PbnNetDesc *d, PbnNet **out) {
     blob.resize((blob.size() + 15) & ~(size_t)15);
     v.blob_bytes = v.blob_fast_bytes = (int)blob.size();
     if (v.off_rec16) v.blob_bytes = v.off_rec16;  // everything but the fast paths stages the image without the 16-byte records
+    if (d->kind == PBN_NET_TT) {
+        // behind the image (not staged by the existing kernels): the constant entries that pbn_ssd_pinned points the node
+        // records of pinned nodes at
+        net->tt_const = (u32)(blob.size() - v.off_thr) / 4u;
+        blob.resize(blob.size() + 16, 0);
+        reinterpret_cast<u32 *>(blob.data() + v.blob_bytes)[1] = 0x80000000u;
+    }
     rc |= upload(net->owned, blob.data(), blob.size(), &v.blob);
     if (rc) { pbn_net_destroy(net); return PBN_ERR_CUDA; }
     v.thr_dev = nullptr;
@@ -307,6 +315,7 @@ __device__ __forceinline__ void red_add_u32(u32 a, u32 v) { asm volatile("red.sh
 __device__ __forceinline__ uint4 ldc_v4(u32 a) {  // read-only image data: free to schedule
     uint4 v; asm("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(a)); return v;
 }
+__device__ __forceinline__ u32 ldc_u32(u32 a) { u32 v; asm("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(a)); return v; }
 __device__ __forceinline__ uint2 ldc_v2(u32 a) { uint2 v; asm("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(v.x), "=r"(v.y) : "r"(a)); return v; }
 __device__ __forceinline__ u32 keep(u32 x) { asm volatile("" : "+r"(x)); return x; }  // pins a loop invariant in a register
 
@@ -1555,13 +1564,21 @@ __device__ __forceinline__ void ssd_round(SsdPerturb &ps, u32 g0, u32 g1) {
     ps.last_p1 = __shfl_sync(0xFFFFFFFFu, ps.e1, 31) + 1u;
 }
 
-template <bool FULL>
-__device__ __forceinline__ void ssd_perturb(SsdPerturb &ps, Draw<PBN_DRAW_PHILOX> &dp, char *warp_cols, u32 W, float inv, float hmd, u32 nvalid) {
+// PIN (k_ssd_pinned): an event on a node outside the free mask s_free (word w = nodes 32w..32w+31) is drawn and not applied
+template <bool FULL, bool PIN = false>
+__device__ __forceinline__ void ssd_perturb(SsdPerturb &ps, Draw<PBN_DRAW_PHILOX> &dp, char *warp_cols, u32 W, float inv, float hmd, u32 nvalid,
+                                            const u32 *s_free = nullptr) {
     auto apply = [&](u32 &e) {
         if (e < W) {
             const u32 tl = e & 31u;
-            // word (node>>5) of column tl: byte offset = tl*4 + (node>>5)*1024, node = e>>5
-            if (FULL || tl < nvalid) atomicXor(reinterpret_cast<u32 *>(warp_cols + tl * 4u + ((e >> 10) << 10)), 1u << ((e >> 5) & 31u));
+            // word (node>>5) of column tl: byte offset = tl*4 + (node>>5)*1024, node = e>>5.  Two statements rather than a
+            // masked bit formed ahead: that form reschedules (changes the SASS of) the unpinned k_ssd instantiations
+            if constexpr (PIN) {
+                if (FULL || tl < nvalid)
+                    atomicXor(reinterpret_cast<u32 *>(warp_cols + tl * 4u + ((e >> 10) << 10)), (1u << ((e >> 5) & 31u)) & s_free[e >> 10]);
+            } else {
+                if (FULL || tl < nvalid) atomicXor(reinterpret_cast<u32 *>(warp_cols + tl * 4u + ((e >> 10) << 10)), 1u << ((e >> 5) & 31u));
+            }
             e = 0xFFFFFFFFu;
         }
     };
@@ -1636,21 +1653,26 @@ struct SsdFastPerturb {
 __device__ __forceinline__ void ssd_fast_apply(u32 t_due, u32 a, u32 m, u32 it) { red_xor_u32(a, t_due == it ? m : 0u); }
 
 // the slot of an event at position e relative to the window of iteration `it`: window e / W (ssd_window_div), and in it
-// bit (c>>5) of chain (c&31), i.e. word (c>>10) of column (c&31) at byte offset (c&31)*4 + (c>>10)*1024
-__device__ __forceinline__ void ssd_fast_slot(const SsdFast &f, const SsdParams &sp, u32 e, u32 it, u32 &t_due, u32 &a, u32 &m) {
+// bit (c>>5) of chain (c&31), i.e. word (c>>10) of column (c&31) at byte offset (c&31)*4 + (c>>10)*1024.  PIN: the bit is
+// masked with word (c>>10) of the free mask at shared address `free` (an event on a pinned node XORs 0)
+template <bool PIN = false>
+__device__ __forceinline__ void ssd_fast_slot(const SsdFast &f, const SsdParams &sp, u32 e, u32 it, u32 &t_due, u32 &a, u32 &m,
+                                              u32 free = 0u) {
     const u32 q = __umulhi(e >> 4, sp.wq_mul) >> sp.wq_sh;
     const u32 c = e - q * f.W;
     t_due = it + q;
     a = f.warp_cols | ((c << 2) & 0x7Cu) | (c & 0xFFFFFC00u);
     m = 1u << ((c >> 5) & 31u);
+    if constexpr (PIN) m &= ldc_u32(free + ((c >> 8) & ~3u));
 }
 
 __device__ __forceinline__ u32 ssd_fast_gap(const SsdFast &f, u32 word, bool &ok) { return geom_gap_approx(word, f.inv, f.gdelta, &ok); }
 
 // iteration `it` of the perturbation process: apply the events due in it, and draw rounds while the last generated event
 // lies inside its window (a round is drawn only when every pending event is due in this iteration, so two slots suffice)
+template <bool PIN = false>
 __device__ __forceinline__ void ssd_fast_perturb(const SsdFast &f, const SsdParams &sp, SsdFastPerturb &ps, const Draw<PBN_DRAW_PHILOX> &dp,
-                                                 const DrawView &dv, u32 it) {
+                                                 const DrawView &dv, u32 it, u32 free = 0u) {
     ssd_fast_apply(ps.t0, ps.a0, ps.m0, it);
     ssd_fast_apply(ps.t1, ps.a1, ps.m1, it);
     if (ps.next == it) {
@@ -1679,8 +1701,8 @@ __device__ __forceinline__ void ssd_fast_perturb(const SsdFast &f, const SsdPara
             const u32 e1 = last_p1 - 1u + incl;
             const u32 e0 = e1 - 1u - g1;
             last_p1 = __reduce_max_sync(0xFFFFFFFFu, e1) + 1u;  // lane 31's: positions ascend with the lane
-            ssd_fast_slot(f, sp, e0, it, ps.t0, ps.a0, ps.m0);
-            ssd_fast_slot(f, sp, e1, it, ps.t1, ps.a1, ps.m1);
+            ssd_fast_slot<PIN>(f, sp, e0, it, ps.t0, ps.a0, ps.m0, free);
+            ssd_fast_slot<PIN>(f, sp, e1, it, ps.t1, ps.a1, ps.m1, free);
             ssd_fast_apply(ps.t0, ps.a0, ps.m0, it);
             ssd_fast_apply(ps.t1, ps.a1, ps.m1, it);
         } while (last_p1 <= f.W);
@@ -1693,9 +1715,9 @@ __device__ __forceinline__ void ssd_fast_perturb(const SsdFast &f, const SsdPara
 
 // STATIC path of predictor networks, full warps, no attractor loop, shared histogram, targets inside one state word:
 // the configuration the headline number is measured in.  Returns the number of iterations done (even).
-template <int TQ>
+template <int TQ, bool PIN = false>
 __device__ __forceinline__ int ssd_loop_pred_static(const SsdLoopArgs &a, const Col &st, Draw<PBN_DRAW_PHILOX> &d,
-                                                    Draw<PBN_DRAW_PHILOX> &dp, SsdPerturb &ps0, SsdCount &cnt) {
+                                                    Draw<PBN_DRAW_PHILOX> &dp, SsdPerturb &ps0, SsdCount &cnt, const u32 *s_free = nullptr) {
     if (a.iters < 2) return 0;
     const NetView &nv = a.nv;
     SsdFast f;
@@ -1713,6 +1735,8 @@ __device__ __forceinline__ int ssd_loop_pred_static(const SsdLoopArgs &a, const 
     f.b_up = keep(32u - (u32)a.sp.g);
     f.inv = a.sp.inv;
     f.gdelta = 0.5f - a.sp.gdelta;  // the shortcut compares against 0.5 - margin (negative: never taken)
+    u32 free = 0u;
+    if constexpr (PIN) free = keep(smem_addr(s_free));
     // entered at the start of the loop: no pending events, the first round due in iteration 0, no buffered words in dp
     // (the empty slots still hold a valid address: every lane XORs through both slots in every iteration)
     SsdFastPerturb ps{~0u, ~0u, f.warp_cols, f.warp_cols, 0u, 0u, 0u, ps0.last_p1, dp.blk, 0u, 0u, 0u};
@@ -1735,12 +1759,12 @@ __device__ __forceinline__ int ssd_loop_pred_static(const SsdLoopArgs &a, const 
         // shared-memory loads are over when the state half needs them
         const FastDraw da = ssd_fast_draw<TQ>(f, x0, x1);
         count();
-        ssd_fast_perturb(f, a.sp, ps, dp, a.dv, (u32)t);
+        ssd_fast_perturb<PIN>(f, a.sp, ps, dp, a.dv, (u32)t, free);
         ssd_fast_apply_update(f, da);
         __syncwarp();
         const FastDraw db = ssd_fast_draw<TQ>(f, x2, x3);
         count();
-        ssd_fast_perturb(f, a.sp, ps, dp, a.dv, (u32)t + 1u);
+        ssd_fast_perturb<PIN>(f, a.sp, ps, dp, a.dv, (u32)t + 1u, free);
         ssd_fast_apply_update(f, db);
         __syncwarp();
     }
@@ -1754,6 +1778,9 @@ __device__ __forceinline__ int ssd_loop_pred_static(const SsdLoopArgs &a, const 
     const u32 tu = (u32)t;
     auto position = [&](u32 t_due, u32 addr, u32 m) {
         if (t_due < tu) return 0xFFFFFFFFu;  // applied
+        if constexpr (PIN) {
+            if (m == 0u) return 0xFFFFFFFFu;  // on a pinned node: never applied
+        }
         const u32 x = addr ^ f.warp_cols;   // (word << 10) | (chain << 2)
         return (t_due - tu) * f.W + ((x & 0xFFFFFC00u) | ((31u - __clz(m)) << 5) | ((x >> 2) & 31u));
     };
@@ -1764,8 +1791,9 @@ __device__ __forceinline__ int ssd_loop_pred_static(const SsdLoopArgs &a, const 
     return t;
 }
 
-template <int NET, int MODE, int TQ, bool HAS_ENV, bool FULL>
-__device__ __forceinline__ void ssd_loop(const SsdLoopArgs &a, const Col &st, Draw<MODE> &d, Draw<MODE> &dp) {
+// PIN (k_ssd_pinned): perturbation events are masked with the free-node mask s_free of the block's variant
+template <int NET, int MODE, int TQ, bool HAS_ENV, bool FULL, bool PIN = false>
+__device__ __forceinline__ void ssd_loop(const SsdLoopArgs &a, const Col &st, Draw<MODE> &d, Draw<MODE> &dp, const u32 *s_free = nullptr) {
     const NetView &nv = a.nv;
     const SsdParams &sp = a.sp;
     const u32 lane = threadIdx.x & 31u;
@@ -1779,7 +1807,7 @@ __device__ __forceinline__ void ssd_loop(const SsdLoopArgs &a, const Col &st, Dr
     SsdCount cnt{active ? ssd_bucket(sp, a.s_tgt, st) : 0, 0u};
     int t = 0;
     if constexpr (MODE == PBN_DRAW_PHILOX && !HAS_ENV && FULL && NET == PBN_NET_PRED && TQ > 0) {
-        if (flips && sp.smem_hist && sp.fast_t0 >= 0 && nv.off_rec16) t = ssd_loop_pred_static<TQ>(a, st, d, dp, ps, cnt);
+        if (flips && sp.smem_hist && sp.fast_t0 >= 0 && nv.off_rec16) t = ssd_loop_pred_static<TQ, PIN>(a, st, d, dp, ps, cnt, s_free);
     }
     if constexpr (MODE == PBN_DRAW_PHILOX && !HAS_ENV && FULL) {
         // STATIC path: one Philox block of the update stream per two iterations, words used in stream order
@@ -1789,11 +1817,11 @@ __device__ __forceinline__ void ssd_loop(const SsdLoopArgs &a, const Col &st, Dr
             philox4x32_10(ublk, d.c1, d.c2, d.c3, d.k0, d.k1, x0, x1, x2, x3);
             ublk++;
             ssd_count(cnt, a, st);
-            if (flips) ssd_perturb<true>(ps, dp, warp_cols, W, inv, hmd, 32u);
+            if (flips) ssd_perturb<true, PIN>(ps, dp, warp_cols, W, inv, hmd, 32u, s_free);
             micro_step_words<NET, TQ>(nv, a.blob, st, x0, x1, d);
             __syncwarp();  // updates land before the next iteration's cross-lane flips
             ssd_count(cnt, a, st);
-            if (flips) ssd_perturb<true>(ps, dp, warp_cols, W, inv, hmd, 32u);
+            if (flips) ssd_perturb<true, PIN>(ps, dp, warp_cols, W, inv, hmd, 32u, s_free);
             micro_step_words<NET, TQ>(nv, a.blob, st, x2, x3, d);
             __syncwarp();
         }
@@ -1870,7 +1898,7 @@ __device__ __forceinline__ void ssd_loop(const SsdLoopArgs &a, const Col &st, Dr
                 for (u32 j = 0; j < n; j++)
                     if (d.dbl() < sp.p) st.flip(j);  // np.random.rand(N) < p ; flipNode(j)  (eval.py:92-95)
         } else {
-            if (flips) ssd_perturb<FULL>(ps, dp, warp_cols, W, inv, hmd, a.nvalid);
+            if (flips) ssd_perturb<FULL, PIN>(ps, dp, warp_cols, W, inv, hmd, a.nvalid, s_free);
         }
         if (active) {
             micro_step<NET, MODE, TQ>(nv, a.blob, st, d);  // env.step(0): pbn_target.py:269-271
@@ -1947,6 +1975,83 @@ __global__ void __launch_bounds__(PBN_BLOCK, HAS_ENV ? 3 : PBN_SSD_MIN_BLOCKS) k
         __syncthreads();
         for (int b = threadIdx.x; b < nb; b += PBN_BLOCK)
             if (shist[b]) atomicAdd(&hist[b], (unsigned long long)shist[b]);
+    }
+}
+
+// k_ssd (no env, Philox draws) under K pin sets (pbn_ssd_pinned): variant k owns blocks (x, k), its chain c is state column
+// k * chains + c and draws from the streams of chain id env0 + c, as in k_ssd.  A pin acts through the block's copy of the
+// network image, where the pinned node's function becomes the constant (an update that picks it draws as usual), and through
+// the perturbation events, whose bit is masked with the variant's free nodes where it is formed.
+template <int NET, int TQ>
+__global__ void __launch_bounds__(PBN_BLOCK, PBN_SSD_MIN_BLOCKS) k_ssd_pinned(NetView nv, DrawView dv, SsdParams sp, u32 *state,
+                                                                              long long chains, long long env0, int iters,
+                                                                              unsigned long long *hist, const u32 *pin_care,
+                                                                              const u32 *pin_value, u32 tt_const) {
+    EnvView ev;
+    memset(&ev, 0, sizeof ev);
+    unsigned char *blob = smem_raw;
+    const SsdSmem L = ssd_smem(nv, ev, sp, false, true);
+    u32 *s_free = reinterpret_cast<u32 *>(smem_raw + L.pin);
+    u32 *s_tgt = reinterpret_cast<u32 *>(smem_raw + L.tgt);
+    u32 *shist = reinterpret_cast<u32 *>(smem_raw + L.hist);
+    const int nb = 1 << sp.g;
+    u32 *sst = align_cols(shist + (sp.smem_hist ? nb : 0), nv.w32);
+    const int w32 = nv.w32;
+    const u32 *care = pin_care + (size_t)blockIdx.y * w32, *value = pin_value + (size_t)blockIdx.y * w32;
+    auto care_word = [&](int w) {  // bits at or above N are ignored
+        return (w == w32 - 1 && (nv.n & 31)) ? care[w] & ((1u << (nv.n & 31)) - 1u) : care[w];
+    };
+    stage(blob, nv.blob, L.image);
+    for (int w = threadIdx.x; w < w32; w += PBN_BLOCK) s_free[w] = ~care_word(w);
+    if (threadIdx.x == 0) {
+#pragma unroll
+        for (int k = 0; k < 24; k++) s_tgt[k] = (u32)sp.tgt[k];
+    }
+    if (sp.smem_hist)
+        for (int b = threadIdx.x; b < nb; b += PBN_BLOCK) shist[b] = 0;
+    __syncthreads();  // the image is staged: patch the records of the pinned nodes
+    for (int i = threadIdx.x; i < nv.n; i += PBN_BLOCK) {
+        if (!((care[i >> 5] >> (i & 31)) & 1u)) continue;
+        const u32 v = (value[i >> 5] >> (i & 31)) & 1u;
+        if constexpr (NET == PBN_NET_PRED) {  // every predictor's LUT all zeros or all ones
+            uint2 *rec = reinterpret_cast<uint2 *>(blob + nv.off_rec) + i * nv.fmax;
+            for (int k = 0; k < nv.fmax; k++) rec[k].y = v ? 0xFFFFu : 0u;
+            if (nv.off_rec16) {  // the doubled LUT field of the 16-byte records
+                uint4 *r16 = reinterpret_cast<uint4 *>(blob + nv.off_rec16) + i * nv.fmax;
+                for (int k = 0; k < nv.fmax; k++) r16[k].z = v ? 0xFFFFFFFFu : 0u;
+            }
+        } else {  // no inputs, table entry tt_const + v (staged behind the image, or read through thr_dev)
+            reinterpret_cast<uint2 *>(blob + nv.off_node)[i] = make_uint2(tt_const + v, 0u);
+        }
+    }
+    const long long e = (long long)blockIdx.x * PBN_BLOCK + threadIdx.x;
+    const long long B = (long long)gridDim.y * chains, col = (long long)blockIdx.y * chains + e;
+    Col st{sst + threadIdx.x};
+    const bool active = e < chains;
+    if (active) {
+        load_state(st, state, B, col, w32);
+        for (int w = 0; w < w32; w++) {
+            const u32 c = care_word(w);
+            st.set_word(w, (st.word(w) & ~c) | (value[w] & c));
+        }
+    }
+    __syncthreads();
+    unsigned long long *vhist = hist + ((size_t)blockIdx.y << sp.g);
+    const long long warp_left = chains - (e - (threadIdx.x & 31));
+    if (warp_left > 0) {
+        Draw<PBN_DRAW_PHILOX> d, dp;
+        d.init(dv, e, env0 + e);
+        dp.init_perturb(dv, e, env0 + e);
+        const u32 nvalid = warp_left >= 32 ? 32u : (u32)warp_left;
+        SsdLoopArgs a{nv, ev, sp, dv, blob, nullptr, nullptr, s_tgt, shist, vhist, sst, iters, nvalid, nullptr, 0, env0 + e, nullptr};
+        if (nvalid == 32u) ssd_loop<NET, PBN_DRAW_PHILOX, TQ, false, true, true>(a, st, d, dp, s_free);
+        else ssd_loop<NET, PBN_DRAW_PHILOX, TQ, false, false, true>(a, st, d, dp, s_free);
+        if (active) store_state(st, state, B, col, w32);
+    }
+    if (sp.smem_hist) {
+        __syncthreads();
+        for (int b = threadIdx.x; b < nb; b += PBN_BLOCK)
+            if (shist[b]) atomicAdd(&vhist[b], (unsigned long long)shist[b]);
     }
 }
 
@@ -2429,23 +2534,22 @@ static void ssd_window_div(int n, SsdParams &sp) {
     sp.wq_mul = (unsigned)(((1ull << (32 + sp.wq_sh)) + d - 1) / d);
 }
 
-extern "C" int pbn_ssd(const PbnNet *net, const PbnEnv *env, uint32_t *state, int64_t chains, int64_t env0, int64_t iters,
-                       double p, const int32_t *tgt, int32_t g, uint64_t *hist, const PbnDraws *draws, void *stream) {
-    if (!net || !state || !tgt || !hist || chains < 0 || iters < 0) return fail(PBN_ERR_ARG, "bad argument");
+// Argument checks and launch parameters shared by pbn_ssd and pbn_ssd_pinned (sp.win is left to the caller).  *run = false:
+// nothing to launch (no chains or no iterations).
+static int ssd_prepare(const NetView &nv, int64_t chains, int64_t env0, int64_t iters, double p, const int32_t *tgt, int32_t g,
+                       const PbnDraws *draws, cudaStream_t s, SsdParams &sp, bool *run) {
+    *run = false;
     if (g < 1 || g > 24) return fail(PBN_ERR_ARG, "1 <= g <= 24 target nodes");
     if (!(p >= 0.0 && p <= 1.0)) return fail(PBN_ERR_ARG, "Invalid Bit Flip Probability value.");  // eval.py:31-33
-    if (env && env->net != net) return fail(PBN_ERR_ARG, "env belongs to another network");
     if (int rc = check_draws(draws)) return rc;
     if (chains == 0 || iters == 0) return PBN_OK;
     if (draws->mode == PBN_DRAW_PHILOX && p > 0 && (env0 & 31))
         return fail(PBN_ERR_ARG, "env0 must be a multiple of 32: the perturbation stream is shared by groups of 32 consecutive chain ids");
     if (p > 0 && p < 1e-6) return fail(PBN_ERR_UNSUPPORTED, "bit_flip_prob below 1e-6 is not supported (gap law is truncated at 2^25)");
-    const NetView &nv = net->v;
-    const DrawView dv = make_draws(draws);
-    SsdParams sp;
     sp.g = g; sp.p = p; sp.smem_hist = g <= 12;
     sp.inv = p <= 0 ? 1.0f : (p >= 1 ? 0.0f : (float)(1.0 / std::log2(1.0 - p)));
     sp.gdelta = 1.0f;
+    sp.win = 0;
     ssd_window_div(nv.n, sp);
     memset(sp.tgt, 0, sizeof sp.tgt);
     for (int k = 0; k < g; k++) {
@@ -2460,6 +2564,22 @@ extern "C" int pbn_ssd(const PbnNet *net, const PbnEnv *env, uint32_t *state, in
     if (sp.fast_t0 >= 0 && (tgt[0] >> 5) != ((tgt[0] + g - 1) >> 5)) sp.fast_t0 = -1;
     if (iters >= (1LL << 31) || (sp.smem_hist && (double)iters * PBN_BLOCK >= 4294967296.0))
         return fail(PBN_ERR_ARG, "iters too large for one launch; split the estimate");
+    if (draws->mode == PBN_DRAW_PHILOX) sp.gdelta = geom_shortcut_delta(sp.inv, s);  // gaps are drawn with the verified shortcut
+    *run = true;
+    return PBN_OK;
+}
+
+extern "C" int pbn_ssd(const PbnNet *net, const PbnEnv *env, uint32_t *state, int64_t chains, int64_t env0, int64_t iters,
+                       double p, const int32_t *tgt, int32_t g, uint64_t *hist, const PbnDraws *draws, void *stream) {
+    if (!net || !state || !tgt || !hist || chains < 0 || iters < 0) return fail(PBN_ERR_ARG, "bad argument");
+    if (env && env->net != net) return fail(PBN_ERR_ARG, "env belongs to another network");
+    const NetView &nv = net->v;
+    cudaStream_t s = (cudaStream_t)stream;
+    SsdParams sp;
+    bool run;
+    if (int rc = ssd_prepare(nv, chains, env0, iters, p, tgt, g, draws, s, sp, &run)) return rc;
+    if (!run) return PBN_OK;
+    const DrawView dv = make_draws(draws);
     const unsigned grid = (unsigned)((chains + PBN_BLOCK - 1) / PBN_BLOCK);
     EnvView ev;
     memset(&ev, 0, sizeof ev);
@@ -2467,8 +2587,6 @@ extern "C" int pbn_ssd(const PbnNet *net, const PbnEnv *env, uint32_t *state, in
     // windowed step-until-attractor path: flip masks of `win` iterations per warp, 2 KB per warp (networks up to 256 nodes)
     sp.win = (env && draws->mode == PBN_DRAW_PHILOX && !ev.force && nv.w32 <= 8) ? (16 / nv.w32 > 2 ? 16 / nv.w32 : 2) : 0;
     const size_t smem = ssd_smem(nv, ev, sp, env != nullptr).bytes;
-    cudaStream_t s = (cudaStream_t)stream;
-    if (draws->mode == PBN_DRAW_PHILOX) sp.gdelta = geom_shortcut_delta(sp.inv, s);  // gaps are drawn with the verified shortcut
     auto launch = [&](auto kernel) -> int {
         if (int rc = fit_smem(kernel, "k_ssd", smem)) return rc;
         kernel<<<grid, PBN_BLOCK, smem, s>>>(nv, ev, dv, sp, state, chains, env0, (int)iters, (unsigned long long *)hist);
@@ -2478,6 +2596,35 @@ extern "C" int pbn_ssd(const PbnNet *net, const PbnEnv *env, uint32_t *state, in
     return dispatch(nv.kind, dv.mode, nv.ts, [&](auto NK, auto MD, auto TQ) {
         return env ? launch(k_ssd<NK, MD, TQ, true>) : launch(k_ssd<NK, MD, TQ, false>);
     });
+}
+
+extern "C" int pbn_ssd_pinned(const PbnNet *net, uint32_t *state, int64_t chains, int64_t env0, int64_t iters, double p,
+                              const uint32_t *pin_care, const uint32_t *pin_value, int32_t K, const int32_t *tgt, int32_t g,
+                              uint64_t *hist, const PbnDraws *draws, void *stream) {
+    if (!net || !state || !pin_care || !pin_value || !tgt || !hist || chains < 0 || iters < 0) return fail(PBN_ERR_ARG, "bad argument");
+    if (K < 1 || K > 65535) return fail(PBN_ERR_ARG, "1 <= K <= 65535 pin sets");
+    if (draws && draws->mode == PBN_DRAW_REPLAY) return fail(PBN_ERR_UNSUPPORTED, "pinned SSD estimates draw from Philox streams only");
+    cudaStream_t s = (cudaStream_t)stream;
+    SsdParams sp;
+    bool run;
+    if (int rc = ssd_prepare(net->v, chains, env0, iters, p, tgt, g, draws, s, sp, &run)) return rc;
+    if (!run) return PBN_OK;
+    NetView nv = net->v;
+    // a truth-table network whose threshold table is staged also stages the two constant entries behind it
+    if (nv.kind == PBN_NET_TT && !nv.thr_dev) nv.blob_bytes = nv.blob_fast_bytes = nv.blob_bytes + 16;
+    const DrawView dv = make_draws(draws);
+    EnvView ev;
+    memset(&ev, 0, sizeof ev);
+    const size_t smem = ssd_smem(nv, ev, sp, false, true).bytes;
+    const dim3 grid((unsigned)((chains + PBN_BLOCK - 1) / PBN_BLOCK), (unsigned)K);
+    auto launch = [&](auto kernel) -> int {
+        if (int rc = fit_smem(kernel, "k_ssd_pinned", smem)) return rc;
+        kernel<<<grid, PBN_BLOCK, smem, s>>>(nv, dv, sp, state, chains, env0, (int)iters, (unsigned long long *)hist, pin_care,
+                                             pin_value, net->tt_const);
+        CK(cudaGetLastError());
+        return PBN_OK;
+    };
+    return dispatch(nv.kind, dv.mode, nv.ts, [&](auto NK, auto, auto TQ) { return launch(k_ssd_pinned<NK, TQ>); });
 }
 
 struct HistParams { int g; short tgt[24]; };

@@ -67,15 +67,17 @@ __host__ __device__ inline IndexSmem index_smem(const EnvView &ev, int w32, bool
 }
 // k_ssd: image (without an env also the 16-byte records), cube image, 32 target words, the block histogram (smem_hist), one
 // aligned column per chain; the windowed path (sp.win) adds win flip masks per warp and the straggler-mode staging behind
-// the aligned columns: flip and coop are their distances in words from the region before them
+// the aligned columns: flip and coop are their distances in words from the region before them.  k_ssd_pinned (pin) adds
+// the free-node mask of the block's variant (w32 words) in front of the target words.
 struct SsdSmem : Smem {
-    size_t img, tgt, hist, cols;
+    size_t img, pin, tgt, hist, cols;
     int flip, coop;
 };
-__host__ __device__ inline SsdSmem ssd_smem(const NetView &nv, const EnvView &ev, const SsdParams &sp, bool env) {
+__host__ __device__ inline SsdSmem ssd_smem(const NetView &nv, const EnvView &ev, const SsdParams &sp, bool env, bool pin = false) {
     SsdSmem L;
     L.bytes = L.image = env ? nv.blob_bytes : nv.blob_fast_bytes;
     L.img = L.add(env ? ev.img_bytes : 0);
+    L.pin = L.add(pin ? (size_t)nv.w32 * 4 : 0);
     L.tgt = L.add(32 * 4);
     L.hist = L.add((size_t)(sp.smem_hist ? 1 << sp.g : 0) * 4);
     L.flip = nv.w32 * PBN_BLOCK;

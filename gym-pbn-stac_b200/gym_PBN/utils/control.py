@@ -8,11 +8,18 @@ detection to (utils/get_attractors_from_cabean.py), solves source-target control
   attractor_transitions      estimates that table on the GPU (env.step kernels + pbn_env_attractor_index)
   attractor_policy           value iteration on the estimated attractor-level MDP (host, NumPy)
   evaluate_attractor_policy  runs a policy table on the real PBNVectorEnv: the Monte-Carlo truth for its prediction
+
+Permanent control holds genes at fixed values instead (structural interventions: knockout = 0, overexpression = 1):
+
+  pinned_ssd                 steady-state histograms of the network under many pin sets at once (pbn_ssd_pinned)
+  rank_pins                  every single-gene knockout and overexpression, ranked by the SSD mass it moves onto
+                             env.target_node_values (the measure of utils.eval.eval_increase)
 """
 import numpy as np
 import torch
 
 from gym_PBN.b200 import abi, engine
+from gym_PBN.b200 import dist as pdist
 
 
 def _target_env(env, multi_ok):
@@ -161,3 +168,106 @@ def evaluate_attractor_policy(env, action_table, target, episodes, seed=0):
             reached |= live & (cls == target)
             failed |= live & (cls < 0)
         return float(reached.double().mean()), float(steps.double().mean())
+
+
+def _node_index(env, net, node):
+    """A node index, or a gene id of the env's graph (resolved as target_node_indices does)."""
+    ids = env.graph.getIDs() if env is not None and hasattr(getattr(env, "graph", None), "getIDs") else None
+    if ids is not None and node in ids:
+        return ids.index(node)
+    if isinstance(node, (int, np.integer)) and 0 <= int(node) < net.n:
+        return int(node)
+    raise ValueError(f"{node!r} is neither a gene id of the env nor a node index in [0, {net.n})")
+
+
+def pinned_ssd(env_or_network, pins, iters, chains, bit_flip_prob=0.01, target_nodes=None, seed=0, distributed=False):
+    """Visit histograms of the target-gene patterns under each pin set of `pins`, from one launch per iteration chunk.
+
+    env_or_network: an env (its network; target_nodes default to env.target_node_indices) or an engine.Network.
+    pins: list of {node: 0 or 1} dicts, node = node index or gene id (Bittner envs); {} = the network unpinned.
+    A variant holds its pinned nodes at their values: they are set before the first iteration, an update that picks one
+    leaves it as it is, and perturbations skip it.  Otherwise every iteration is the one of utils.eval.ssd_histogram without
+    an env: count the pattern, flip each gene w.p. bit_flip_prob, one asynchronous update (include/pbn_b200.h:
+    pbn_ssd_pinned).  Every variant starts from the same uniform random states (Graph.genRandState) and runs on the same
+    random numbers, so differences between rows are not drowned in independent sampling noise, and the row of {} is
+    utils.eval.ssd_histogram's estimate for those start states.  With distributed=True chains are sharded over ranks by
+    global chain id (multiples of 32) and the histograms are summed.
+
+    Returns int64 [K][2^g] (NumPy), bucket = target-node bits, first target most significant; each row sums to
+    iters * chains."""
+    from gym_PBN.utils.eval import MAX_ITERS_PER_LAUNCH
+
+    env = None if isinstance(env_or_network, engine.Network) else getattr(env_or_network, "unwrapped", env_or_network)
+    net = env_or_network if env is None else env.network
+    if target_nodes is None:
+        if env is None:
+            raise ValueError("target_nodes are needed with a bare network")
+        target_nodes = env.target_node_indices
+    tgt = np.asarray([_node_index(env, net, t) for t in target_nodes], np.int32)
+    pins = list(pins)
+    K = len(pins)
+    if not 1 <= K <= 65535:
+        raise ValueError("1 <= len(pins) <= 65535 pin sets")
+    care = np.zeros((K, net.w32), np.uint32)
+    value = np.zeros((K, net.w32), np.uint32)
+    for k, pin in enumerate(pins):
+        for node, v in dict(pin).items():
+            if v not in (0, 1):
+                raise ValueError(f"pinned values are 0 or 1, got {v!r}")
+            i = _node_index(env, net, node)
+            care[k, i >> 5] |= np.uint32(1 << (i & 31))
+            value[k, i >> 5] |= np.uint32(int(v) << (i & 31))
+    start, stop = pdist.shard_range(chains, align=32) if distributed else (0, int(chains))
+    local = stop - start
+    hist = torch.zeros((K, 1 << len(tgt)), dtype=torch.int64, device=net.device)
+    if local > 0:
+        sim = engine.Simulator(net, local, seed=seed, env0=start)
+        with engine.on_device(net.device):
+            sim.rand_state()
+            state = sim.state.repeat(1, K)  # column k * local + c: chain c of variant k, one start per chain
+            left = int(iters)
+            while left > 0:
+                chunk = min(left, MAX_ITERS_PER_LAUNCH)
+                engine.ssd_pinned(sim, state, chunk, bit_flip_prob, tgt, care, value, hist)
+                left -= chunk
+    if distributed:
+        pdist.allreduce_sum_(hist)
+    return hist.cpu().numpy()
+
+
+def _bucket_ids(patterns, g, what):
+    """Histogram buckets of target-gene patterns (first target most significant)."""
+    out = []
+    for p in patterns or ():
+        if len(p) != g or any(b not in (0, 1) for b in p):
+            raise ValueError(f"env.{what} must hold patterns of {g} target-gene values 0/1, got {p!r}")
+        out.append(int("".join(str(int(b)) for b in p), 2))
+    return out
+
+
+def rank_pins(env, genes=None, iters=4000, chains=300, bit_flip_prob=0.01, seed=0):
+    """Every single-gene pin (gene -> 0, gene -> 1) of `genes` (gene ids or node indices; default every node), ranked by the
+    change of steady-state mass on env.target_node_values against the unpinned network: eval_increase's measure, with the
+    pin in place of a controller.  One pinned_ssd launch estimates all 1 + 2 * len(genes) variants on common random numbers;
+    the default budget is the reference's (1.2e6 iterations per SSD: 300 chains x 4000).
+
+    Returns {"unpinned": {"target_mass", "undesired_mass"}, "ranking": [...]}: one dict per pin with "gene" (id or index as
+    given), "node" (index), "value", "target_mass", "undesired_mass" (mass on env.undesired_node_values) and "increase"
+    (target_mass minus the unpinned one), best first."""
+    env = getattr(env, "unwrapped", env)
+    net = env.network
+    if genes is None:
+        genes = list(env.graph.getIDs()) if hasattr(getattr(env, "graph", None), "getIDs") else list(range(net.n))
+    genes = list(genes)
+    pins = [{}] + [{g: v} for g in genes for v in (0, 1)]
+    hist = pinned_ssd(env, pins, iters, chains, bit_flip_prob=bit_flip_prob, seed=seed).astype(np.float64)
+    mass = hist / hist.sum(1, keepdims=True)
+    g = len(env.target_node_indices)
+    good = _bucket_ids(env.target_node_values, g, "target_node_values")
+    bad = _bucket_ids(env.undesired_node_values, g, "undesired_node_values")
+    tm, um = mass[:, good].sum(1), mass[:, bad].sum(1)
+    ranking = [{"gene": pin_gene, "node": _node_index(env, net, pin_gene), "value": v, "target_mass": float(tm[k]),
+                "undesired_mass": float(um[k]), "increase": float(tm[k] - tm[0])}
+               for k, (pin_gene, v) in enumerate(((g, v) for g in genes for v in (0, 1)), start=1)]
+    ranking.sort(key=lambda r: -r["increase"])
+    return {"unpinned": {"target_mass": float(tm[0]), "undesired_mass": float(um[0])}, "ranking": ranking}

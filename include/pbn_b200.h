@@ -227,6 +227,28 @@ int pbn_ssd(const PbnNet *net, const PbnEnv *env, uint32_t *state, int64_t chain
             double bit_flip_prob, const int32_t *tgt_nodes_host, int32_t g, uint64_t *hist, const PbnDraws *draws,
             void *stream);
 
+/* K3 without an env under K pin sets at once: the steady state of the network with genes held at fixed values, for each of
+   K variants (structural interventions: knockout = pinned at 0, overexpression = pinned at 1).  This serves
+   gym_PBN.utils.control.pinned_ssd / rank_pins; the reference has no such call.
+   Variant k pins the nodes set in care[k] to their bits in value[k] (value bits outside care, and bits at or above N, are
+   ignored).  One iteration of a variant is the iteration of pbn_ssd with env = NULL (count the bucket, perturb, one
+   asynchronous update), changed in three ways:
+     1. before the first iteration every pinned node is set to its value;
+     2. an update that picks a pinned node consumes its draws as usual (node index, predictor or table draw) and the node
+        keeps its value: the pinned node's function is the constant;
+     3. a perturbation event on a pinned node is drawn as usual and not applied.
+   Chain c of every variant draws from the update and perturbation streams of chain id env0 + c: the variants run on common
+   random numbers, and a variant without pins reproduces pbn_ssd on the same draws, env0 and start states bit for bit.
+     state      planes [W32][K * chains]: column k * chains + c = chain c of variant k (in: start states, out: final states)
+     pin_care   device uint32 [K][W32]
+     pin_value  device uint32 [K][W32]
+     hist       uint64 [K][2^g], accumulated
+   The argument rules of pbn_ssd apply (g, bit_flip_prob, env0 % 32 with bit_flip_prob > 0, iteration limits), and
+   1 <= K <= 65535 (PBN_ERR_ARG otherwise).  Replay draws give PBN_ERR_UNSUPPORTED. */
+int pbn_ssd_pinned(const PbnNet *net, uint32_t *state, int64_t chains, int64_t env0, int64_t iters, double bit_flip_prob,
+                   const uint32_t *pin_care, const uint32_t *pin_value, int32_t K, const int32_t *tgt_nodes_host, int32_t g,
+                   uint64_t *hist, const PbnDraws *draws, void *stream);
+
 /* hist[bucket(state_e)] += 1 for every env e — the first two lines of an _ssd_run iteration (utils/eval.py:88-89) as a
    stand-alone kernel, for estimates whose actions come from a policy between steps (eval.py:97-101). */
 int pbn_bucket_hist(const uint32_t *state, int64_t B, int32_t n_nodes, const int32_t *tgt_nodes_host, int32_t g,
