@@ -231,6 +231,8 @@ extern "C" int pbn_env_create(const PbnNet *net, const PbnEnvDesc *d, PbnEnv **o
     if (self_trig && (!d->gamma_pow || d->n_gamma < 1 || d->max_interval < 0))
         return fail(PBN_ERR_ARG, "self-triggering envs need the gamma**i table and T >= 0");
     const int n = net->v.n, w32 = net->v.w32;
+    // control="write" stores the control vector into nodes 0..M-1 of the env's own state column: M > N would write past it
+    if (d->n_control < 0 || d->n_control > n) return fail(PBN_ERR_ARG, "n_control must be in 0..n_nodes");
     PbnEnv *env = new PbnEnv();
     env->net = net;
     EnvView &v = env->v;
@@ -299,10 +301,12 @@ __device__ __forceinline__ void resolve_epoch(DrawView &dv) {
 }
 
 // An intervention on node `pos`; an index outside the network (a policy network can emit anything) is ignored and counted —
-// it must not flip a bit of a neighbouring env's column or of the staged network image.
-__device__ __forceinline__ void flip_node(const Col &st, int pos, int n, int &bad) {
-    if (pos >= 0 && pos < n) st.flip((u32)pos);
-    else bad++;
+// it must not flip a bit of a neighbouring env's column or of the staged network image.  Returns 1 iff the flip was applied:
+// an ignored intervention costs nothing either (the env.step equals one with action 0).
+__device__ __forceinline__ int flip_node(const Col &st, int pos, int n, int &bad) {
+    if (pos >= 0 && pos < n) { st.flip((u32)pos); return 1; }
+    bad++;
+    return 0;
 }
 
 // ---- shared-memory accesses by 32-bit shared-window address (the hot SSD loop keeps its base addresses in registers;
@@ -947,10 +951,10 @@ __global__ void __launch_bounds__(PBN_BLOCK, 4) k_env_step(NetView nv, EnvView e
     switch (ev.kind) {
     case PBN_ENV_PBN: {  // pbn_env.py:141-154, reward :171-183
         int a = act[0];
-        if (a != 0) flip_node(st, a, nv.n, bad);  // flips index `action` itself (Q3)
+        const int cost = a != 0 ? flip_node(st, a, nv.n, bad) : 0;  // flips index `action` itself (Q3)
         update(); in = 1;
         if (match_range_sa(cv, ev.tgt_first, ev.tgt_first + ev.n_tgt)) { rew = 20; tm = 1; }
-        else rew = -4 - (a != 0);
+        else rew = -4 - cost;
     } break;
     case PBN_ENV_PBCN: {  // pbcn_env.py:67-80
         int a = act[0];
@@ -961,10 +965,10 @@ __global__ void __launch_bounds__(PBN_BLOCK, 4) k_env_step(NetView nv, EnvView e
     case PBN_ENV_PBN_SD: {  // sampled_data.py:52-88
         int a = act[0], interval = act[1];
         for (int i = 0; i < interval; i++) {
-            if (a != 0) flip_node(st, a - 1, nv.n, bad);
+            const int cost = a != 0 ? flip_node(st, a - 1, nv.n, bad) : 0;
             update(); in++;
             if (match_range_sa(cv, ev.tgt_first, ev.tgt_first + ev.n_tgt)) { rew += 20; tm = 1; }
-            else { rew += -4 - (a != 0); tm = 0; }
+            else { rew += -4 - cost; tm = 0; }
         }
     } break;
     case PBN_ENV_PBCN_SD: {  // sampled_data.py:139-189
@@ -1010,10 +1014,10 @@ __global__ void __launch_bounds__(PBN_BLOCK, 4) k_env_step(NetView nv, EnvView e
         while (!end) {
             int r;
             if (!pbcn) {
-                if (a != 0) flip_node(st, a - 1, nv.n, bad);
+                const int cost = a != 0 ? flip_node(st, a - 1, nv.n, bad) : 0;
                 update();
                 if (match_range_sa(cv, ev.tgt_first, ev.tgt_first + ev.n_tgt)) { r = 20; tm = 1; }
-                else { r = -4 - (a != 0); tm = 0; }
+                else { r = -4 - cost; tm = 0; }
             } else {
                 cw.apply(ev, st);
                 update();
@@ -1091,7 +1095,7 @@ __device__ __forceinline__ bool is_attracting_flat(const EnvView &ev, const int 
 // ---- pieces of one env.step of the step-until-attractor envs, shared by the kernels below
 // the intervention: pbn_target.py:261-269 (one node) / pbn_target_multi.py:120-134 (a set of nodes, the observation captured
 // BEFORE the first update).  An env.step with an out-of-range node is counted here, once, whichever pass finishes it.
-// Returns the pending action cost (MULTI: -len(actions)).
+// Returns the pending action cost (MULTI: -len(actions), the ignored slots left out).
 __device__ __forceinline__ int att_begin(const NetView &nv, const EnvView &ev, const VecView &vx, unsigned long long *s_stats,
                                          const Col &st, const Col &ob, const int *act, int K) {
     int bad = 0, cnt = 0;
@@ -1107,8 +1111,7 @@ __device__ __forceinline__ int att_begin(const NetView &nv, const EnvView &ev, c
                 for (int j = 0; j < k; j++) dup |= (act[j] == a);
                 if (dup) continue;
             }
-            cnt++;
-            if (a != 0) flip_node(st, a - 1, nv.n, bad);
+            cnt += a != 0 ? flip_node(st, a - 1, nv.n, bad) : 1;  // an ignored slot is not an action: it costs nothing
         }
         for (int w = 0; w < nv.w32; w++) ob.set_word(w, st.word(w));  // observation captured BEFORE the update (:133)
     }

@@ -143,8 +143,10 @@ int pbn_env_step_f64(const PbnEnv *env, uint32_t *state, int32_t *n_steps, const
 
 /* Vector-env step: K2 plus, in the same launch, the bookkeeping a batched env needs — running episode return/length,
    block-aggregated statistics (episodes, return sum, length sum, successes, inner-cap hits, env steps, env steps whose
-   intervention was out of range and therefore ignored, reserved; accumulated into stats[8]), the step's observation copied to final_obs, and for finished envs the reset (reset_draws, its own epoch), after
-   which obs_state holds the NEW state of those envs.  Bit-identical to pbn_env_step followed by a masked pbn_env_reset.
+   intervention was out of range and therefore ignored, reserved; accumulated into stats[8]), the step's observation copied to
+   final_obs, and for finished envs the reset (reset_draws, its own epoch), after which obs_state holds the NEW state of those
+   envs.  An ignored intervention is neither applied nor charged for: the env.step equals one with action 0 (MULTI: one with
+   that slot absent).  Bit-identical to pbn_env_step followed by a masked pbn_env_reset.
    The reference has no vector env (SURVEY.md §2.1); this serves gym_PBN.b200.vector_env.PBNVectorEnv.step. */
 typedef struct {
     int64_t *ep_return;     /* [B] */

@@ -903,17 +903,22 @@ def test_vector_env_curriculum_matches_oracle(sample_pair, plan):
     assert torch.equal(vec.step(act)[0].clone(), vec2.step(act)[0]) and torch.equal(vec.probabilities, vec2.probabilities)
 
 
-@pytest.mark.parametrize("family", ["target", "multi"])
+@pytest.mark.parametrize("family", ["target", "multi", "pbn_sd", "pbcn_sd"])
 def test_vector_env_cuda_graph_step_is_bit_identical(family):
     """cuda_graph=True: step() replays one captured graph (the planned step launches + unpack + epoch increment, epoch in
-    device memory) — same observations, rewards, flags and statistics as the eager env, resets and reloads in between."""
+    device memory) — same observations, rewards, flags and statistics as the eager env, resets and reloads in between.  The
+    sampled-data envs run k_env_step, which reads its epochs from device memory too."""
     import gym_PBN
     from gym_PBN.b200.vector_env import PBNVectorEnv
 
-    z = load("b28_target_env.npz" if family == "target" else "b28_multi_env.npz")
-    atts = cubes_to_attractors(z["att_cubes"], z["att_off"])
-    env = gym_PBN.make("gym-PBN/Bittner-28-v0" if family == "target" else "gym-PBN/BittnerMulti-28-v0", all_attractors=atts,
-                       max_inner_steps=200)
+    if family in ("target", "multi"):
+        z = load("b28_target_env.npz" if family == "target" else "b28_multi_env.npz")
+        atts = cubes_to_attractors(z["att_cubes"], z["att_off"])
+        env = gym_PBN.make("gym-PBN/Bittner-28-v0" if family == "target" else "gym-PBN/BittnerMulti-28-v0", all_attractors=atts,
+                           max_inner_steps=200)
+    else:
+        env = gym_PBN.make("gym-PBN/PBN-sampled-data-v0" if family == "pbn_sd" else "gym-PBN/PBCN-sampled-data-v0",
+                           logic_func_data=EX5, goal_config=dict(GOAL), T=8)
     B, seed = 3000, 5
     kw = dict(curriculum=True, action_slots=2) if family == "multi" else {}
     a, b = PBNVectorEnv(env, B, seed=seed, **kw), PBNVectorEnv(env, B, seed=seed, cuda_graph=True, **kw)
@@ -922,8 +927,10 @@ def test_vector_env_cuda_graph_step_is_bit_identical(family):
     assert torch.equal(oa, ob)
     rng = np.random.default_rng(1)
     width = a.action_width
+    # (lowest, highest + 1) per action column: (node, interval 1..8) | (interval, control bits) | node ids
+    lo, hi = {"pbn_sd": ([0, 1], [6, 9]), "pbcn_sd": ([1] + [0] * (width - 1), [9] + [2] * (width - 1))}.get(family, (0, 29))
     for t in range(12):
-        act = torch.from_numpy(rng.integers(0, 29, size=(B, width)).astype(np.int32))
+        act = torch.from_numpy(rng.integers(lo, hi, size=(B, width)).astype(np.int32))
         ra, rb = a.step(act), b.step(act)
         for x, y in zip(ra[:4], rb[:4]):
             assert torch.equal(x, y), t
