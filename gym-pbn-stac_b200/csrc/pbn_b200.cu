@@ -1981,15 +1981,62 @@ __global__ void __launch_bounds__(PBN_BLOCK, HAS_ENV ? 3 : PBN_SSD_MIN_BLOCKS) k
     }
 }
 
-// k_ssd (no env, Philox draws) under K pin sets (pbn_ssd_pinned): variant k owns blocks (x, k), its chain c is state column
-// k * chains + c and draws from the streams of chain id env0 + c, as in k_ssd.  A pin acts through the block's copy of the
-// network image, where the pinned node's function becomes the constant (an update that picks it draws as usual), and through
-// the perturbation events, whose bit is masked with the variant's free nodes where it is formed.
+// A 16-bit predictor LUT (or its doubled 32-bit form) whose index bit b reads the constant c: every entry takes the value of
+// its partner with bit b = c.  M = the indices with bit b clear, s = the distance to their partners.
+__device__ __forceinline__ u32 lut_fold(u32 lut, u32 b, u32 c) {
+    const u32 M = b == 0 ? 0x55555555u : (b == 1 ? 0x33333333u : (b == 2 ? 0x0F0F0F0Fu : 0x00FF00FFu));
+    const u32 s = 1u << b;
+    return c ? (lut & ~M) | ((lut & ~M) >> s) : (lut & M) | ((lut & M) << s);
+}
+
+// Edge pin (src -> dst, c) on the block's copy of the image: node dst's function reads c in place of node src; src not an
+// input of dst: nothing changes.  A second pin of the same edge changes nothing either (it folds a bit the function no
+// longer depends on), so the first entry of a row applies.  Called, not inlined, with the image fields by value: inlined,
+// or given the kernel's NetView, it changes how ptxas schedules the SSD loop of k_ssd_pinned behind the patch.
+//   Predictor networks fold LUT bit 3 - j of each of dst's fmax records (padding records too) whose input byte j is src,
+//   in the 8-byte records and, when present, both halves of the doubled LUT of the 16-byte ones.
+//   Truth-table networks (threshold table staged) fold index bit k - 1 - j of dst's 2^k thresholds where its input j is
+//   src, in place: an entry the fold reads is never written by it.
+struct FoldImage { unsigned char *blob; int off_rec, off_rec16, fmax, off_node, off_in, off_thr; };
+template <int NET>
+__device__ __noinline__ void fold_edge(FoldImage im, u32 dst, u32 src, u32 c) {
+    if constexpr (NET == PBN_NET_PRED) {
+        uint2 *rec = reinterpret_cast<uint2 *>(im.blob + im.off_rec) + dst * im.fmax;
+        uint4 *r16 = reinterpret_cast<uint4 *>(im.blob + im.off_rec16) + dst * im.fmax;
+        for (int k = 0; k < im.fmax; k++)
+            for (u32 j = 0; j < 4; j++) {
+                if (((rec[k].x >> (8 * j)) & 0xFFu) != src) continue;
+                rec[k].y = lut_fold(rec[k].y, 3u - j, c);
+                if (im.off_rec16) r16[k].z = lut_fold(r16[k].z, 3u - j, c);
+            }
+    } else {
+        const uint2 nr = reinterpret_cast<const uint2 *>(im.blob + im.off_node)[dst];
+        const unsigned short *in = reinterpret_cast<const unsigned short *>(im.blob + im.off_in) + (nr.y & 0xFFFFu);
+        u32 *thr = reinterpret_cast<u32 *>(im.blob + im.off_thr) + nr.x;
+        const u32 k = nr.y >> 16;
+        for (u32 j = 0; j < k; j++) {
+            if (in[j] != src) continue;
+            const u32 s = 1u << (k - 1u - j);
+            for (u32 idx = 0; idx < (1u << k); idx++)
+                if (!(idx & s)) {
+                    if (c) thr[idx] = thr[idx | s];
+                    else thr[idx | s] = thr[idx];
+                }
+        }
+    }
+}
+
+// k_ssd (no env, Philox draws) under K pin sets (pbn_ssd_pinned_edges): variant k owns blocks (x, k), its chain c is state
+// column k * chains + c and draws from the streams of chain id env0 + c, as in k_ssd.  A pin acts through the block's copy of
+// the network image, where the pinned node's function becomes the constant (an update that picks it draws as usual) and an
+// edge pin folds the input it pins out of its target's function, and through the perturbation events, whose bit is masked
+// with the variant's free nodes where it is formed.  The edge row of variant k is pin_edges[k * E .. k * E + E).
 template <int NET, int TQ>
 __global__ void __launch_bounds__(PBN_BLOCK, PBN_SSD_MIN_BLOCKS) k_ssd_pinned(NetView nv, DrawView dv, SsdParams sp, u32 *state,
                                                                               long long chains, long long env0, int iters,
                                                                               unsigned long long *hist, const u32 *pin_care,
-                                                                              const u32 *pin_value, u32 tt_const) {
+                                                                              const u32 *pin_value, u32 tt_const,
+                                                                              const u32 *pin_edges, int E) {
     EnvView ev;
     memset(&ev, 0, sizeof ev);
     unsigned char *blob = smem_raw;
@@ -2012,9 +2059,20 @@ __global__ void __launch_bounds__(PBN_BLOCK, PBN_SSD_MIN_BLOCKS) k_ssd_pinned(Ne
     }
     if (sp.smem_hist)
         for (int b = threadIdx.x; b < nb; b += PBN_BLOCK) shist[b] = 0;
-    __syncthreads();  // the image is staged: patch the records of the pinned nodes
+    __syncthreads();  // the image is staged: fold the pinned edges of the free nodes, patch the records of the pinned ones
+    // (edge entry dst | src << 12 | c << 24, 0xFFFFFFFF = empty: 12 bits hold every node index that gets here, as predictor
+    // networks have at most 256 nodes and a staged threshold table at most 4096 entries, one or more per node)
+    const u32 *edges = pin_edges + (size_t)blockIdx.y * E;
     for (int i = threadIdx.x; i < nv.n; i += PBN_BLOCK) {
-        if (!((care[i >> 5] >> (i & 31)) & 1u)) continue;
+        if (!((care[i >> 5] >> (i & 31)) & 1u)) {
+            for (int k = 0; k < E; k++) {
+                const u32 x = edges[k];
+                if (x != 0xFFFFFFFFu && (x & 0xFFFu) == (u32)i)
+                    fold_edge<NET>(FoldImage{blob, nv.off_rec, nv.off_rec16, nv.fmax, nv.off_node, nv.off_in, nv.off_thr}, (u32)i,
+                                   (x >> 12) & 0xFFFu, (x >> 24) & 1u);
+            }
+            continue;
+        }
         const u32 v = (value[i >> 5] >> (i & 31)) & 1u;
         if constexpr (NET == PBN_NET_PRED) {  // every predictor's LUT all zeros or all ones
             uint2 *rec = reinterpret_cast<uint2 *>(blob + nv.off_rec) + i * nv.fmax;
@@ -2601,12 +2659,16 @@ extern "C" int pbn_ssd(const PbnNet *net, const PbnEnv *env, uint32_t *state, in
     });
 }
 
-extern "C" int pbn_ssd_pinned(const PbnNet *net, uint32_t *state, int64_t chains, int64_t env0, int64_t iters, double p,
-                              const uint32_t *pin_care, const uint32_t *pin_value, int32_t K, const int32_t *tgt, int32_t g,
-                              uint64_t *hist, const PbnDraws *draws, void *stream) {
+extern "C" int pbn_ssd_pinned_edges(const PbnNet *net, uint32_t *state, int64_t chains, int64_t env0, int64_t iters, double p,
+                                    const uint32_t *pin_care, const uint32_t *pin_value, int32_t K, const uint32_t *pin_edges,
+                                    int32_t E, const int32_t *tgt, int32_t g, uint64_t *hist, const PbnDraws *draws, void *stream) {
     if (!net || !state || !pin_care || !pin_value || !tgt || !hist || chains < 0 || iters < 0) return fail(PBN_ERR_ARG, "bad argument");
     if (K < 1 || K > 65535) return fail(PBN_ERR_ARG, "1 <= K <= 65535 pin sets");
+    if (E < 0 || E > 64) return fail(PBN_ERR_ARG, "0 <= E <= 64 edge slots per pin set");
+    if (E > 0 && !pin_edges) return fail(PBN_ERR_ARG, "E > 0 edge slots need pin_edges");
     if (draws && draws->mode == PBN_DRAW_REPLAY) return fail(PBN_ERR_UNSUPPORTED, "pinned SSD estimates draw from Philox streams only");
+    // folding an edge rewrites the node's thresholds, which a table read through thr_dev would need a per-variant copy of
+    if (E > 0 && net->v.thr_dev) return fail(PBN_ERR_UNSUPPORTED, "edge pins need the threshold table in shared memory (at most PBN_TT_THR_SMEM_MAX bytes)");
     cudaStream_t s = (cudaStream_t)stream;
     SsdParams sp;
     bool run;
@@ -2623,11 +2685,17 @@ extern "C" int pbn_ssd_pinned(const PbnNet *net, uint32_t *state, int64_t chains
     auto launch = [&](auto kernel) -> int {
         if (int rc = fit_smem(kernel, "k_ssd_pinned", smem)) return rc;
         kernel<<<grid, PBN_BLOCK, smem, s>>>(nv, dv, sp, state, chains, env0, (int)iters, (unsigned long long *)hist, pin_care,
-                                             pin_value, net->tt_const);
+                                             pin_value, net->tt_const, pin_edges, (int)E);
         CK(cudaGetLastError());
         return PBN_OK;
     };
     return dispatch(nv.kind, dv.mode, nv.ts, [&](auto NK, auto, auto TQ) { return launch(k_ssd_pinned<NK, TQ>); });
+}
+
+extern "C" int pbn_ssd_pinned(const PbnNet *net, uint32_t *state, int64_t chains, int64_t env0, int64_t iters, double p,
+                              const uint32_t *pin_care, const uint32_t *pin_value, int32_t K, const int32_t *tgt, int32_t g,
+                              uint64_t *hist, const PbnDraws *draws, void *stream) {
+    return pbn_ssd_pinned_edges(net, state, chains, env0, iters, p, pin_care, pin_value, K, nullptr, 0, tgt, g, hist, draws, stream);
 }
 
 struct HistParams { int g; short tgt[24]; };

@@ -446,19 +446,28 @@ class Simulator:
         return hist
 
 
-def ssd_pinned(sim: "Simulator", state, iters, bit_flip_prob, tgt_nodes, care, value, hist):
-    """pbn_ssd_pinned: the sim.B chains of `sim` (chain ids sim.env0 + c, one epoch of its stream, like Simulator.ssd) under
-    K pin sets.  state: int32 planes [W32][K * sim.B] on sim's device (column k * B + c = chain c of variant k);
+def ssd_pinned(sim: "Simulator", state, iters, bit_flip_prob, tgt_nodes, care, value, hist, edges=None):
+    """pbn_ssd_pinned_edges: the sim.B chains of `sim` (chain ids sim.env0 + c, one epoch of its stream, like Simulator.ssd)
+    under K pin sets.  state: int32 planes [W32][K * sim.B] on sim's device (column k * B + c = chain c of variant k);
     care / value: uint32 [K][W32] host arrays (variant k pins the nodes set in care[k] to their bits in value[k]);
-    hist: int64 [K][2^g] device tensor, accumulated."""
+    edges: None (no edge pins) or a uint32 [K][E] host array, E <= 64 (row k = the edge pins of variant k, entry
+    dst | src << 12 | c << 24, 0xFFFFFFFF = empty slot); hist: int64 [K][2^g] device tensor, accumulated."""
     tgt = np.ascontiguousarray(tgt_nodes, np.int32)
     care = torch.from_numpy(np.ascontiguousarray(care, np.uint32).view(np.int32)).to(sim.device)
     value = torch.from_numpy(np.ascontiguousarray(value, np.uint32).view(np.int32)).to(sim.device)
+    E, eptr = 0, None
+    if edges is not None:
+        edges = np.ascontiguousarray(edges, np.uint32)
+        if edges.ndim != 2 or edges.shape[0] != care.shape[0]:
+            raise ValueError(f"edges must be [K][E] with K = {care.shape[0]} pin sets, got shape {edges.shape}")
+        E = edges.shape[1]
+        edges = torch.from_numpy(edges.view(np.int32)).to(sim.device)
+        eptr = _ptr(edges) if E else None
     d = sim._draws()
     with on_device(sim.device):
-        abi.check(abi.lib().pbn_ssd_pinned(sim.net.handle, _ptr(state), sim.B, sim.env0, int(iters), float(bit_flip_prob),
-                                           _ptr(care), _ptr(value), care.shape[0], _np_ptr(tgt), len(tgt), _ptr(hist),
-                                           C.byref(d), _stream()))
+        abi.check(abi.lib().pbn_ssd_pinned_edges(sim.net.handle, _ptr(state), sim.B, sim.env0, int(iters),
+                                                 float(bit_flip_prob), _ptr(care), _ptr(value), care.shape[0], eptr, E,
+                                                 _np_ptr(tgt), len(tgt), _ptr(hist), C.byref(d), _stream()))
     sim.launches += 1
     return hist
 

@@ -9,11 +9,14 @@ detection to (utils/get_attractors_from_cabean.py), solves source-target control
   attractor_policy           value iteration on the estimated attractor-level MDP (host, NumPy)
   evaluate_attractor_policy  runs a policy table on the real PBNVectorEnv: the Monte-Carlo truth for its prediction
 
-Permanent control holds genes at fixed values instead (structural interventions: knockout = 0, overexpression = 1):
+Permanent control holds genes at fixed values instead (structural interventions: knockout = 0, overexpression = 1), or
+blocks or forces single regulatory interactions (edge pins: the target gene's function reads a constant for one input):
 
-  pinned_ssd                 steady-state histograms of the network under many pin sets at once (pbn_ssd_pinned)
+  pinned_ssd                 steady-state histograms of the network under many pin sets at once (pbn_ssd_pinned_edges)
   rank_pins                  every single-gene knockout and overexpression, ranked by the SSD mass it moves onto
                              env.target_node_values (the measure of utils.eval.eval_increase)
+  regulatory_edges           the (src, dst) pairs of the network: src is read by some function of dst
+  rank_edge_pins             every single-edge pin (src -> dst read as 0, as 1), ranked the same way
 """
 import numpy as np
 import torch
@@ -186,9 +189,12 @@ def pinned_ssd(env_or_network, pins, iters, chains, bit_flip_prob=0.01, target_n
     env_or_network: an env (its network; target_nodes default to env.target_node_indices) or an engine.Network.
     pins: list of {node: 0 or 1} dicts, node = node index or gene id (Bittner envs); {} = the network unpinned.
     A variant holds its pinned nodes at their values: they are set before the first iteration, an update that picks one
-    leaves it as it is, and perturbations skip it.  Otherwise every iteration is the one of utils.eval.ssd_histogram without
-    an env: count the pattern, flip each gene w.p. bit_flip_prob, one asynchronous update (include/pbn_b200.h:
-    pbn_ssd_pinned).  Every variant starts from the same uniform random states (Graph.genRandState) and runs on the same
+    leaves it as it is, and perturbations skip it.  A key (src, dst), both ends resolved as node keys are, pins that edge
+    of regulatory_edges: whenever dst is updated its function reads the pinned value in place of src (src itself, and every
+    other node that reads it, are unchanged); a pair that is not an edge raises ValueError.  Up to 64 edge pins per
+    variant; truth-table networks with more than 16 KB of threshold table take none.  Otherwise every iteration is the one
+    of utils.eval.ssd_histogram without an env: count the pattern, flip each gene w.p. bit_flip_prob, one asynchronous
+    update (include/pbn_b200.h: pbn_ssd_pinned_edges).  Every variant starts from the same uniform random states (Graph.genRandState) and runs on the same
     random numbers, so differences between rows are not drowned in independent sampling noise, and the row of {} is
     utils.eval.ssd_histogram's estimate for those start states.  With distributed=True chains are sharded over ranks by
     global chain id (multiples of 32) and the histograms are summed.
@@ -210,13 +216,33 @@ def pinned_ssd(env_or_network, pins, iters, chains, bit_flip_prob=0.01, target_n
         raise ValueError("1 <= len(pins) <= 65535 pin sets")
     care = np.zeros((K, net.w32), np.uint32)
     value = np.zeros((K, net.w32), np.uint32)
+    rows, known = [], None
     for k, pin in enumerate(pins):
+        row = []
         for node, v in dict(pin).items():
             if v not in (0, 1):
                 raise ValueError(f"pinned values are 0 or 1, got {v!r}")
+            if isinstance(node, tuple) and len(node) == 2:
+                src, dst = (_node_index(env, net, x) for x in node)
+                if known is None:
+                    known = set(_edge_nodes(net.spec))
+                if (src, dst) not in known:
+                    raise ValueError(f"{node!r} is not a regulatory edge (src, dst) of the network: no function of "
+                                     f"{node[1]!r} reads {node[0]!r}")
+                row.append(dst | src << 12 | int(v) << 24)
+                continue
             i = _node_index(env, net, node)
             care[k, i >> 5] |= np.uint32(1 << (i & 31))
             value[k, i >> 5] |= np.uint32(int(v) << (i & 31))
+        rows.append(row)
+    E = max(len(r) for r in rows)
+    if E > 64:
+        raise ValueError(f"at most 64 edge pins per pin set, got {E}")
+    edges = None
+    if E:
+        edges = np.full((K, E), 0xFFFFFFFF, np.uint32)
+        for k, row in enumerate(rows):
+            edges[k, :len(row)] = row
     start, stop = pdist.shard_range(chains, align=32) if distributed else (0, int(chains))
     local = stop - start
     hist = torch.zeros((K, 1 << len(tgt)), dtype=torch.int64, device=net.device)
@@ -228,7 +254,7 @@ def pinned_ssd(env_or_network, pins, iters, chains, bit_flip_prob=0.01, target_n
             left = int(iters)
             while left > 0:
                 chunk = min(left, MAX_ITERS_PER_LAUNCH)
-                engine.ssd_pinned(sim, state, chunk, bit_flip_prob, tgt, care, value, hist)
+                engine.ssd_pinned(sim, state, chunk, bit_flip_prob, tgt, care, value, hist, edges=edges)
                 left -= chunk
     if distributed:
         pdist.allreduce_sum_(hist)
@@ -243,6 +269,21 @@ def _bucket_ids(patterns, g, what):
             raise ValueError(f"env.{what} must hold patterns of {g} target-gene values 0/1, got {p!r}")
         out.append(int("".join(str(int(b)) for b in p), 2))
     return out
+
+
+def _rank(env, pins, rows, iters, chains, bit_flip_prob, seed):
+    """The ranking of rank_pins and rank_edge_pins: pins[0] = {} and pins[k] the variant of rows[k - 1] (the identifying
+    fields of its ranking entry), all estimated by one pinned_ssd launch."""
+    hist = pinned_ssd(env, pins, iters, chains, bit_flip_prob=bit_flip_prob, seed=seed).astype(np.float64)
+    mass = hist / hist.sum(1, keepdims=True)
+    g = len(env.target_node_indices)
+    good = _bucket_ids(env.target_node_values, g, "target_node_values")
+    bad = _bucket_ids(env.undesired_node_values, g, "undesired_node_values")
+    tm, um = mass[:, good].sum(1), mass[:, bad].sum(1)
+    ranking = [dict(row, target_mass=float(tm[k]), undesired_mass=float(um[k]), increase=float(tm[k] - tm[0]))
+               for k, row in enumerate(rows, start=1)]
+    ranking.sort(key=lambda r: -r["increase"])
+    return {"unpinned": {"target_mass": float(tm[0]), "undesired_mass": float(um[0])}, "ranking": ranking}
 
 
 def rank_pins(env, genes=None, iters=4000, chains=300, bit_flip_prob=0.01, seed=0):
@@ -260,14 +301,58 @@ def rank_pins(env, genes=None, iters=4000, chains=300, bit_flip_prob=0.01, seed=
         genes = list(env.graph.getIDs()) if hasattr(getattr(env, "graph", None), "getIDs") else list(range(net.n))
     genes = list(genes)
     pins = [{}] + [{g: v} for g in genes for v in (0, 1)]
-    hist = pinned_ssd(env, pins, iters, chains, bit_flip_prob=bit_flip_prob, seed=seed).astype(np.float64)
-    mass = hist / hist.sum(1, keepdims=True)
-    g = len(env.target_node_indices)
-    good = _bucket_ids(env.target_node_values, g, "target_node_values")
-    bad = _bucket_ids(env.undesired_node_values, g, "undesired_node_values")
-    tm, um = mass[:, good].sum(1), mass[:, bad].sum(1)
-    ranking = [{"gene": pin_gene, "node": _node_index(env, net, pin_gene), "value": v, "target_mass": float(tm[k]),
-                "undesired_mass": float(um[k]), "increase": float(tm[k] - tm[0])}
-               for k, (pin_gene, v) in enumerate(((g, v) for g in genes for v in (0, 1)), start=1)]
-    ranking.sort(key=lambda r: -r["increase"])
-    return {"unpinned": {"target_mass": float(tm[0]), "undesired_mass": float(um[0])}, "ranking": ranking}
+    rows = [{"gene": g, "node": _node_index(env, net, g), "value": v} for g in genes for v in (0, 1)]
+    return _rank(env, pins, rows, iters, chains, bit_flip_prob, seed)
+
+
+def _edge_nodes(spec):
+    """The distinct (src, dst) node-index pairs of a compiled network, in (dst, input slot) order: src is an input of some
+    predictor of dst (its three regulators and dst itself), or of dst's truth table."""
+    a, out, seen = spec.arrays, [], set()
+    for dst in range(spec.n):
+        if "pr_in" in a:
+            srcs = a["pr_in"][4 * a["pr_off"][dst]:4 * a["pr_off"][dst + 1]]
+        else:
+            srcs = a["tt_in"][a["tt_in_off"][dst]:a["tt_in_off"][dst + 1]]
+        for src in srcs:
+            e = (int(src), dst)
+            if e not in seen:
+                seen.add(e)
+                out.append(e)
+    return out
+
+
+def regulatory_edges(env_or_network):
+    """The regulatory edges of a network: every distinct pair (src, dst) such that some function of node dst reads node src
+    (for predictor networks each predictor reads three regulators and dst itself, so every node has its self-input), in
+    (dst, input slot) order.  env_or_network: an env (pairs of gene ids when its graph has them, node indices otherwise), an
+    engine.Network or a compiler.NetworkSpec (node indices)."""
+    if isinstance(env_or_network, engine.Network):
+        env, spec = None, env_or_network.spec
+    elif hasattr(env_or_network, "arrays") and hasattr(env_or_network, "n"):
+        env, spec = None, env_or_network
+    else:
+        env = getattr(env_or_network, "unwrapped", env_or_network)
+        spec = env.network.spec
+    edges = _edge_nodes(spec)
+    ids = env.graph.getIDs() if env is not None and hasattr(getattr(env, "graph", None), "getIDs") else None
+    return [(ids[s], ids[d]) for s, d in edges] if ids is not None else edges
+
+
+def rank_edge_pins(env, edges=None, iters=4000, chains=300, bit_flip_prob=0.01, seed=0):
+    """Every single-edge pin ((src, dst) -> 0, -> 1) of `edges` ((src, dst) pairs of gene ids or node indices; default
+    regulatory_edges(env), self-inputs included), ranked as rank_pins ranks gene pins: by the change of steady-state mass
+    on env.target_node_values against the unpinned network.  Pinning (src, dst) at c makes dst's function read c in place
+    of src, and leaves src and every other reader of src as they are: it blocks (or forces) one interaction where a gene
+    pin removes all of the gene's.  One pinned_ssd launch estimates all 1 + 2 * len(edges) variants on common random
+    numbers (at most 65 535 variants).
+
+    Returns {"unpinned": {"target_mass", "undesired_mass"}, "ranking": [...]}: one dict per edge pin with "src", "dst" (as
+    given), "src_node", "dst_node" (indices), "value", "target_mass", "undesired_mass" and "increase", best first."""
+    env = getattr(env, "unwrapped", env)
+    net = env.network
+    edges = regulatory_edges(env) if edges is None else [tuple(e) for e in edges]
+    pins = [{}] + [{e: v} for e in edges for v in (0, 1)]
+    rows = [{"src": s, "dst": d, "src_node": _node_index(env, net, s), "dst_node": _node_index(env, net, d), "value": v}
+            for s, d in edges for v in (0, 1)]
+    return _rank(env, pins, rows, iters, chains, bit_flip_prob, seed)

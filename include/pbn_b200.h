@@ -246,10 +246,32 @@ int pbn_ssd(const PbnNet *net, const PbnEnv *env, uint32_t *state, int64_t chain
      pin_value  device uint32 [K][W32]
      hist       uint64 [K][2^g], accumulated
    The argument rules of pbn_ssd apply (g, bit_flip_prob, env0 % 32 with bit_flip_prob > 0, iteration limits), and
-   1 <= K <= 65535 (PBN_ERR_ARG otherwise).  Replay draws give PBN_ERR_UNSUPPORTED. */
+   1 <= K <= 65535 (PBN_ERR_ARG otherwise).  Replay draws give PBN_ERR_UNSUPPORTED.
+   This is pbn_ssd_pinned_edges with no edge slots (E = 0). */
 int pbn_ssd_pinned(const PbnNet *net, uint32_t *state, int64_t chains, int64_t env0, int64_t iters, double bit_flip_prob,
                    const uint32_t *pin_care, const uint32_t *pin_value, int32_t K, const int32_t *tgt_nodes_host, int32_t g,
                    uint64_t *hist, const PbnDraws *draws, void *stream);
+
+/* pbn_ssd_pinned with regulatory edges pinned as well: variant k is the node pin set (care[k], value[k]) plus up to E edge
+   pins, row k of pin_edges.  An edge pin (src, dst, c) blocks or forces one interaction: whenever node dst is updated, its
+   function reads c in place of the current bit of node src.  Nothing else changes: src itself updates and is perturbed as
+   usual, other nodes that read src see its real value, and the update of dst consumes its draws as before (node index,
+   predictor or table draw).  This serves gym_PBN.utils.control.pinned_ssd / rank_edge_pins; the reference has no such call.
+   The edges of node dst are the nodes its function reads: for predictor networks the four inputs of each of its predictors
+   (three regulators and dst itself), for truth-table networks its input list.  So:
+     - an edge pin of a node pin's node (dst pinned in care[k]) changes nothing: dst's function is already the constant;
+     - an entry whose src is not an input of dst, or whose dst is not below N, changes nothing;
+     - when a row names the same edge twice, the first entry applies.
+   With E = 0, or rows of empty slots only, every variant is pbn_ssd_pinned's, bit for bit.
+     pin_edges  device uint32 [K][E]: entry dst | src << 12 | c << 24 (c = bit 24; bits 25..31 are ignored), 0xFFFFFFFF =
+                an empty slot
+     E          0 <= E <= 64 (PBN_ERR_ARG otherwise); E > 0 needs pin_edges != NULL (PBN_ERR_ARG)
+   Every rule of pbn_ssd_pinned applies.  Truth-table networks whose threshold table is read from global memory (more than
+   16 KB of table: PBN_TT_THR_SMEM_MAX) give PBN_ERR_UNSUPPORTED with E > 0: the edge pin rewrites dst's thresholds in the
+   block's shared copy of the image, and a table outside it would need a copy per variant.  They run with E = 0. */
+int pbn_ssd_pinned_edges(const PbnNet *net, uint32_t *state, int64_t chains, int64_t env0, int64_t iters, double bit_flip_prob,
+                         const uint32_t *pin_care, const uint32_t *pin_value, int32_t K, const uint32_t *pin_edges, int32_t E,
+                         const int32_t *tgt_nodes_host, int32_t g, uint64_t *hist, const PbnDraws *draws, void *stream);
 
 /* hist[bucket(state_e)] += 1 for every env e — the first two lines of an _ssd_run iteration (utils/eval.py:88-89) as a
    stand-alone kernel, for estimates whose actions come from a policy between steps (eval.py:97-101). */
