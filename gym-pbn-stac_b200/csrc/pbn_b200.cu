@@ -1637,6 +1637,14 @@ __device__ __forceinline__ void ssd_count(SsdCount &c, const SsdLoopArgs &a, con
     c.run++;
 }
 
+// GOAL (k_passage): the count of an iteration becomes a goal test.  Bit b of the goal mask (staged where the histogram
+// would sit, a.shist) says whether bucket b lies in the goal; hit = the first iteration whose bucket does, ~0u while none
+// has (iterations ascend, so the first hit is the least)
+__device__ __forceinline__ void ssd_goal(u32 &hit, const SsdLoopArgs &a, const Col &st, u32 it) {
+    const int b = ssd_bucket(a.sp, a.s_tgt, st);
+    hit = min(hit, (a.shist[b >> 5] >> (b & 31)) & 1u ? it : ~0u);
+}
+
 // Perturbation state of the static loop.  Each event is resolved once, when its round is drawn: the iteration it is due in,
 // the shared address of the word it flips and the bit.  Checking a slot in an iteration is then a compare, a select and one
 // shared-memory XOR.  An applied event stays in its slot until the next round overwrites it: its iteration has passed, and
@@ -1717,10 +1725,12 @@ __device__ __forceinline__ void ssd_fast_perturb(const SsdFast &f, const SsdPara
 }
 
 // STATIC path of predictor networks, full warps, no attractor loop, shared histogram, targets inside one state word:
-// the configuration the headline number is measured in.  Returns the number of iterations done (even).
-template <int TQ, bool PIN = false>
+// the configuration the headline number is measured in.  Returns the number of iterations done (even), or -1 when (GOAL)
+// the warp left because every lane's chain has arrived: then nothing is handed back, as no iteration follows.
+template <int TQ, bool PIN = false, bool GOAL = false>
 __device__ __forceinline__ int ssd_loop_pred_static(const SsdLoopArgs &a, const Col &st, Draw<PBN_DRAW_PHILOX> &d,
-                                                    Draw<PBN_DRAW_PHILOX> &dp, SsdPerturb &ps0, SsdCount &cnt, const u32 *s_free = nullptr) {
+                                                    Draw<PBN_DRAW_PHILOX> &dp, SsdPerturb &ps0, SsdCount &cnt, const u32 *s_free = nullptr,
+                                                    u32 *hit = nullptr) {
     if (a.iters < 2) return 0;
     const NetView &nv = a.nv;
     SsdFast f;
@@ -1746,27 +1756,46 @@ __device__ __forceinline__ int ssd_loop_pred_static(const SsdLoopArgs &a, const 
     u32 ublk = 0;
     int t = 0;
     u32 cur = (u32)cnt.cur, run = cnt.run;
-    auto count = [&]() {
+    u32 h = 0u, c2 = d.c2, c3 = d.c3;
+    if constexpr (GOAL) {
+        h = *hit;
+        // the chain-id words of the update stream held in registers: left to ptxas, the goal loop recomputes them from
+        // the block and thread index in every trip (10 instructions)
+        c2 = keep(c2);
+        c3 = keep(c3);
+    }
+    auto count = [&](u32 it) {
         const u32 b = __brev((lds_u32(f.col + f.b_off) >> f.b_sh) << f.b_up);
-        u32 r0;  // run-length aggregation, predicated: flush the run when the bucket changes
-        asm volatile("{ .reg .pred p; setp.ne.u32 p, %1, %2; @p red.shared.add.u32 [%3], %4; selp.u32 %0, 0, %4, p; }"
-                     : "=r"(r0) : "r"(b), "r"(cur), "r"(f.shist + cur * 4u), "r"(run) : "memory");
-        cur = b;
-        run = r0 + 1u;
+        if constexpr (GOAL) {  // the goal word of bucket b, a bit test, the hit iteration selected: no atomics
+            const u32 w = lds_u32(f.shist + ((b >> 5) << 2));
+            h = min(h, (w >> (b & 31u)) & 1u ? it : ~0u);
+        } else {
+            u32 r0;  // run-length aggregation, predicated: flush the run when the bucket changes
+            asm volatile("{ .reg .pred p; setp.ne.u32 p, %1, %2; @p red.shared.add.u32 [%3], %4; selp.u32 %0, 0, %4, p; }"
+                         : "=r"(r0) : "r"(b), "r"(cur), "r"(f.shist + cur * 4u), "r"(run) : "memory");
+            cur = b;
+            run = r0 + 1u;
+        }
     };
     for (int left = a.iters >> 1; left > 0; left--, t += 2) {  // (a count-down: the bound is not re-read from the parameter bank)
+        if constexpr (GOAL) {
+            if (__all_sync(0xFFFFFFFFu, h != ~0u)) {  // no live lane: leave without handing anything back
+                *hit = h;
+                return -1;
+            }
+        }
         u32 x0, x1, x2, x3;
-        philox4x32_10_rk(ublk, d.c1, d.c2, d.c3, a.dv, x0, x1, x2, x3);
+        philox4x32_10_rk(ublk, d.c1, c2, c3, a.dv, x0, x1, x2, x3);
         ublk++;
         // the draw half of an update does not depend on the state: issued ahead of the perturbation, its two dependent
         // shared-memory loads are over when the state half needs them
         const FastDraw da = ssd_fast_draw<TQ>(f, x0, x1);
-        count();
+        count((u32)t);
         ssd_fast_perturb<PIN>(f, a.sp, ps, dp, a.dv, (u32)t, free);
         ssd_fast_apply_update(f, da);
         __syncwarp();
         const FastDraw db = ssd_fast_draw<TQ>(f, x2, x3);
-        count();
+        count((u32)t + 1u);
         ssd_fast_perturb<PIN>(f, a.sp, ps, dp, a.dv, (u32)t + 1u, free);
         ssd_fast_apply_update(f, db);
         __syncwarp();
@@ -1791,12 +1820,17 @@ __device__ __forceinline__ int ssd_loop_pred_static(const SsdLoopArgs &a, const 
     ps0.e1 = position(ps.t1, ps.a1, ps.m1);
     ps0.last_p1 = (ps.next - tu) * f.W + ps.last_p1;
     cnt.cur = (int)cur; cnt.run = run;
+    if constexpr (GOAL) *hit = h;
     return t;
 }
 
-// PIN (k_ssd_pinned): perturbation events are masked with the free-node mask s_free of the block's variant
-template <int NET, int MODE, int TQ, bool HAS_ENV, bool FULL, bool PIN = false>
-__device__ __forceinline__ void ssd_loop(const SsdLoopArgs &a, const Col &st, Draw<MODE> &d, Draw<MODE> &dp, const u32 *s_free = nullptr) {
+// PIN (k_ssd_pinned, k_passage): perturbation events are masked with the free-node mask s_free of the block's variant.
+// GOAL (k_passage): each count is a goal test recording this lane's first hit in *hit (ssd_goal), and the warp leaves the
+// loop when no lane is live (*hit != ~0u in every lane): checked once per two-iteration trip on the static paths, once per
+// iteration in the tail.
+template <int NET, int MODE, int TQ, bool HAS_ENV, bool FULL, bool PIN = false, bool GOAL = false>
+__device__ __forceinline__ void ssd_loop(const SsdLoopArgs &a, const Col &st, Draw<MODE> &d, Draw<MODE> &dp, const u32 *s_free = nullptr,
+                                         u32 *hit = nullptr) {
     const NetView &nv = a.nv;
     const SsdParams &sp = a.sp;
     const u32 lane = threadIdx.x & 31u;
@@ -1810,20 +1844,31 @@ __device__ __forceinline__ void ssd_loop(const SsdLoopArgs &a, const Col &st, Dr
     SsdCount cnt{active ? ssd_bucket(sp, a.s_tgt, st) : 0, 0u};
     int t = 0;
     if constexpr (MODE == PBN_DRAW_PHILOX && !HAS_ENV && FULL && NET == PBN_NET_PRED && TQ > 0) {
-        if (flips && sp.smem_hist && sp.fast_t0 >= 0 && nv.off_rec16) t = ssd_loop_pred_static<TQ, PIN>(a, st, d, dp, ps, cnt, s_free);
+        if (flips && sp.smem_hist && sp.fast_t0 >= 0 && nv.off_rec16) t = ssd_loop_pred_static<TQ, PIN, GOAL>(a, st, d, dp, ps, cnt, s_free, hit);
+        if constexpr (GOAL) {
+            if (t < 0) return;  // the warp left early: d, dp and ps were not handed back, and nothing follows
+        }
     }
     if constexpr (MODE == PBN_DRAW_PHILOX && !HAS_ENV && FULL) {
         // STATIC path: one Philox block of the update stream per two iterations, words used in stream order
         u32 ublk = d.blk;
         for (; t + 1 < a.iters; t += 2) {
+            if constexpr (GOAL) {
+                if (__all_sync(0xFFFFFFFFu, *hit != ~0u)) {
+                    t = a.iters;
+                    break;
+                }
+            }
             u32 x0, x1, x2, x3;
             philox4x32_10(ublk, d.c1, d.c2, d.c3, d.k0, d.k1, x0, x1, x2, x3);
             ublk++;
-            ssd_count(cnt, a, st);
+            if constexpr (GOAL) ssd_goal(*hit, a, st, (u32)t);
+            else ssd_count(cnt, a, st);
             if (flips) ssd_perturb<true, PIN>(ps, dp, warp_cols, W, inv, hmd, 32u, s_free);
             micro_step_words<NET, TQ>(nv, a.blob, st, x0, x1, d);
             __syncwarp();  // updates land before the next iteration's cross-lane flips
-            ssd_count(cnt, a, st);
+            if constexpr (GOAL) ssd_goal(*hit, a, st, (u32)t + 1u);
+            else ssd_count(cnt, a, st);
             if (flips) ssd_perturb<true, PIN>(ps, dp, warp_cols, W, inv, hmd, 32u, s_free);
             micro_step_words<NET, TQ>(nv, a.blob, st, x2, x3, d);
             __syncwarp();
@@ -1895,7 +1940,12 @@ __device__ __forceinline__ void ssd_loop(const SsdLoopArgs &a, const Col &st, Dr
         }
     }
     for (; t < a.iters; t++) {
-        if (active) ssd_count(cnt, a, st);
+        if constexpr (GOAL) {
+            if (__all_sync(0xFFFFFFFFu, *hit != ~0u)) break;
+            if (active) ssd_goal(*hit, a, st, (u32)t);
+        } else {
+            if (active) ssd_count(cnt, a, st);
+        }
         if constexpr (MODE == PBN_DRAW_REPLAY) {
             if (active)
                 for (u32 j = 0; j < n; j++)
@@ -1917,9 +1967,11 @@ __device__ __forceinline__ void ssd_loop(const SsdLoopArgs &a, const Col &st, Dr
         }
         if constexpr (MODE == PBN_DRAW_PHILOX) __syncwarp();  // updates land before the next iteration's cross-lane flips
     }
-    if (active && cnt.run) {
-        if (sp.smem_hist) atomicAdd(&a.shist[cnt.cur], cnt.run);
-        else atomicAdd(&a.hist[cnt.cur], (unsigned long long)cnt.run);
+    if constexpr (!GOAL) {
+        if (active && cnt.run) {
+            if (sp.smem_hist) atomicAdd(&a.shist[cnt.cur], cnt.run);
+            else atomicAdd(&a.hist[cnt.cur], (unsigned long long)cnt.run);
+        }
     }
 }
 
@@ -2026,43 +2078,25 @@ __device__ __noinline__ void fold_edge(FoldImage im, u32 dst, u32 src, u32 c) {
     }
 }
 
-// k_ssd (no env, Philox draws) under K pin sets (pbn_ssd_pinned_edges): variant k owns blocks (x, k), its chain c is state
-// column k * chains + c and draws from the streams of chain id env0 + c, as in k_ssd.  A pin acts through the block's copy of
-// the network image, where the pinned node's function becomes the constant (an update that picks it draws as usual) and an
-// edge pin folds the input it pins out of its target's function, and through the perturbation events, whose bit is masked
-// with the variant's free nodes where it is formed.  The edge row of variant k is pin_edges[k * E .. k * E + E).
-template <int NET, int TQ>
-__global__ void __launch_bounds__(PBN_BLOCK, PBN_SSD_MIN_BLOCKS) k_ssd_pinned(NetView nv, DrawView dv, SsdParams sp, u32 *state,
-                                                                              long long chains, long long env0, int iters,
-                                                                              unsigned long long *hist, const u32 *pin_care,
-                                                                              const u32 *pin_value, u32 tt_const,
-                                                                              const u32 *pin_edges, int E) {
-    EnvView ev;
-    memset(&ev, 0, sizeof ev);
-    unsigned char *blob = smem_raw;
-    const SsdSmem L = ssd_smem(nv, ev, sp, false, true);
-    u32 *s_free = reinterpret_cast<u32 *>(smem_raw + L.pin);
-    u32 *s_tgt = reinterpret_cast<u32 *>(smem_raw + L.tgt);
-    u32 *shist = reinterpret_cast<u32 *>(smem_raw + L.hist);
-    const int nb = 1 << sp.g;
-    u32 *sst = align_cols(shist + (sp.smem_hist ? nb : 0), nv.w32);
-    const int w32 = nv.w32;
-    const u32 *care = pin_care + (size_t)blockIdx.y * w32, *value = pin_value + (size_t)blockIdx.y * w32;
-    auto care_word = [&](int w) {  // bits at or above N are ignored
-        return (w == w32 - 1 && (nv.n & 31)) ? care[w] & ((1u << (nv.n & 31)) - 1u) : care[w];
-    };
-    stage(blob, nv.blob, L.image);
-    for (int w = threadIdx.x; w < w32; w += PBN_BLOCK) s_free[w] = ~care_word(w);
-    if (threadIdx.x == 0) {
-#pragma unroll
-        for (int k = 0; k < 24; k++) s_tgt[k] = (u32)sp.tgt[k];
-    }
-    if (sp.smem_hist)
-        for (int b = threadIdx.x; b < nb; b += PBN_BLOCK) shist[b] = 0;
-    __syncthreads();  // the image is staged: fold the pinned edges of the free nodes, patch the records of the pinned ones
-    // (edge entry dst | src << 12 | c << 24, 0xFFFFFFFF = empty: 12 bits hold every node index that gets here, as predictor
-    // networks have at most 256 nodes and a staged threshold table at most 4096 entries, one or more per node)
-    const u32 *edges = pin_edges + (size_t)blockIdx.y * E;
+// Word w of a variant's care mask: bits at or above N are ignored
+__device__ __forceinline__ u32 pin_care_word(int n, int w32, const u32 *care, int w) {
+    return (w == w32 - 1 && (n & 31)) ? care[w] & ((1u << (n & 31)) - 1u) : care[w];
+}
+
+// The pins of variant blockIdx.y (k_ssd_pinned, k_passage) on the block's copy of the image, called when the image has been
+// staged: the free-node mask s_free (read by the SSD loop behind a later barrier), the caller's other shared words
+// (`stage_rest`), then behind a block barrier the pinned edges of the free nodes folded and the records of the pinned nodes
+// patched.  `edges` is the variant's row of E edge entries.  Inlined, in this order: ptxas schedules the static SSD loop
+// of k_ssd_pinned behind it differently otherwise (109.5 instructions per iteration as a call taking the image fields by
+// value, as fold_edge does; 103, or longer perturbation rounds, when the barrier or s_free move).
+// (edge entry dst | src << 12 | c << 24, 0xFFFFFFFF = empty: 12 bits hold every node index that gets here, as predictor
+// networks have at most 256 nodes and a staged threshold table at most 4096 entries, one or more per node)
+template <int NET, class F>
+__device__ __forceinline__ void pin_patch(const NetView &nv, unsigned char *blob, u32 *s_free, const u32 *care, const u32 *value,
+                                          u32 tt_const, const u32 *edges, int E, F &&stage_rest) {
+    for (int w = threadIdx.x; w < nv.w32; w += PBN_BLOCK) s_free[w] = ~pin_care_word(nv.n, nv.w32, care, w);
+    stage_rest();
+    __syncthreads();
     for (int i = threadIdx.x; i < nv.n; i += PBN_BLOCK) {
         if (!((care[i >> 5] >> (i & 31)) & 1u)) {
             for (int k = 0; k < E; k++) {
@@ -2085,16 +2119,54 @@ __global__ void __launch_bounds__(PBN_BLOCK, PBN_SSD_MIN_BLOCKS) k_ssd_pinned(Ne
             reinterpret_cast<uint2 *>(blob + nv.off_node)[i] = make_uint2(tt_const + v, 0u);
         }
     }
+}
+
+// A chain's start state under its variant's pins: every pinned node set to its value
+__device__ __forceinline__ void pin_state(const NetView &nv, const Col &st, const u32 *care, const u32 *value) {
+    for (int w = 0; w < nv.w32; w++) {
+        const u32 c = pin_care_word(nv.n, nv.w32, care, w);
+        st.set_word(w, (st.word(w) & ~c) | (value[w] & c));
+    }
+}
+
+// k_ssd (no env, Philox draws) under K pin sets (pbn_ssd_pinned_edges): variant k owns blocks (x, k), its chain c is state
+// column k * chains + c and draws from the streams of chain id env0 + c, as in k_ssd.  A pin acts through the block's copy of
+// the network image, where the pinned node's function becomes the constant (an update that picks it draws as usual) and an
+// edge pin folds the input it pins out of its target's function, and through the perturbation events, whose bit is masked
+// with the variant's free nodes where it is formed (pin_patch).
+template <int NET, int TQ>
+__global__ void __launch_bounds__(PBN_BLOCK, PBN_SSD_MIN_BLOCKS) k_ssd_pinned(NetView nv, DrawView dv, SsdParams sp, u32 *state,
+                                                                              long long chains, long long env0, int iters,
+                                                                              unsigned long long *hist, const u32 *pin_care,
+                                                                              const u32 *pin_value, u32 tt_const,
+                                                                              const u32 *pin_edges, int E) {
+    EnvView ev;
+    memset(&ev, 0, sizeof ev);
+    unsigned char *blob = smem_raw;
+    const SsdSmem L = ssd_smem(nv, ev, sp, false, true);
+    u32 *s_free = reinterpret_cast<u32 *>(smem_raw + L.pin);
+    u32 *s_tgt = reinterpret_cast<u32 *>(smem_raw + L.tgt);
+    u32 *shist = reinterpret_cast<u32 *>(smem_raw + L.hist);
+    const int nb = 1 << sp.g;
+    u32 *sst = align_cols(shist + (sp.smem_hist ? nb : 0), nv.w32);
+    const int w32 = nv.w32;
+    const u32 *care = pin_care + (size_t)blockIdx.y * w32, *value = pin_value + (size_t)blockIdx.y * w32;
+    stage(blob, nv.blob, L.image);
+    pin_patch<NET>(nv, blob, s_free, care, value, tt_const, pin_edges + (size_t)blockIdx.y * E, E, [&] {
+        if (threadIdx.x == 0) {
+#pragma unroll
+            for (int k = 0; k < 24; k++) s_tgt[k] = (u32)sp.tgt[k];
+        }
+        if (sp.smem_hist)
+            for (int b = threadIdx.x; b < nb; b += PBN_BLOCK) shist[b] = 0;
+    });
     const long long e = (long long)blockIdx.x * PBN_BLOCK + threadIdx.x;
     const long long B = (long long)gridDim.y * chains, col = (long long)blockIdx.y * chains + e;
     Col st{sst + threadIdx.x};
     const bool active = e < chains;
     if (active) {
         load_state(st, state, B, col, w32);
-        for (int w = 0; w < w32; w++) {
-            const u32 c = care_word(w);
-            st.set_word(w, (st.word(w) & ~c) | (value[w] & c));
-        }
+        pin_state(nv, st, care, value);
     }
     __syncthreads();
     unsigned long long *vhist = hist + ((size_t)blockIdx.y << sp.g);
@@ -2113,6 +2185,68 @@ __global__ void __launch_bounds__(PBN_BLOCK, PBN_SSD_MIN_BLOCKS) k_ssd_pinned(Ne
         __syncthreads();
         for (int b = threadIdx.x; b < nb; b += PBN_BLOCK)
             if (shist[b]) atomicAdd(&vhist[b], (unsigned long long)shist[b]);
+    }
+}
+
+// The goal of k_passage: bit b (bit b & 31 of word b >> 5) = bucket b lies in the goal, 2^g <= 4096 buckets.  A parameter
+// of its own rather than a field of SsdParams, whose size sets the parameter offsets of every k_ssd instantiation.
+struct GoalMask { u32 w[128]; };
+
+// First passage into the goal (pbn_first_passage): k_ssd_pinned's chains, variants and draws, with the count of each
+// iteration replaced by a goal test (ssd_loop's GOAL).  The goal mask is staged where k_ssd_pinned keeps its histogram.
+// t_hit [K][chains] (index = state column): a chain whose entry is >= 0 has arrived and is neither run nor written (its lane
+// still draws the warp's perturbation stream); any other gets t0 + its first hit, or keeps -1 and has its state stored.
+template <int NET, int TQ>
+__global__ void __launch_bounds__(PBN_BLOCK, PBN_SSD_MIN_BLOCKS) k_passage(NetView nv, DrawView dv, SsdParams sp, u32 *state,
+                                                                           long long chains, long long env0, int iters,
+                                                                           long long t0, long long *t_hit, const u32 *pin_care,
+                                                                           const u32 *pin_value, u32 tt_const,
+                                                                           const u32 *pin_edges, int E, GoalMask goal) {
+    EnvView ev;
+    memset(&ev, 0, sizeof ev);
+    unsigned char *blob = smem_raw;
+    const SsdSmem L = ssd_smem(nv, ev, sp, false, true);  // sp.smem_hist: g <= 12
+    u32 *s_free = reinterpret_cast<u32 *>(smem_raw + L.pin);
+    u32 *s_tgt = reinterpret_cast<u32 *>(smem_raw + L.tgt);
+    u32 *s_goal = reinterpret_cast<u32 *>(smem_raw + L.hist);
+    const int nb = 1 << sp.g;
+    u32 *sst = align_cols(s_goal + nb, nv.w32);
+    const int w32 = nv.w32;
+    const u32 *care = pin_care + (size_t)blockIdx.y * w32, *value = pin_value + (size_t)blockIdx.y * w32;
+    stage(blob, nv.blob, L.image);
+    pin_patch<NET>(nv, blob, s_free, care, value, tt_const, pin_edges + (size_t)blockIdx.y * E, E, [&] {
+        if (threadIdx.x == 0) {
+#pragma unroll
+            for (int k = 0; k < 24; k++) s_tgt[k] = (u32)sp.tgt[k];
+#pragma unroll
+            for (int k = 0; k < 128; k++)  // static indices: read straight from the parameter bank
+                if (k < ((nb + 31) >> 5)) s_goal[k] = goal.w[k];
+        }
+    });
+    const long long e = (long long)blockIdx.x * PBN_BLOCK + threadIdx.x;
+    const long long B = (long long)gridDim.y * chains, col = (long long)blockIdx.y * chains + e;
+    Col st{sst + threadIdx.x};
+    const bool active = e < chains;
+    const bool run = active && t_hit[col] < 0;
+    if (run) {
+        load_state(st, state, B, col, w32);
+        pin_state(nv, st, care, value);
+    }
+    __syncthreads();
+    const long long warp_left = chains - (e - (threadIdx.x & 31));
+    if (warp_left > 0) {
+        Draw<PBN_DRAW_PHILOX> d, dp;
+        d.init(dv, e, env0 + e);
+        dp.init_perturb(dv, e, env0 + e);
+        const u32 nvalid = warp_left >= 32 ? 32u : (u32)warp_left;
+        u32 hit = run ? ~0u : 0u;  // a lane without a chain to run is never live
+        SsdLoopArgs a{nv, ev, sp, dv, blob, nullptr, nullptr, s_tgt, s_goal, nullptr, sst, iters, nvalid, nullptr, 0, env0 + e, nullptr};
+        if (nvalid == 32u) ssd_loop<NET, PBN_DRAW_PHILOX, TQ, false, true, true, true>(a, st, d, dp, s_free, &hit);
+        else ssd_loop<NET, PBN_DRAW_PHILOX, TQ, false, false, true, true>(a, st, d, dp, s_free, &hit);
+        if (run) {
+            if (hit != ~0u) t_hit[col] = t0 + (long long)hit;
+            else store_state(st, state, B, col, w32);
+        }
     }
 }
 
@@ -2659,37 +2793,81 @@ extern "C" int pbn_ssd(const PbnNet *net, const PbnEnv *env, uint32_t *state, in
     });
 }
 
-extern "C" int pbn_ssd_pinned_edges(const PbnNet *net, uint32_t *state, int64_t chains, int64_t env0, int64_t iters, double p,
-                                    const uint32_t *pin_care, const uint32_t *pin_value, int32_t K, const uint32_t *pin_edges,
-                                    int32_t E, const int32_t *tgt, int32_t g, uint64_t *hist, const PbnDraws *draws, void *stream) {
-    if (!net || !state || !pin_care || !pin_value || !tgt || !hist || chains < 0 || iters < 0) return fail(PBN_ERR_ARG, "bad argument");
+// Argument checks and launch set-up shared by pbn_ssd_pinned_edges and pbn_first_passage.  *run = false: nothing to launch.
+struct PinnedLaunch {
+    SsdParams sp;
+    NetView nv;
+    DrawView dv;
+    size_t smem;
+    dim3 grid;
+};
+static int pinned_prepare(const PbnNet *net, const uint32_t *state, int64_t chains, int64_t env0, int64_t iters, double p,
+                          const uint32_t *pin_care, const uint32_t *pin_value, int32_t K, const uint32_t *pin_edges, int32_t E,
+                          const int32_t *tgt, int32_t g, const PbnDraws *draws, cudaStream_t s, PinnedLaunch &P, bool *run) {
+    *run = false;
+    if (!net || !state || !pin_care || !pin_value || !tgt || chains < 0 || iters < 0) return fail(PBN_ERR_ARG, "bad argument");
     if (K < 1 || K > 65535) return fail(PBN_ERR_ARG, "1 <= K <= 65535 pin sets");
     if (E < 0 || E > 64) return fail(PBN_ERR_ARG, "0 <= E <= 64 edge slots per pin set");
     if (E > 0 && !pin_edges) return fail(PBN_ERR_ARG, "E > 0 edge slots need pin_edges");
     if (draws && draws->mode == PBN_DRAW_REPLAY) return fail(PBN_ERR_UNSUPPORTED, "pinned SSD estimates draw from Philox streams only");
     // folding an edge rewrites the node's thresholds, which a table read through thr_dev would need a per-variant copy of
     if (E > 0 && net->v.thr_dev) return fail(PBN_ERR_UNSUPPORTED, "edge pins need the threshold table in shared memory (at most PBN_TT_THR_SMEM_MAX bytes)");
-    cudaStream_t s = (cudaStream_t)stream;
-    SsdParams sp;
-    bool run;
-    if (int rc = ssd_prepare(net->v, chains, env0, iters, p, tgt, g, draws, s, sp, &run)) return rc;
-    if (!run) return PBN_OK;
-    NetView nv = net->v;
+    if (int rc = ssd_prepare(net->v, chains, env0, iters, p, tgt, g, draws, s, P.sp, run)) return rc;
+    if (!*run) return PBN_OK;
+    P.nv = net->v;
     // a truth-table network whose threshold table is staged also stages the two constant entries behind it
-    if (nv.kind == PBN_NET_TT && !nv.thr_dev) nv.blob_bytes = nv.blob_fast_bytes = nv.blob_bytes + 16;
-    const DrawView dv = make_draws(draws);
+    if (P.nv.kind == PBN_NET_TT && !P.nv.thr_dev) P.nv.blob_bytes = P.nv.blob_fast_bytes = P.nv.blob_bytes + 16;
+    P.dv = make_draws(draws);
     EnvView ev;
     memset(&ev, 0, sizeof ev);
-    const size_t smem = ssd_smem(nv, ev, sp, false, true).bytes;
-    const dim3 grid((unsigned)((chains + PBN_BLOCK - 1) / PBN_BLOCK), (unsigned)K);
+    P.smem = ssd_smem(P.nv, ev, P.sp, false, true).bytes;
+    P.grid = dim3((unsigned)((chains + PBN_BLOCK - 1) / PBN_BLOCK), (unsigned)K);
+    return PBN_OK;
+}
+
+extern "C" int pbn_ssd_pinned_edges(const PbnNet *net, uint32_t *state, int64_t chains, int64_t env0, int64_t iters, double p,
+                                    const uint32_t *pin_care, const uint32_t *pin_value, int32_t K, const uint32_t *pin_edges,
+                                    int32_t E, const int32_t *tgt, int32_t g, uint64_t *hist, const PbnDraws *draws, void *stream) {
+    if (!hist) return fail(PBN_ERR_ARG, "bad argument");
+    cudaStream_t s = (cudaStream_t)stream;
+    PinnedLaunch P;
+    bool run;
+    if (int rc = pinned_prepare(net, state, chains, env0, iters, p, pin_care, pin_value, K, pin_edges, E, tgt, g, draws, s, P, &run))
+        return rc;
+    if (!run) return PBN_OK;
     auto launch = [&](auto kernel) -> int {
-        if (int rc = fit_smem(kernel, "k_ssd_pinned", smem)) return rc;
-        kernel<<<grid, PBN_BLOCK, smem, s>>>(nv, dv, sp, state, chains, env0, (int)iters, (unsigned long long *)hist, pin_care,
-                                             pin_value, net->tt_const, pin_edges, (int)E);
+        if (int rc = fit_smem(kernel, "k_ssd_pinned", P.smem)) return rc;
+        kernel<<<P.grid, PBN_BLOCK, P.smem, s>>>(P.nv, P.dv, P.sp, state, chains, env0, (int)iters, (unsigned long long *)hist,
+                                                 pin_care, pin_value, net->tt_const, pin_edges, (int)E);
         CK(cudaGetLastError());
         return PBN_OK;
     };
-    return dispatch(nv.kind, dv.mode, nv.ts, [&](auto NK, auto, auto TQ) { return launch(k_ssd_pinned<NK, TQ>); });
+    return dispatch(P.nv.kind, P.dv.mode, P.nv.ts, [&](auto NK, auto, auto TQ) { return launch(k_ssd_pinned<NK, TQ>); });
+}
+
+extern "C" int pbn_first_passage(const PbnNet *net, uint32_t *state, int64_t chains, int64_t env0, int64_t iters, int64_t t0,
+                                 double p, const uint32_t *pin_care, const uint32_t *pin_value, int32_t K,
+                                 const uint32_t *pin_edges, int32_t E, const int32_t *tgt, int32_t g, const uint32_t *goal_host,
+                                 int64_t *t_hit, const PbnDraws *draws, void *stream) {
+    if (!goal_host || !t_hit || t0 < 0) return fail(PBN_ERR_ARG, "bad argument");
+    if (g < 1 || g > 12) return fail(PBN_ERR_ARG, "1 <= g <= 12 target nodes: the goal mask sits where the block histogram would");
+    cudaStream_t s = (cudaStream_t)stream;
+    PinnedLaunch P;
+    bool run;
+    if (int rc = pinned_prepare(net, state, chains, env0, iters, p, pin_care, pin_value, K, pin_edges, E, tgt, g, draws, s, P, &run))
+        return rc;
+    if (!run) return PBN_OK;
+    GoalMask goal;
+    memset(&goal, 0, sizeof goal);
+    memcpy(goal.w, goal_host, (g >= 5 ? (size_t)1 << (g - 5) : 1) * 4);
+    auto launch = [&](auto kernel) -> int {
+        if (int rc = fit_smem(kernel, "k_passage", P.smem)) return rc;
+        kernel<<<P.grid, PBN_BLOCK, P.smem, s>>>(P.nv, P.dv, P.sp, state, chains, env0, (int)iters, (long long)t0,
+                                                 (long long *)t_hit, pin_care, pin_value, net->tt_const, pin_edges, (int)E, goal);
+        CK(cudaGetLastError());
+        return PBN_OK;
+    };
+    return dispatch(P.nv.kind, P.dv.mode, P.nv.ts, [&](auto NK, auto, auto TQ) { return launch(k_passage<NK, TQ>); });
 }
 
 extern "C" int pbn_ssd_pinned(const PbnNet *net, uint32_t *state, int64_t chains, int64_t env0, int64_t iters, double p,

@@ -87,6 +87,9 @@ EXPORTS = {
     "pbn_ssd_pinned_edges": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_double, C.c_void_p,
                                        C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p,
                                        C.POINTER(PbnDraws), C.c_void_p]),
+    "pbn_first_passage": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_int64, C.c_double,
+                                    C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_int32,
+                                    C.c_void_p, C.c_void_p, C.POINTER(PbnDraws), C.c_void_p]),
     "pbn_bucket_hist": (C.c_int, [C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]),
     "pbn_ssd_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_double, C.c_void_p,
                                C.c_int32, C.c_uint64, C.c_uint32, C.c_void_p]),

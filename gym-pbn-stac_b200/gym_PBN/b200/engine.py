@@ -446,6 +446,19 @@ class Simulator:
         return hist
 
 
+def _pin_args(sim, care, value, edges):
+    """Device copies of a launch's pin arguments: (care, value, edges or None, E)."""
+    care = torch.from_numpy(np.ascontiguousarray(care, np.uint32).view(np.int32)).to(sim.device)
+    value = torch.from_numpy(np.ascontiguousarray(value, np.uint32).view(np.int32)).to(sim.device)
+    if edges is None:
+        return care, value, None, 0
+    edges = np.ascontiguousarray(edges, np.uint32)
+    if edges.ndim != 2 or edges.shape[0] != care.shape[0]:
+        raise ValueError(f"edges must be [K][E] with K = {care.shape[0]} pin sets, got shape {edges.shape}")
+    E = edges.shape[1]
+    return care, value, torch.from_numpy(edges.view(np.int32)).to(sim.device) if E else None, E
+
+
 def ssd_pinned(sim: "Simulator", state, iters, bit_flip_prob, tgt_nodes, care, value, hist, edges=None):
     """pbn_ssd_pinned_edges: the sim.B chains of `sim` (chain ids sim.env0 + c, one epoch of its stream, like Simulator.ssd)
     under K pin sets.  state: int32 planes [W32][K * sim.B] on sim's device (column k * B + c = chain c of variant k);
@@ -453,23 +466,35 @@ def ssd_pinned(sim: "Simulator", state, iters, bit_flip_prob, tgt_nodes, care, v
     edges: None (no edge pins) or a uint32 [K][E] host array, E <= 64 (row k = the edge pins of variant k, entry
     dst | src << 12 | c << 24, 0xFFFFFFFF = empty slot); hist: int64 [K][2^g] device tensor, accumulated."""
     tgt = np.ascontiguousarray(tgt_nodes, np.int32)
-    care = torch.from_numpy(np.ascontiguousarray(care, np.uint32).view(np.int32)).to(sim.device)
-    value = torch.from_numpy(np.ascontiguousarray(value, np.uint32).view(np.int32)).to(sim.device)
-    E, eptr = 0, None
-    if edges is not None:
-        edges = np.ascontiguousarray(edges, np.uint32)
-        if edges.ndim != 2 or edges.shape[0] != care.shape[0]:
-            raise ValueError(f"edges must be [K][E] with K = {care.shape[0]} pin sets, got shape {edges.shape}")
-        E = edges.shape[1]
-        edges = torch.from_numpy(edges.view(np.int32)).to(sim.device)
-        eptr = _ptr(edges) if E else None
+    care, value, edges, E = _pin_args(sim, care, value, edges)
     d = sim._draws()
     with on_device(sim.device):
         abi.check(abi.lib().pbn_ssd_pinned_edges(sim.net.handle, _ptr(state), sim.B, sim.env0, int(iters),
-                                                 float(bit_flip_prob), _ptr(care), _ptr(value), care.shape[0], eptr, E,
-                                                 _np_ptr(tgt), len(tgt), _ptr(hist), C.byref(d), _stream()))
+                                                 float(bit_flip_prob), _ptr(care), _ptr(value), care.shape[0],
+                                                 _ptr(edges) if E else None, E, _np_ptr(tgt), len(tgt), _ptr(hist),
+                                                 C.byref(d), _stream()))
     sim.launches += 1
     return hist
+
+
+def first_passage(sim: "Simulator", state, iters, t0, bit_flip_prob, tgt_nodes, goal_words, care, value, t_hit, edges=None):
+    """pbn_first_passage: ssd_pinned's chains, variants and arguments (one epoch of sim's stream), with each iteration's
+    count replaced by a test against the goal.  goal_words: uint32 [max(1, 2^g / 32)] host array, bit b = bucket b is in the
+    goal; t_hit: int64 [K][sim.B] device tensor, in/out (>= 0 on entry: arrived, neither run nor written; otherwise t0 + the
+    first iteration whose state lies in the goal, or -1)."""
+    tgt = np.ascontiguousarray(tgt_nodes, np.int32)
+    goal = np.ascontiguousarray(goal_words, np.uint32)
+    if goal.size < max(1, (1 << len(tgt)) // 32):
+        raise ValueError(f"goal_words needs {max(1, (1 << len(tgt)) // 32)} words for {len(tgt)} target nodes")
+    care, value, edges, E = _pin_args(sim, care, value, edges)
+    d = sim._draws()
+    with on_device(sim.device):
+        abi.check(abi.lib().pbn_first_passage(sim.net.handle, _ptr(state), sim.B, sim.env0, int(iters), int(t0),
+                                              float(bit_flip_prob), _ptr(care), _ptr(value), care.shape[0],
+                                              _ptr(edges) if E else None, E, _np_ptr(tgt), len(tgt), _np_ptr(goal),
+                                              _ptr(t_hit), C.byref(d), _stream()))
+    sim.launches += 1
+    return t_hit
 
 
 def bucket_hist(sim: "Simulator", tgt_nodes, hist):

@@ -17,6 +17,8 @@ blocks or forces single regulatory interactions (edge pins: the target gene's fu
                              env.target_node_values (the measure of utils.eval.eval_increase)
   regulatory_edges           the (src, dst) pairs of the network: src is read by some function of dst
   rank_edge_pins             every single-edge pin (src -> dst read as 0, as 1), ranked the same way
+  first_passage              how many iterations each chain needs to reach a set of target-gene patterns under each pin
+                             set (pbn_first_passage); rank_pins / rank_edge_pins(measure="passage") rank pins by it
 """
 import numpy as np
 import torch
@@ -183,33 +185,15 @@ def _node_index(env, net, node):
     raise ValueError(f"{node!r} is neither a gene id of the env nor a node index in [0, {net.n})")
 
 
-def pinned_ssd(env_or_network, pins, iters, chains, bit_flip_prob=0.01, target_nodes=None, seed=0, distributed=False):
-    """Visit histograms of the target-gene patterns under each pin set of `pins`, from one launch per iteration chunk.
-
-    env_or_network: an env (its network; target_nodes default to env.target_node_indices) or an engine.Network.
-    pins: list of {node: 0 or 1} dicts, node = node index or gene id (Bittner envs); {} = the network unpinned.
-    A variant holds its pinned nodes at their values: they are set before the first iteration, an update that picks one
-    leaves it as it is, and perturbations skip it.  A key (src, dst), both ends resolved as node keys are, pins that edge
-    of regulatory_edges: whenever dst is updated its function reads the pinned value in place of src (src itself, and every
-    other node that reads it, are unchanged); a pair that is not an edge raises ValueError.  Up to 64 edge pins per
-    variant; truth-table networks with more than 16 KB of threshold table take none.  Otherwise every iteration is the one
-    of utils.eval.ssd_histogram without an env: count the pattern, flip each gene w.p. bit_flip_prob, one asynchronous
-    update (include/pbn_b200.h: pbn_ssd_pinned_edges).  Every variant starts from the same uniform random states (Graph.genRandState) and runs on the same
-    random numbers, so differences between rows are not drowned in independent sampling noise, and the row of {} is
-    utils.eval.ssd_histogram's estimate for those start states.  With distributed=True chains are sharded over ranks by
-    global chain id (multiples of 32) and the histograms are summed.
-
-    Returns int64 [K][2^g] (NumPy), bucket = target-node bits, first target most significant; each row sums to
-    iters * chains."""
-    from gym_PBN.utils.eval import MAX_ITERS_PER_LAUNCH
-
+def _env_and_net(env_or_network):
+    """(env or None, engine.Network) of pinned_ssd's and first_passage's first argument."""
     env = None if isinstance(env_or_network, engine.Network) else getattr(env_or_network, "unwrapped", env_or_network)
-    net = env_or_network if env is None else env.network
-    if target_nodes is None:
-        if env is None:
-            raise ValueError("target_nodes are needed with a bare network")
-        target_nodes = env.target_node_indices
-    tgt = np.asarray([_node_index(env, net, t) for t in target_nodes], np.int32)
+    return env, (env_or_network if env is None else env.network)
+
+
+def _pin_masks(env, net, pins):
+    """The launch arguments of a list of pin sets (pinned_ssd's `pins`): care, value uint32 [K][W32] and edges uint32 [K][E]
+    (None when no set pins an edge)."""
     pins = list(pins)
     K = len(pins)
     if not 1 <= K <= 65535:
@@ -243,6 +227,37 @@ def pinned_ssd(env_or_network, pins, iters, chains, bit_flip_prob=0.01, target_n
         edges = np.full((K, E), 0xFFFFFFFF, np.uint32)
         for k, row in enumerate(rows):
             edges[k, :len(row)] = row
+    return care, value, edges
+
+
+def pinned_ssd(env_or_network, pins, iters, chains, bit_flip_prob=0.01, target_nodes=None, seed=0, distributed=False):
+    """Visit histograms of the target-gene patterns under each pin set of `pins`, from one launch per iteration chunk.
+
+    env_or_network: an env (its network; target_nodes default to env.target_node_indices) or an engine.Network.
+    pins: list of {node: 0 or 1} dicts, node = node index or gene id (Bittner envs); {} = the network unpinned.
+    A variant holds its pinned nodes at their values: they are set before the first iteration, an update that picks one
+    leaves it as it is, and perturbations skip it.  A key (src, dst), both ends resolved as node keys are, pins that edge
+    of regulatory_edges: whenever dst is updated its function reads the pinned value in place of src (src itself, and every
+    other node that reads it, are unchanged); a pair that is not an edge raises ValueError.  Up to 64 edge pins per
+    variant; truth-table networks with more than 16 KB of threshold table take none.  Otherwise every iteration is the one
+    of utils.eval.ssd_histogram without an env: count the pattern, flip each gene w.p. bit_flip_prob, one asynchronous
+    update (include/pbn_b200.h: pbn_ssd_pinned_edges).  Every variant starts from the same uniform random states (Graph.genRandState) and runs on the same
+    random numbers, so differences between rows are not drowned in independent sampling noise, and the row of {} is
+    utils.eval.ssd_histogram's estimate for those start states.  With distributed=True chains are sharded over ranks by
+    global chain id (multiples of 32) and the histograms are summed.
+
+    Returns int64 [K][2^g] (NumPy), bucket = target-node bits, first target most significant; each row sums to
+    iters * chains."""
+    from gym_PBN.utils.eval import MAX_ITERS_PER_LAUNCH
+
+    env, net = _env_and_net(env_or_network)
+    if target_nodes is None:
+        if env is None:
+            raise ValueError("target_nodes are needed with a bare network")
+        target_nodes = env.target_node_indices
+    tgt = np.asarray([_node_index(env, net, t) for t in target_nodes], np.int32)
+    care, value, edges = _pin_masks(env, net, pins)
+    K = care.shape[0]
     start, stop = pdist.shard_range(chains, align=32) if distributed else (0, int(chains))
     local = stop - start
     hist = torch.zeros((K, 1 << len(tgt)), dtype=torch.int64, device=net.device)
@@ -261,24 +276,112 @@ def pinned_ssd(env_or_network, pins, iters, chains, bit_flip_prob=0.01, target_n
     return hist.cpu().numpy()
 
 
+def goal_words(patterns, g):
+    """The goal mask of pbn_first_passage for a list of target-gene patterns (g values 0/1 each, first target most
+    significant, as env.target_node_values holds them): uint32 [max(1, 2^g / 32)], bit b set for every pattern's bucket b."""
+    words = np.zeros(max(1, (1 << g) // 32), np.uint32)
+    for b in _bucket_ids(patterns, g, "goal patterns"):
+        words[b >> 5] |= np.uint32(1 << (b & 31))
+    return words
+
+
+def first_passage(env_or_network, pins, iters, chains, goal=None, start=None, bit_flip_prob=0.01, target_nodes=None, seed=0,
+                  distributed=False):
+    """First-passage times into the goal patterns of the target genes, for each pin set of `pins` (pinned_ssd's keys: node,
+    gene id or (src, dst) edge) on common random numbers.
+
+    An iteration is pinned_ssd's (look at the pattern, flip each gene w.p. bit_flip_prob, one asynchronous update) with the
+    count replaced by a test: a chain whose pattern lies in `goal` at iteration t has first-passage time t and stops.  So 0
+    means the start state, with its pins applied, is already there; -1 means the goal was not reached within `iters`.
+    goal: list of patterns of the target genes (default env.target_node_values), at most 12 target genes.
+    start: None = the env's reset states (a uniform attractor, a uniform cube of it) when it has at least two attractors,
+    otherwise uniform random states (Graph.genRandState), as utils.eval.ssd_histogram chooses; or a uint8 [chains][N] array.
+    Every variant starts chain c from the same state.  Launches run MAX_ITERS_PER_LAUNCH iterations at most and stop once
+    every chain has arrived.  With distributed=True chains are sharded over ranks by global chain id (multiples of 32) and
+    every rank gets the whole table.
+
+    Returns {"time": int64 [K][chains] (NumPy, -1 = not reached), "source": int64 [chains], the attractor index of each
+    reset start (pbn_env_attractor_index, -1 = none), or None for other starts}."""
+    from gym_PBN.utils.eval import MAX_ITERS_PER_LAUNCH
+
+    env, net = _env_and_net(env_or_network)
+    if target_nodes is None:
+        if env is None:
+            raise ValueError("target_nodes are needed with a bare network")
+        target_nodes = env.target_node_indices
+    tgt = np.asarray([_node_index(env, net, t) for t in target_nodes], np.int32)
+    if goal is None:
+        if env is None:
+            raise ValueError("a goal is needed with a bare network")
+        goal = env.target_node_values
+    words = goal_words(goal, len(tgt))
+    care, value, edges = _pin_masks(env, net, pins)
+    K, chains, iters = care.shape[0], int(chains), int(iters)
+    image = getattr(env, "env_image", None) if start is None else None
+    reset = image is not None and image.n_att >= 2
+    if start is not None:
+        start = np.asarray(start, np.uint8)
+        if start.shape != (chains, net.n):
+            raise ValueError(f"start must be uint8 [{chains}][{net.n}], got shape {start.shape}")
+    lo, hi = pdist.shard_range(chains, align=32) if distributed else (0, chains)
+    local = hi - lo
+    time = torch.zeros((K, chains), dtype=torch.int64, device=net.device)  # t + 1 on this rank's chains, 0 elsewhere
+    source = torch.zeros(chains, dtype=torch.int64, device=net.device)     # attractor index + 1 likewise
+    if local > 0:
+        sim = engine.Simulator(net, local, seed=seed, env0=lo)
+        with engine.on_device(net.device):
+            if start is not None:
+                sim.set_state(start[lo:hi])
+            elif reset:
+                sim.env_reset(image)
+                source[lo:hi] = engine.attractor_index(sim, image).long() + 1
+            else:
+                sim.rand_state()
+            state = sim.state.repeat(1, K)  # column k * local + c: chain c of variant k
+            t_hit = torch.full((K, local), -1, dtype=torch.int64, device=net.device)
+            t0 = 0
+            while t0 < iters and bool((t_hit < 0).any()):
+                chunk = min(iters - t0, MAX_ITERS_PER_LAUNCH)
+                engine.first_passage(sim, state, chunk, t0, bit_flip_prob, tgt, words, care, value, t_hit, edges=edges)
+                t0 += chunk
+            time[:, lo:hi] = t_hit + 1
+    if distributed:
+        pdist.allreduce_sum_(time)
+        pdist.allreduce_sum_(source)
+    return {"time": (time - 1).cpu().numpy(), "source": (source - 1).cpu().numpy() if reset else None}
+
+
 def _bucket_ids(patterns, g, what):
     """Histogram buckets of target-gene patterns (first target most significant)."""
     out = []
     for p in patterns or ():
         if len(p) != g or any(b not in (0, 1) for b in p):
-            raise ValueError(f"env.{what} must hold patterns of {g} target-gene values 0/1, got {p!r}")
+            raise ValueError(f"{what} must hold patterns of {g} target-gene values 0/1, got {p!r}")
         out.append(int("".join(str(int(b)) for b in p), 2))
     return out
 
 
-def _rank(env, pins, rows, iters, chains, bit_flip_prob, seed):
+def _rank(env, pins, rows, iters, chains, bit_flip_prob, seed, measure="ssd"):
     """The ranking of rank_pins and rank_edge_pins: pins[0] = {} and pins[k] the variant of rows[k - 1] (the identifying
-    fields of its ranking entry), all estimated by one pinned_ssd launch."""
+    fields of its ranking entry), all estimated on common random numbers by one pinned_ssd (measure "ssd") or
+    first_passage (measure "passage") run.  The passage fields: "reached" = the fraction of chains that arrived,
+    "mean_time" = the restricted mean mean(min(T, iters)) (a chain that did not arrive counts as iters), "change" =
+    mean_time minus the unpinned one; fastest first."""
+    if measure == "passage":
+        t = first_passage(env, pins, iters, chains, bit_flip_prob=bit_flip_prob, seed=seed)["time"]
+        reached = (t >= 0).mean(1)
+        mean_time = np.where(t >= 0, np.minimum(t, iters), iters).mean(1)
+        ranking = [dict(row, reached=float(reached[k]), mean_time=float(mean_time[k]),
+                        change=float(mean_time[k] - mean_time[0])) for k, row in enumerate(rows, start=1)]
+        ranking.sort(key=lambda r: r["change"])
+        return {"unpinned": {"reached": float(reached[0]), "mean_time": float(mean_time[0])}, "ranking": ranking}
+    if measure != "ssd":
+        raise ValueError(f'measure is "ssd" or "passage", got {measure!r}')
     hist = pinned_ssd(env, pins, iters, chains, bit_flip_prob=bit_flip_prob, seed=seed).astype(np.float64)
     mass = hist / hist.sum(1, keepdims=True)
     g = len(env.target_node_indices)
-    good = _bucket_ids(env.target_node_values, g, "target_node_values")
-    bad = _bucket_ids(env.undesired_node_values, g, "undesired_node_values")
+    good = _bucket_ids(env.target_node_values, g, "env.target_node_values")
+    bad = _bucket_ids(env.undesired_node_values, g, "env.undesired_node_values")
     tm, um = mass[:, good].sum(1), mass[:, bad].sum(1)
     ranking = [dict(row, target_mass=float(tm[k]), undesired_mass=float(um[k]), increase=float(tm[k] - tm[0]))
                for k, row in enumerate(rows, start=1)]
@@ -286,7 +389,7 @@ def _rank(env, pins, rows, iters, chains, bit_flip_prob, seed):
     return {"unpinned": {"target_mass": float(tm[0]), "undesired_mass": float(um[0])}, "ranking": ranking}
 
 
-def rank_pins(env, genes=None, iters=4000, chains=300, bit_flip_prob=0.01, seed=0):
+def rank_pins(env, genes=None, iters=4000, chains=300, bit_flip_prob=0.01, seed=0, measure="ssd"):
     """Every single-gene pin (gene -> 0, gene -> 1) of `genes` (gene ids or node indices; default every node), ranked by the
     change of steady-state mass on env.target_node_values against the unpinned network: eval_increase's measure, with the
     pin in place of a controller.  One pinned_ssd launch estimates all 1 + 2 * len(genes) variants on common random numbers;
@@ -294,7 +397,13 @@ def rank_pins(env, genes=None, iters=4000, chains=300, bit_flip_prob=0.01, seed=
 
     Returns {"unpinned": {"target_mass", "undesired_mass"}, "ranking": [...]}: one dict per pin with "gene" (id or index as
     given), "node" (index), "value", "target_mass", "undesired_mass" (mass on env.undesired_node_values) and "increase"
-    (target_mass minus the unpinned one), best first."""
+    (target_mass minus the unpinned one), best first.
+
+    measure="passage" ranks by how fast the pin gets there instead: first_passage (from the env's reset states) into
+    env.target_node_values, `iters` iterations at most, all variants in one run.  Each dict then has "reached" (fraction of
+    chains that got there), "mean_time" (mean of min(T, iters), a chain that did not get there counting as iters) and
+    "change" (mean_time minus the unpinned one) in place of the mass fields, fastest first; "unpinned" has "reached" and
+    "mean_time"."""
     env = getattr(env, "unwrapped", env)
     net = env.network
     if genes is None:
@@ -302,7 +411,7 @@ def rank_pins(env, genes=None, iters=4000, chains=300, bit_flip_prob=0.01, seed=
     genes = list(genes)
     pins = [{}] + [{g: v} for g in genes for v in (0, 1)]
     rows = [{"gene": g, "node": _node_index(env, net, g), "value": v} for g in genes for v in (0, 1)]
-    return _rank(env, pins, rows, iters, chains, bit_flip_prob, seed)
+    return _rank(env, pins, rows, iters, chains, bit_flip_prob, seed, measure)
 
 
 def _edge_nodes(spec):
@@ -339,7 +448,7 @@ def regulatory_edges(env_or_network):
     return [(ids[s], ids[d]) for s, d in edges] if ids is not None else edges
 
 
-def rank_edge_pins(env, edges=None, iters=4000, chains=300, bit_flip_prob=0.01, seed=0):
+def rank_edge_pins(env, edges=None, iters=4000, chains=300, bit_flip_prob=0.01, seed=0, measure="ssd"):
     """Every single-edge pin ((src, dst) -> 0, -> 1) of `edges` ((src, dst) pairs of gene ids or node indices; default
     regulatory_edges(env), self-inputs included), ranked as rank_pins ranks gene pins: by the change of steady-state mass
     on env.target_node_values against the unpinned network.  Pinning (src, dst) at c makes dst's function read c in place
@@ -348,11 +457,12 @@ def rank_edge_pins(env, edges=None, iters=4000, chains=300, bit_flip_prob=0.01, 
     numbers (at most 65 535 variants).
 
     Returns {"unpinned": {"target_mass", "undesired_mass"}, "ranking": [...]}: one dict per edge pin with "src", "dst" (as
-    given), "src_node", "dst_node" (indices), "value", "target_mass", "undesired_mass" and "increase", best first."""
+    given), "src_node", "dst_node" (indices), "value", "target_mass", "undesired_mass" and "increase", best first.
+    measure="passage" ranks them by first-passage time, with rank_pins' passage fields."""
     env = getattr(env, "unwrapped", env)
     net = env.network
     edges = regulatory_edges(env) if edges is None else [tuple(e) for e in edges]
     pins = [{}] + [{e: v} for e in edges for v in (0, 1)]
     rows = [{"src": s, "dst": d, "src_node": _node_index(env, net, s), "dst_node": _node_index(env, net, d), "value": v}
             for s, d in edges for v in (0, 1)]
-    return _rank(env, pins, rows, iters, chains, bit_flip_prob, seed)
+    return _rank(env, pins, rows, iters, chains, bit_flip_prob, seed, measure)

@@ -273,6 +273,34 @@ int pbn_ssd_pinned_edges(const PbnNet *net, uint32_t *state, int64_t chains, int
                          const uint32_t *pin_care, const uint32_t *pin_value, int32_t K, const uint32_t *pin_edges, int32_t E,
                          const int32_t *tgt_nodes_host, int32_t g, uint64_t *hist, const PbnDraws *draws, void *stream);
 
+/* First-passage times into a set of target-gene patterns under K variants (node pins plus edge pins, as in
+   pbn_ssd_pinned_edges): how long each chain takes to reach the goal, where pbn_ssd_pinned_edges says how much time it
+   spends there.  This serves gym_PBN.utils.control.first_passage and the passage measure of rank_pins / rank_edge_pins.
+   The closest reference interface is utils.eval.eval_winrate, which reports the mean number of steps a controller needs to
+   reach the target; the reference has no such call for pinned networks.
+   The goal is a set of buckets, bucket = target-node bits with the first target most significant (the SSD's encoding).
+   One iteration of a chain is pbn_ssd_pinned_edges's (count, perturb, one asynchronous update) with the count replaced by
+   a goal test: if the bucket of the current state lies in the goal, the chain's first-passage time is t0 + t (t = the
+   iteration index within this call) and the chain stops.  So time t0 means the start state, its pins applied, is already in
+   the goal.  A chain that has not reached the goal after `iters` iterations keeps -1, and its state is the state after
+   them: the start state of a following call (with t0 + iters and the next epoch).  Chain c of every variant draws from the
+   streams of chain id env0 + c, as in pbn_ssd_pinned_edges; with an empty goal no chain stops and every final state is
+   pbn_ssd_pinned_edges's with the same arguments, bit for bit.
+     state      planes [W32][K * chains], the column layout of pbn_ssd_pinned_edges
+     goal_host  host uint32 [max(1, 2^g / 32)]: bit b (bit b % 32 of word b / 32) = bucket b lies in the goal
+     t_hit      device int64 [K][chains], in/out.  A chain whose entry is >= 0 has arrived: it is neither run nor written
+                (its entry and its state column stay as they are; its lane still takes part in the warp's perturbation
+                stream, as the missing lanes of a partial warp do).  Any other chain gets its first-passage time or keeps
+                -1.  The state of a chain that stops is unspecified.
+   Every rule of pbn_ssd_pinned_edges applies (env0 % 32 == 0 with bit_flip_prob > 0, 1 <= K <= 65535, 0 <= E <= 64, the
+   iteration limits, PBN_ERR_UNSUPPORTED for replay draws and for edge pins on a threshold table in global memory), and
+   1 <= g <= 12 (the goal mask takes the place of the block histogram), goal_host and t_hit non-null and t0 >= 0
+   (PBN_ERR_ARG otherwise). */
+int pbn_first_passage(const PbnNet *net, uint32_t *state, int64_t chains, int64_t env0, int64_t iters, int64_t t0,
+                      double bit_flip_prob, const uint32_t *pin_care, const uint32_t *pin_value, int32_t K,
+                      const uint32_t *pin_edges, int32_t E, const int32_t *tgt_nodes_host, int32_t g,
+                      const uint32_t *goal_host, int64_t *t_hit, const PbnDraws *draws, void *stream);
+
 /* hist[bucket(state_e)] += 1 for every env e — the first two lines of an _ssd_run iteration (utils/eval.py:88-89) as a
    stand-alone kernel, for estimates whose actions come from a policy between steps (eval.py:97-101). */
 int pbn_bucket_hist(const uint32_t *state, int64_t B, int32_t n_nodes, const int32_t *tgt_nodes_host, int32_t g,
